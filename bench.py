@@ -18,6 +18,7 @@ A step = one pass of the hot path over the rank's shard:
     python bench.py                      # 1 GPU
     torchrun --nproc-per-node 8 bench.py --gpus 8
     python bench.py --impl reference     # the reference's CPU path on this box's host cores
+    python bench.py --dump-outputs DIR   # also write the last timed step's tables to DIR/*.npy (compare two builds)
 """
 from __future__ import annotations
 
@@ -67,7 +68,22 @@ def parse_args():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --reads-per-gpu on every GPU (the default; 8 GPUs = the 200 M reads of configs[1]); "
                          "strong: the 8 x --reads-per-gpu reads of configs[1] split over the GPUs in use")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/pss_fwd.npy, pss_rev.npy, pss_stats.npy (float64)")
     return ap.parse_args()
+
+
+def dump_outputs(d, tables, stats, R):
+    """The last timed step's result as float64 arrays (exact: every count is far below 2**53).  pss_fwd / pss_rev are
+    the (R+2) x 16 count tables pssgpu_pss_finish_device wrote (all-reduced when N > 1); pss_stats holds rank 0's
+    outcome counters lines, counted, no_contig, filtered, parse_fail, undefined.  The inputs are seeded, so two builds
+    run with the same arguments can be compared array for array."""
+    os.makedirs(d, exist_ok=True)
+    t = tables.numpy().astype(np.float64).reshape(2, R + 2, 16)
+    np.save(os.path.join(d, "pss_fwd.npy"), t[0])
+    np.save(os.path.join(d, "pss_rev.npy"), t[1])
+    keys = ("lines", "counted", "no_contig", "filtered", "parse_fail", "undefined")
+    np.save(os.path.join(d, "pss_stats.npy"), np.array([stats[k] for k in keys], dtype=np.float64))
 
 
 def contig_plan(scale):
@@ -172,7 +188,7 @@ class ReferenceSample:
     def __init__(self, n_proc, reads_per_proc, genome_mb, seed):
         from pss_testlib import Synth, reads_cfg_config2
         d, exe, shim = ref_paths()
-        # "reference": the unmodified binary built from /root/reference; "port": the oracle restatement, used only
+        # "reference": the unmodified binary (make -C oracle ref); "port": the oracle restatement, used only
         # when that binary did not travel to this box
         self.kind = "reference" if (os.path.exists(exe) and os.path.exists(shim)) else "port"
         self.exe, self.n_proc, self.reads = exe, n_proc, n_proc * reads_per_proc
@@ -435,6 +451,8 @@ def main_b200(a):
     stats = ctx.stats()
     ctx.timing_reset(False)
     check_tables = tables_host.clone()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, check_tables, stats, R)
 
     # ---- end to end through the C ABI with HOST buffers, copies inside the timed region.  Two inputs: the SAM text
     #      `samtools view` would have piped (pssgpu_feed) and the BAM file itself (pssgpu_feed_bam: BGZF inflate + BAM

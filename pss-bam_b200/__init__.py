@@ -39,7 +39,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
     rank ever dlopens a half-written library."""
     import fcntl
     srcs = [os.path.join(CSRC, f) for f in ("pssgpu.cu", "pssgpu_bam.cu", "pssgpu_group.cu", "pssgpu_internal.h", "pss_kernels.cuh", "pss_record.h",
-                                            "pss_inflate.h", "pss_bamrec.h")]
+                                            "pss_inflate.h", "pss_bamrec.h", "pss_crc32.h")]
     srcs.append(os.path.join(ROOT, "include", "pssgpu.h"))
     newest = max(os.path.getmtime(s) for s in srcs)
 

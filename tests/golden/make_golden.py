@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Generate the golden fixtures under tests/golden/ by running the UNMODIFIED reference programs.
 
-Needs oracle/_ref (built by `make -C oracle ref` from /root/reference, only possible where the reference is
-mounted).  Inputs come from the seeded generators in tests/synth plus a hand-written edge-case corpus (the cases
+Needs oracle/_ref (built by `make -C oracle ref REF=<dir>` from the reference's sources, which this repository
+does not carry).  Inputs come from the seeded generators in tests/synth plus a hand-written edge-case corpus (the cases
 SURVEY.md section 8c lists); outputs are whatever the reference binaries print.  Everything written here is
 committed, so the CPU test-suite can pin the oracle on machines without the reference.
 

@@ -4,7 +4,7 @@
 * ``Oracle`` -- ctypes binding of oracle/liboracle.so (CPU restatement of the reference,
   see oracle/oracle_pss.h for who may use it)
 * ``RefBin`` -- runner for the unmodified reference binaries in oracle/_ref (only when
-  they exist; they are built from /root/reference by ``make -C oracle ref``)
+  they exist; they are built from the reference's sources by ``make -C oracle ref REF=<dir>``)
 """
 from __future__ import annotations
 
@@ -478,6 +478,7 @@ def _count_lines(buf) -> int:
 # --------------------------------------------------------------------------- reference binaries
 class RefBin:
     """The unmodified reference programs (oracle/_ref), run with the samtools shim on PATH."""
+    MISSING = "reference programs not built: make -C oracle ref REF=<directory of the unmodified pss-bam sources>"
 
     @staticmethod
     def available() -> bool:

@@ -1,6 +1,6 @@
 """Format contract with the consumers of the two pss-bam tables (SURVEY 4.2 / 8f-4).
 
-`/root/reference/pss-bam-plot.py:37-71` (`get_counts`, `get_rates`) and `pss-bam-gnuplot-template.gp:45-80` are what
+The reference's `pss-bam-plot.py:37-71` (`get_counts`, `get_rates`) and `pss-bam-gnuplot-template.gp:45-80` are what
 reads `<prefix>.pss.counts.txt` / `<prefix>.pss.rates.txt`.  Their parsing is restated here call for call (same pandas
 calls, same arguments -- matplotlib and gnuplot are not in the image, and the plotting itself is out of scope) and run
 over files written by THIS repo's table writers (host/pss_tables.c, no GPU needed) for -r 5 / 15 / 30, and over the

@@ -77,8 +77,13 @@ def test_cli_with_packed_genome_cache(env):
     and a cache of another FASTA of the same basename are all refused and the FASTA is parsed again."""
     import glob
     import shutil
-    d, e = env
+    d0, e = env
     case = MAN["pss"][0]
+    # copies, not the links to tests/golden: the test changes the FASTA's mtime
+    d = os.path.join(d0, "cached")
+    os.makedirs(d, exist_ok=True)
+    for fn in (MAN["fasta"], case["sam"] + ".sam"):
+        shutil.copy(os.path.join(d0, fn), d)
     cdir = os.path.join(d, "cache")
     shutil.rmtree(cdir, ignore_errors=True)
     os.makedirs(cdir)

@@ -116,15 +116,19 @@ def test_full_size_spectrum_vs_oracle(full, k):
         del os.environ["PSSGPU_SPECTRUM_WIDE"]
 
 
+def _spectrum_genome(mb):
+    """A genome as large as the reference's trie walk counts in seconds."""
+    Synth.set_threads(CORES)
+    return Synth.genome(77, [mb * 600_000, mb * 400_000 - 7], n_frac=0.01, lower_frac=0.03)
+
+
 @pytest.mark.parametrize("k,mb", [(8, 48), (12, 8)])
 def test_spectrum_vs_reference_binary(k, mb):
-    """The same two paths against the UNMODIFIED reference program (oracle/_ref/genome-kmer-count-O2, stdout parsed) on
-    a genome as large as its trie walk finishes in seconds; 32- and 64-bit bins; also k = 5 and 13 (the atomics paths)
-    in 64-bit bins against the oracle."""
+    """The same two paths against the UNMODIFIED reference program (oracle/_ref/genome-kmer-count-O2, stdout parsed);
+    32- and 64-bit bins."""
     if not RefBin.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    Synth.set_threads(CORES)
-    g = Synth.genome(77, [mb * 600_000, mb * 400_000 - 7], n_frac=0.01, lower_frac=0.03)
+        pytest.skip(RefBin.MISSING)
+    g = _spectrum_genome(mb)
     d = tmpdir()
     fa = os.path.join(d, "g.fa")
     with open(fa, "wb") as f:
@@ -137,7 +141,24 @@ def test_spectrum_vs_reference_binary(k, mb):
     ctx = pkg.Context(0)
     ctx.upload_genome(list(zip(g.names, g.seqs)))
     assert np.array_equal(ctx.kmer_spectrum(k), want)
+    os.environ["PSSGPU_SPECTRUM_WIDE"] = "1"
+    try:
+        assert np.array_equal(ctx.kmer_spectrum(k), want)
+    finally:
+        del os.environ["PSSGPU_SPECTRUM_WIDE"]
+    ctx.close()
+
+
+@pytest.mark.parametrize("k,mb", [(8, 48), (12, 8)])
+def test_spectrum_wide_bins_vs_oracle(k, mb):
+    """The genomes of test_spectrum_vs_reference_binary against the oracle, which needs no reference binary: k in 32-
+    and 64-bit bins, and k = 5, 9, 13 (the atomics paths) in 64-bit bins."""
+    g = _spectrum_genome(mb)
+    ctx = pkg.Context(0)
+    ctx.upload_genome(list(zip(g.names, g.seqs)))
     ora = Oracle(contigs=list(zip(g.names, g.seqs)))
+    want = oracle_spectrum_parallel(ora, k, CORES)
+    assert np.array_equal(ctx.kmer_spectrum(k), want)
     os.environ["PSSGPU_SPECTRUM_WIDE"] = "1"
     try:
         assert np.array_equal(ctx.kmer_spectrum(k), want)

@@ -1,6 +1,6 @@
-"""Oracle vs the UNMODIFIED reference binaries (oracle/_ref, built from /root/reference by `make -C oracle ref`).
-Runs where those binaries exist (this container; they also travel to the GPU box); elsewhere the committed golden
-fixtures (test_oracle_golden.py) pin the oracle.  Fresh seeded inputs, including malformed lines, byte-compared."""
+"""Oracle vs the UNMODIFIED reference binaries (oracle/_ref, built by `make -C oracle ref REF=<reference sources>`).
+Runs where those binaries exist; elsewhere the committed golden fixtures (test_oracle_golden.py) pin the oracle.
+Fresh seeded inputs, including malformed lines, byte-compared."""
 import os
 import random
 
@@ -10,7 +10,7 @@ import pytest
 from pss_testlib import FkParams, Oracle, PssParams, RefBin, Synth, reads_cfg_config1, reads_cfg_config2, tmpdir
 from test_record_logic import _mutate
 
-pytestmark = pytest.mark.skipif(not RefBin.available(), reason="oracle/_ref not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not RefBin.available(), reason=RefBin.MISSING)
 
 
 @pytest.fixture(scope="module")
