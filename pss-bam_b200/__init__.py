@@ -133,10 +133,7 @@ def load_library():
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("PSSGPU_LIB")          # developer switch: try a differently tuned build of the same ABI
-    if not path:
-        path = build_library()
-    lib = C.CDLL(path)
+    lib = C.CDLL(build_library())
     P = C.c_void_p
     lib.pssgpu_abi_version.restype = C.c_int
     lib.pssgpu_device_count.restype = C.c_int

@@ -1,7 +1,8 @@
 // pss_kernels.cuh -- the sm_100a kernels of the pss-bam hot path.
 //
 //   pack_kernel      K6  ASCII contig -> 4-bit packed genome groups
-//   spectrum_kernel / spectrum_smem_kernel  K5  genome-kmer-count.c:68-79 + kmer.c:43-110 as a flat 4^k histogram
+//   spectrum_kernel / spectrum_smem16_kernel / radix_*_kernel
+//                    K5  genome-kmer-count.c:68-79 + kmer.c:43-110 as a flat 4^k histogram
 //   tally_kernel     K1-K4  SAM text tile -> records -> filters -> genome gather
 //                           -> pss-bam count tables / fragkon end-context histograms
 //
@@ -162,51 +163,17 @@ __global__ void __launch_bounds__(256) spectrum_kernel(const uint64_t *__restric
         }
     }
 }
-// k = 7 .. 9: privatised in shared memory, 32 768 u32 bins (128 KB) per CTA and pass.  4^8 bins take two passes over
-// the packed genome (0.25 ms each from HBM), 4^9 eight; each CTA (slice, pass) counts the k-mers of its slice whose
-// index falls into the pass's bin range with shared-memory atomics and adds its bins to the global table once.  The
-// global-atomic kernel above spends 21 ms on the 3.1 Gb genome at k = 8 (65 536 hot bins in L2, 185 G atomics/s);
-// this one is bound by instruction issue.  The window is turned MSB-first once, so a k-mer index is one shift and
-// one mask (kmer.c:184-214 order).
+// k = 7 .. 9: privatised in shared memory.  The global-atomic kernel above spends 21 ms on the 3.1 Gb genome at k = 8
+// (65 536 hot bins in L2, 185 G atomics/s); counting with shared-memory atomics instead is bound by instruction issue.
+// Each CTA (slice, pass) counts the k-mers of its slice whose index falls into the pass's bin range and adds its bins
+// to the global table once.  The window is turned MSB-first once, so a k-mer index is one shift and one mask
+// (kmer.c:184-214 order).
 constexpr int kSpecSmemLog  = 15;
 constexpr int kSpecSmemBins = 1 << kSpecSmemLog;
 constexpr int kSpecSmemThreads = 1024;
-template <int K, typename CT>
-__global__ void __launch_bounds__(kSpecSmemThreads, 1) spectrum_smem_kernel(const uint64_t *__restrict__ groups, uint64_t g_begin,
-                                                                             uint64_t g_end, uint32_t n_slices, CT *__restrict__ counts)
-{
-    extern __shared__ uint32_t s_bins[];
-    constexpr uint32_t n_bins = 1u << (2 * K);
-    constexpr uint32_t pass_bins = n_bins < (uint32_t)kSpecSmemBins ? n_bins : (uint32_t)kSpecSmemBins;
-    constexpr uint64_t kmask = n_bins - 1u;
-    const uint32_t slice = blockIdx.x % n_slices, pass = blockIdx.x / n_slices;
-    for (uint32_t i = threadIdx.x; i < pass_bins; i += kSpecSmemThreads) s_bins[i] = 0;
-    __syncthreads();
-    const uint64_t n = g_end - g_begin;
-    const uint64_t lo = g_begin + n * slice / n_slices, hi = g_begin + n * (slice + 1) / n_slices;
-    for (uint64_t gi = lo + threadIdx.x; gi < hi; gi += kSpecSmemThreads) {
-        const uint64_t g0 = __ldg(groups + gi), g1 = __ldg(groups + gi + 1);
-        const uint64_t codes = (uint64_t)(uint32_t)g0 | ((uint64_t)(uint32_t)g1 << 32);
-        const uint64_t cls = (g0 >> 32) | (g1 & 0xffffffff00000000ull);
-        const uint64_t bad = (cls | (cls >> 1)) & kEvenBits;
-        if ((uint32_t)bad == 0x55555555u) continue;          // whole group invalid (padding / N run)
-        const uint64_t msb = rev_fields64(codes, 32);        // base j of the window at field 31 - j
-#pragma unroll
-        for (int o = 0; o < 16; o++) {
-            if (((bad >> (2 * o)) & kmask) != 0) continue;
-            const uint32_t idx = (uint32_t)(msb >> (2 * (32 - o - K))) & (uint32_t)kmask;
-            if ((idx >> kSpecSmemLog) == pass) atomicAdd(&s_bins[idx & (uint32_t)(kSpecSmemBins - 1)], 1u);
-        }
-    }
-    __syncthreads();
-    for (uint32_t i = threadIdx.x; i < pass_bins; i += kSpecSmemThreads) {
-        const uint32_t v = s_bins[i];
-        if (v) atomicAdd(counts + ((size_t)pass << kSpecSmemLog) + i, (CT)v);
-    }
-}
-// k = 7 .. 9, second generation: 65 536 bins per pass in the same 128 KB, as 16-bit counters packed two to a word
-// -- bin b lives in half (b >> 15) & 1 of word b & 0x7fff -- so 4^8 bins take ONE pass over the packed genome instead of
-// two (4^9: four instead of eight), and the per-k-mer code has no pass test.  A 16-bit counter cannot hold a hot bin
+// 65 536 bins per pass in 128 KB of shared memory, as 16-bit counters packed two to a word -- bin b lives in half
+// (b >> 15) & 1 of word b & 0x7fff -- so 4^8 bins take ONE pass over the packed genome (0.25 ms from HBM), with no pass
+// test in the per-k-mer code, and 4^9 take four.  A 16-bit counter cannot hold a hot bin
 // (poly-A: 10^8 hits), so it is drained on the fly, exactly: an increment is a 32-bit shared-memory atomic add of 1 or
 // 0x10000 that returns the old word; the old words of a group's 16 increments are OR-ed and looked at once -- if some
 // half had reached 0x8000, the thread clears that bit with an atomicAnd and, if it was the one that cleared it, adds
@@ -499,26 +466,12 @@ __global__ void __launch_bounds__(256) widen_kernel(const unsigned int *__restri
 // ===========================================================================
 // K1-K4  SAM tile scan + per-record tally
 // ===========================================================================
-// tuning knobs (defaults = the measured best; other values are only used by tuning builds)
-#ifndef PSS_TALLY_CTAS_PER_SM
-#define PSS_TALLY_CTAS_PER_SM 2
-#endif
-#ifndef PSS_TALLY_THREADS
-#define PSS_TALLY_THREADS 256
-#endif
-#ifndef PSS_TALLY_ITERS
-#define PSS_TALLY_ITERS 4
-#endif
-#ifndef PSS_TALLY_PREFETCH
-#define PSS_TALLY_PREFETCH 1                                  // L2 prefetch of the next tile while the records of this one are processed
-#endif
-constexpr int kThreads    = PSS_TALLY_THREADS;                // threads per CTA = records a CTA takes per tile
+// measured best: 2 CTAs of 256 threads per SM, 4 scan steps per tile
+constexpr int kCtasPerSm  = 2;
+constexpr int kThreads    = 256;                              // threads per CTA = records a CTA takes per tile
 constexpr int kWarps      = kThreads / 32;
-#ifndef PSS_TALLY_SLOTS
-#define PSS_TALLY_SLOTS (PSS_TALLY_ITERS * PSS_TALLY_THREADS)
-#endif
-constexpr int kSlots      = PSS_TALLY_SLOTS;                  // 64-byte slots (two 32-byte chunks) of one tile; whole warps
-constexpr int kIters      = (kSlots + kThreads - 1) / kThreads;   // steps of the scan (the last one may leave warps out)
+constexpr int kIters      = 4;                                // steps of the scan
+constexpr int kSlots      = kIters * kThreads;                // 64-byte slots (two 32-byte chunks) of one tile
 constexpr int kChunks     = 2 * kSlots;                       // chunks = mask words of one tile
 constexpr int kSpan       = kChunks * 32;                     // bytes of staged text
 constexpr int kPrefix     = 16;                               // the bulk copy lands at bytes + kPrefix; the byte before the first
@@ -847,9 +800,6 @@ __device__ __forceinline__ uint32_t ballot_bits(uint32_t word, uint32_t mask)
 // Rows 16 and 17 (-r 15 has 17 rows) still go the ballot way: lane l owns cell (l & 15) of table (l >> 4).
 // All 32 lanes must be converged.
 // ---------------------------------------------------------------------------
-#ifndef PSS_TALLY_TRANSPOSE
-#define PSS_TALLY_TRANSPOSE 1
-#endif
 struct XposeConsts {
     uint32_t sel16, sel8, s4, s2, s1, r4, r2, r1;
 };
@@ -900,7 +850,6 @@ template <int NACC, int ROWS>
 __device__ __forceinline__ void tally_rows(const PssStreams &st, uint32_t (&acc)[NACC ? NACC : 1], int rows, uint32_t lane, uint32_t one)
 {
     static_assert(NACC == 0 || NACC == 9 || NACC == 16, "9: rows 0..15 transposed + rows 16, 17 by ballots; 16: two transposed sets");
-#if PSS_TALLY_TRANSPOSE
     constexpr uint32_t E = 0x55555555u;
     const XposeConsts xc = xpose_consts(lane);
     {
@@ -919,9 +868,6 @@ __device__ __forceinline__ void tally_rows(const PssStreams &st, uint32_t (&acc)
         return;
     }
     constexpr int kFirstBallotRow = 16;
-#else
-    constexpr int kFirstBallotRow = 0;
-#endif
     const uint32_t tbi = lane >> 4;                           // which table this lane counts for
     const uint32_t neg1 = 0u - one;
     const uint32_t cell = lane & 15u;
@@ -953,7 +899,6 @@ __device__ __forceinline__ void tally_rows(const PssStreams &st, uint32_t (&acc)
 template <int NACC>
 __device__ __forceinline__ void flush_acc(uint32_t (&acc)[NACC ? NACC : 1], int rows, uint32_t lane, uint32_t *table)
 {
-#if PSS_TALLY_TRANSPOSE
     {
         const uint32_t tb = lane & 1u, row = lane >> 1;
 #pragma unroll
@@ -967,9 +912,6 @@ __device__ __forceinline__ void flush_acc(uint32_t (&acc)[NACC ? NACC : 1], int 
         }
     }
     constexpr int kFirstBallotRow = NACC == 16 ? 32 : 16;
-#else
-    constexpr int kFirstBallotRow = 0;
-#endif
     const uint32_t tb = lane >> 4, cell = lane & 15u;
 #pragma unroll
     for (int j = kFirstBallotRow; j < 2 * NACC; j++) {
@@ -1184,7 +1126,7 @@ __device__ __forceinline__ void process_batch(const TallyArgs &A, TallyShared &T
 // 0 = any -r, through pss_record_wide() and global atomics (exact, not tuned).  ROWS = R + 2 as a compile-time
 // constant for the default -r 15 (the ballot loop then has no per-row exit test), 0 = taken from the arguments
 template <int MODE, int NACC, int ROWS>
-__global__ void __launch_bounds__(kThreads, PSS_TALLY_CTAS_PER_SM) tally_kernel(const __grid_constant__ TallyArgs A)
+__global__ void __launch_bounds__(kThreads, kCtasPerSm) tally_kernel(const __grid_constant__ TallyArgs A)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     TallySmem &S = *reinterpret_cast<TallySmem *>(smem_raw);
@@ -1268,7 +1210,7 @@ __global__ void __launch_bounds__(kThreads, PSS_TALLY_CTAS_PER_SM) tally_kernel(
 #pragma unroll
             for (int it = 0; it < kIters; it++) {
                 pk[it] = kNoNl;
-                if (it * 2 * kThreads < n_valid + 8 && ((it + 1) * kThreads <= kSlots || it * kThreads + (int)tid < kSlots)) {   // block- / warp-uniform
+                if (it * 2 * kThreads < n_valid + 8) {                        // block uniform
                     const int      c = 2 * (it * kThreads + (int)tid);           // this thread's two chunks: c, c + 1
                     const uint8_t *src = S.bytes + 32 * c;
                     // the four 16-byte quads of the slot are loaded in the order 0^r, 1^r, 2^r, 3^r, r = (lane / 2) % 4:
@@ -1355,7 +1297,7 @@ __global__ void __launch_bounds__(kThreads, PSS_TALLY_CTAS_PER_SM) tally_kernel(
                 const float per = (float)used / (float)n_take;
                 int e2 = (int)(per * (float)kThreads * 1.03f) + 768;
                 est = e2 > kStageMax ? kStageMax : e2;
-                if (PSS_TALLY_PREFETCH && tid == 0 && next < range_end) {
+                if (tid == 0 && next < range_end) {          // L2 prefetch of the next tile while the records of this one are processed
                     const uint64_t nsrc = (next - 1) & ~15ull;
                     const uint64_t nleft = len16 - nsrc;
                     const uint32_t nbytes = nleft < (uint64_t)est ? (uint32_t)nleft : (uint32_t)(est & ~15);
@@ -1388,260 +1330,6 @@ __global__ void __launch_bounds__(kThreads, PSS_TALLY_CTAS_PER_SM) tally_kernel(
     cta_epilogue<MODE>(S.sh, A, tid, kThreads, rows);
 }
 
-// ---------------------------------------------------------------------------
-// tally kernel, warp-autonomous variant ("warp tiles").
-//
-// Same work, same per-record code (process_batch), different choreography: every WARP owns its own tile of exactly 32
-// records -- its own stretch of shared memory, its own mbarrier, its own bulk copy -- and walks its own ranges of the
-// text.  There is no block-wide barrier in the steady state: the CTA kernel above marches all eight warps of a CTA
-// through stage / scan / rank / records in lock step (four __syncthreads per tile; ncu: 0.85 barrier stalls per issue,
-// 60 % of the issue slots used), and at any moment all of them want the same pipe -- the scan is FMA+ALU balanced, the
-// record phase ALU heavy.  Sixteen independent warps per SM are in sixteen different phases: copies, scans and record
-// code of different warps overlap, and the ALU pipe sees a steadier mix.
-//   stage     lane 0: one cp.async.bulk of the bytes 32 records are expected to take, on the warp's mbarrier
-//   pass A    a 64-byte slot per lane and step, as above; the ballots of the steps stay in registers
-//   pass B    ordinals = prefix of the ballots' popcounts (warp uniform registers), positions 0..32 to shared memory
-//   records   one lane per record
-// ---------------------------------------------------------------------------
-#ifndef PSS_WTILE_SLOTS
-#define PSS_WTILE_SLOTS 160                                   // 64-byte slots of a warp tile: 10 KB, 32 records of up to 320 bytes
-#endif
-constexpr int kWSlots    = PSS_WTILE_SLOTS;
-constexpr int kWIters    = (kWSlots + 31) / 32;
-constexpr int kWChunks   = 2 * kWSlots;
-constexpr int kWSpan     = kWChunks * 32;
-constexpr int kWStageMax = kWSpan - 80;
-static_assert(kWSlots % 32 == 0, "whole warp steps");
-
-struct WarpTile {
-    alignas(128) uint8_t bytes[kWSpan + 32];
-    alignas(8) uint32_t le[kWChunks + 8];
-    uint32_t nlpos[36];
-    alignas(8) uint64_t bar;
-};
-struct TallyWarpSmem {
-    WarpTile    w[kWarps];
-    TallyShared sh;
-};
-
-// exact newline listing of a warp tile (two candidates in one slot, or a false candidate): every lane walks its own
-// run of consecutive chunks.  Returns the number of newlines; positions of ordinals 0..32 go to nlpos.
-__device__ __noinline__ uint32_t wlist_newlines_generic(WarpTile *Wp, int n_valid, uint32_t one)
-{
-    WarpTile      &W = *Wp;
-    const uint32_t lane = threadIdx.x & 31u, full = 0xffffffffu;
-    const int      per = (n_valid + 31) / 32, c0 = (int)lane * per;
-    uint32_t       sum = 0;
-    for (int k = 0; k < per; k++) {
-        if (c0 + k >= n_valid) break;
-        uint32_t le32, nl32;
-        classify32(W.bytes + 32 * (c0 + k), one, le32, nl32);
-        sum += (uint32_t)__popc(nl32);
-    }
-    uint32_t inc = sum;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t t = __shfl_up_sync(full, inc, d);
-        if ((int)lane >= d) inc += t;
-    }
-    const uint32_t total = __shfl_sync(full, inc, 31);
-    uint32_t ord = inc - sum;
-    for (int k = 0; k < per; k++) {
-        if (c0 + k >= n_valid) break;
-        uint32_t le32, nl32;
-        classify32(W.bytes + 32 * (c0 + k), one, le32, nl32);
-        while (nl32) {
-            if (ord <= 32u) W.nlpos[ord] = (uint32_t)((c0 + k) * 32 + __ffs((int)nl32) - 1);
-            nl32 &= nl32 - 1u;
-            ord++;
-        }
-    }
-    return total;
-}
-
-template <int MODE, int NACC, int ROWS>
-__global__ void __launch_bounds__(kThreads, PSS_TALLY_CTAS_PER_SM) tally_warp_kernel(const __grid_constant__ TallyArgs A)
-{
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    TallyWarpSmem &S = *reinterpret_cast<TallyWarpSmem *>(smem_raw);
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    const uint32_t full = 0xffffffffu;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-    WarpTile      &W = S.w[warp];
-
-    if (lane < 8) W.le[kWChunks + lane] = ~0u;
-    if (lane < kPrefix) W.bytes[lane] = 'x';
-    if (lane == 0) { mbar_init(&W.bar, 1); fence_mbar_init(); }
-    cta_prologue(S.sh, A, tid, kThreads);                     // (ends with a __syncthreads: the only one before the epilogue)
-
-    const int      rows = A.cfg.R + 2;
-    const uint32_t one = A.one;
-    uint32_t       phase = 0;
-    uint32_t       acc[NACC ? NACC : 1];
-    int            acc_iters = 0;
-    uint32_t       st_acc = 0, st_acc_fk = 0;
-#pragma unroll
-    for (int i = 0; i < (NACC ? NACC : 1); i++) acc[i] = 0;
-    const uint64_t text_len = A.len_dev ? (uint64_t)__ldg(A.len_dev) : A.len;
-    const uint64_t len16 = (text_len + 15) & ~15ull;
-    int            est = kWStageMax;
-
-    for (;;) {
-        // ---- next range of this warp ----
-        uint32_t r = 0;
-        if (lane == 0) r = atomicAdd(A.range_ctr, 1u);
-        r = __shfl_sync(full, r, 0);
-        const uint64_t range_begin = (uint64_t)r * A.range_bytes;
-        if (range_begin >= text_len) break;
-        const uint64_t range_end = (range_begin + A.range_bytes < text_len) ? range_begin + A.range_bytes : text_len;
-        uint64_t       pos = range_begin;
-        bool           want_full = false;
-
-        while (pos < range_end) {
-            // ---- stage ----
-            const uint64_t gsrc = pos ? ((pos - 1) & ~15ull) : 0;
-            const int64_t  gbase = (int64_t)gsrc - kPrefix;
-            const int      head = (int)((int64_t)pos - 1 - gbase);
-            int            want = want_full ? kWStageMax : est;
-            want = (want + 16) & ~63; want -= 16;
-            if (want > kWStageMax) want = kWStageMax;
-            const uint64_t left = len16 - gsrc;
-            const bool     sees_end = left <= (uint64_t)want;
-            const int      nb = sees_end ? (int)left : want;
-            const bool     is_full = sees_end || want >= kWStageMax;
-            const int      data_end = sees_end ? (int)((int64_t)text_len - gbase) : kPrefix + nb;
-            __syncwarp();                                     // every lane is done with the previous tile
-            if (lane == 0) {
-                fence_proxy_async();
-                mbar_expect_tx(&W.bar, (uint32_t)nb);
-                bulk_g2s(W.bytes + kPrefix, A.sam + gsrc, (uint32_t)nb, &W.bar);
-            }
-            mbar_wait(&W.bar, phase);
-            phase ^= 1u;
-
-            const int tail_slot = data_end >> 6;
-            const int n_valid = 2 * (sees_end ? tail_slot + 1 : tail_slot);
-            if (lane == 0) {
-                W.bytes[kPrefix - 1] = pos == 0 ? '\n' : 'x';
-                for (int i = kPrefix; i < head; i++) W.bytes[i] = 'x';
-            }
-            if (sees_end && lane == (uint32_t)(tail_slot & 31)) {
-                W.bytes[data_end] = '\n';
-                for (int i = data_end + 1; i < 64 * (tail_slot + 1); i++) W.bytes[i] = 'x';
-            }
-            __syncwarp();
-
-            // ---- pass A ----
-            constexpr uint32_t kNoNl = 0xfffffu;
-            uint32_t pk[kWIters], bal[kWIters];
-            uint32_t redo = 0;
-            const uint32_t r4 = (lane >> 1) & 3u;
-            const uint32_t qo0 = 16u * r4, qo1 = 16u * (1u ^ r4), qo2 = 16u * (2u ^ r4), qo3 = 16u * (3u ^ r4);
-            const uint32_t rot16 = 16u * (r4 & 1u), hi_x = r4 >> 1, swz = 16u * r4;
-#pragma unroll
-            for (int it = 0; it < kWIters; it++) {
-                pk[it] = kNoNl;
-                bal[it] = 0u;
-                if (it * 64 < n_valid + 8) {                  // warp uniform
-                    const int      c = 2 * (it * 32 + (int)lane);
-                    const uint8_t *src = W.bytes + 32 * c;
-                    const uint4    q0 = *reinterpret_cast<const uint4 *>(src + qo0), q1 = *reinterpret_cast<const uint4 *>(src + qo1);
-                    const uint4    q2 = *reinterpret_cast<const uint4 *>(src + qo2), q3 = *reinterpret_cast<const uint4 *>(src + qo3);
-                    uint32_t le_x, nc_x, le_y, nc_y;
-                    classify32_fast(q0, q1, one, le_x, nc_x);
-                    classify32_fast(q2, q3, one, le_y, nc_y);
-                    le_x = __funnelshift_l(le_x, le_x, rot16);
-                    le_y = __funnelshift_l(le_y, le_y, rot16);
-                    W.le[c + (int)hi_x] = le_x;
-                    W.le[c + 1 - (int)hi_x] = le_y;
-                    const bool     has = (nc_x | nc_y) != 0u && c < n_valid;
-                    const uint32_t b = __ballot_sync(full, has);
-                    const uint32_t rank = (uint32_t)__popc(b & lt_mask);
-                    const uint32_t x = nc_x ? nc_x : nc_y;
-                    const uint32_t p = (uint32_t)(32 * c) + ((((nc_x ? 0u : 32u) + (uint32_t)__ffs((int)x) - 1u) ^ swz) & 63u);
-                    redo |= has ? ((x & (x - 1u)) | (nc_x ? nc_y : 0u) | ((uint32_t)W.bytes[has ? p : 0u] ^ 0x0au)) : 0u;
-                    pk[it] = has ? (p + (rank << 20)) : kNoNl;
-                    bal[it] = b;
-                }
-            }
-            const bool any_multi = __any_sync(full, redo != 0u);
-            __syncwarp();
-            if (lane < 8) W.le[n_valid + (int)lane] = ~0u;    // sentinels (the words they overwrite belong to slots past the text)
-
-            // ---- pass B ----
-            uint32_t n_nl;
-            if (!any_multi) {
-                uint32_t base = 0;
-#pragma unroll
-                for (int it = 0; it < kWIters; it++) {
-                    const uint32_t v = pk[it];
-                    const uint32_t ord = base + (v >> 20);
-                    if (v != kNoNl && ord <= 32u) W.nlpos[ord] = v & 0xfffffu;
-                    base += (uint32_t)__popc(bal[it]);
-                }
-                n_nl = base;
-            } else {
-                n_nl = wlist_newlines_generic(&W, n_valid, one);
-            }
-            __syncwarp();
-
-            const int n_take = (int)n_nl - 1 < 32 ? (int)n_nl - 1 : 32;
-
-            // ---- where the next tile begins ----
-            uint64_t next;
-            bool     next_full = false;
-            if (n_nl == 0) {
-                next = (uint64_t)(gbase + data_end);
-            } else if (n_take <= 0) {
-                const uint64_t first = (uint64_t)(gbase + (int)W.nlpos[0] + 1);
-                if (first > pos || !is_full) {
-                    next = first; next_full = true;
-                } else {                                       // a record longer than a warp tile
-                    unsigned long long e = first;
-                    if (lane == 0 && first < range_end) e = long_record<MODE>(&A, &S.sh, first, text_len);
-                    e = __shfl_sync(full, e, 0);
-                    next = first < range_end ? (uint64_t)e : range_end;
-                }
-            } else {
-                const int used = (int)W.nlpos[n_take] - (int)W.nlpos[0];
-                next = (uint64_t)(gbase + (int)W.nlpos[n_take] + 1);
-                const float per = (float)used / (float)n_take;
-                int e2 = (int)(per * 32.0f * 1.04f) + 192;
-                est = e2 > kWStageMax ? kWStageMax : e2;
-                if (PSS_TALLY_PREFETCH && lane == 0 && next < range_end) {
-                    const uint64_t nsrc = (next - 1) & ~15ull;
-                    const uint64_t nleft = len16 - nsrc;
-                    const uint32_t nbytes = nleft < (uint64_t)est ? (uint32_t)nleft : (uint32_t)(est & ~15);
-                    bulk_prefetch_l2(A.sam + nsrc, nbytes);
-                }
-            }
-            // ---- records ----
-            {
-                const bool     in = (int)lane < n_take;
-                const int      start = in ? (int)W.nlpos[lane] + 1 : kPrefix;
-                const int      pe = in ? (int)W.nlpos[lane + 1] : kPrefix;
-                const uint64_t goff = (uint64_t)(gbase + start);
-                const bool     has = in && start < data_end && goff < range_end;
-                if (__any_sync(full, has))
-                    process_batch<MODE, NACC, ROWS>(A, S.sh, W.bytes, W.le, has, start, pe, goff, lane, acc, acc_iters, rows, st_acc, st_acc_fk);
-            }
-            want_full = next_full;
-            pos = next;
-        }
-    }
-
-    if (MODE != kModeFragkon && NACC > 0) flush_acc<NACC>(acc, rows, lane, S.sh.table);
-    if (lane < (uint32_t)kStN) {
-        if (st_acc) atomicAdd(&S.sh.stats[lane], st_acc);
-        if (MODE == kModeBoth && st_acc_fk) atomicAdd(&S.sh.stats_fk[lane], st_acc_fk);
-    }
-    __syncthreads();
-    cta_epilogue<MODE>(S.sh, A, tid, kThreads, rows);
-}
-#if PSS_TALLY_THREADS == 256      // (tuning builds with other CTA sizes do not use the warp-tile variant)
-static_assert(sizeof(TallyWarpSmem) + 1024 <= 232448 / PSS_TALLY_CTAS_PER_SM, "the CTAs of the warp-tile kernel must fit one SM");
-#endif
-
-static_assert(sizeof(TallySmem) + 1024 <= 232448 / PSS_TALLY_CTAS_PER_SM, "the CTAs of the tally kernel must fit one SM");
+static_assert(sizeof(TallySmem) + 1024 <= 232448 / kCtasPerSm, "the CTAs of the tally kernel must fit one SM");
 
 }  // namespace pssgpu

@@ -17,7 +17,6 @@
 using namespace pssgpu;
 
 namespace {
-constexpr bool   kTallyWarpDefault = false;      // PSSGPU_TALLY_KERNEL=warp|cta overrides
 constexpr size_t kPackPiece   = 128ull << 20;    // ASCII bases per pack launch when uploading from the host
 constexpr uint64_t kExcCap    = 4ull << 20;      // logged "other" symbols (beyond: -U/-D with such bytes unsupported)
 thread_local std::string g_init_error;
@@ -309,9 +308,9 @@ int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t str
     a.dbg_cap = ctx->dbg_cap;
     const int      max_grid = MODE == kModeFragkon ? ctx->tally_grid_fk : ctx->tally_grid_pss;
     // ranges handed out by an atomic counter: about eight per CTA on large inputs, never below 128 KiB
-    uint64_t rb = len / ((uint64_t)max_grid * (ctx->tally_warp ? 8u * (uint64_t)kWarps : 8u));      // (the warp variant deals ranges to warps)
+    uint64_t rb = len / ((uint64_t)max_grid * 8u);
     if (const char *e = getenv("PSSGPU_RANGE_KB")) rb = std::max<uint64_t>(1, strtoull(e, nullptr, 10)) << 10;   // developer / test switch
-    else rb = std::min<uint64_t>(std::max<uint64_t>(rb, ctx->tally_warp ? (32u << 10) : (128u << 10)), 1u << 20);
+    else rb = std::min<uint64_t>(std::max<uint64_t>(rb, 128u << 10), 1u << 20);
     rb = (rb + 31) & ~31ull;
     const uint64_t n_ranges = (len + rb - 1) / rb;
     a.range_bytes = rb;
@@ -319,19 +318,14 @@ int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t str
     a.one = 1u;
     CU(cudaMemsetAsync(ctx->d_range_ctr, 0, sizeof(unsigned int), ctx->stream));
     time_begin(ctx, len);
-    const unsigned grid = (unsigned)std::min<uint64_t>(ctx->tally_warp ? (n_ranges + kWarps - 1) / kWarps : n_ranges, (uint64_t)max_grid);
+    const unsigned grid = (unsigned)std::min<uint64_t>(n_ranges, (uint64_t)max_grid);
     constexpr int PM = MODE == kModeFragkon ? kModePss : MODE;          // (never launched with MODE == kModeFragkon)
-#define PSS_LAUNCH(KERNEL, SMEM)                                                                                          \
-    do {                                                                                                                 \
-        if (MODE == kModeFragkon) KERNEL<kModeFragkon, 9, 0><<<grid, kThreads, SMEM, ctx->stream>>>(a);                  \
-        else if (ctx->cfg.R == 15) KERNEL<PM, 9, 17><<<grid, kThreads, SMEM, ctx->stream>>>(a);     /* the default -r */   \
-        else if (ctx->cfg.R + 2 <= 18) KERNEL<PM, 9, 0><<<grid, kThreads, SMEM, ctx->stream>>>(a);                       \
-        else if (ctx->cfg.R <= kMaxRegion) KERNEL<PM, 16, 0><<<grid, kThreads, SMEM, ctx->stream>>>(a);                  \
-        else KERNEL<PM, 0, 0><<<grid, kThreads, SMEM, ctx->stream>>>(a);   /* any -r: exact, not tuned */                \
-    } while (0)
-    if (ctx->tally_warp) PSS_LAUNCH(tally_warp_kernel, sizeof(TallyWarpSmem));
-    else PSS_LAUNCH(tally_kernel, sizeof(TallySmem));
-#undef PSS_LAUNCH
+    constexpr size_t smem = sizeof(TallySmem);
+    if (MODE == kModeFragkon) tally_kernel<kModeFragkon, 9, 0><<<grid, kThreads, smem, ctx->stream>>>(a);
+    else if (ctx->cfg.R == 15) tally_kernel<PM, 9, 17><<<grid, kThreads, smem, ctx->stream>>>(a);         // the default -r
+    else if (ctx->cfg.R + 2 <= 18) tally_kernel<PM, 9, 0><<<grid, kThreads, smem, ctx->stream>>>(a);
+    else if (ctx->cfg.R <= kMaxRegion) tally_kernel<PM, 16, 0><<<grid, kThreads, smem, ctx->stream>>>(a);
+    else tally_kernel<PM, 0, 0><<<grid, kThreads, smem, ctx->stream>>>(a);                                // any -r: exact, not tuned
     time_end(ctx);
     CU(cudaGetLastError());
     return PSSGPU_OK;
@@ -407,24 +401,10 @@ int pssgpu_init(int device, pssgpu_ctx **out)
             (const void *)tally_kernel<kModeBoth, 9, 0>, (const void *)tally_kernel<kModeBoth, 16, 0>, (const void *)tally_kernel<kModeBoth, 0, 0> };
         for (const void *k : kernels)
             if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TallySmem));
-        const void *wkernels[] = {
-            (const void *)tally_warp_kernel<kModePss, 9, 17>, (const void *)tally_warp_kernel<kModePss, 9, 0>, (const void *)tally_warp_kernel<kModePss, 16, 0>,
-            (const void *)tally_warp_kernel<kModePss, 0, 0>, (const void *)tally_warp_kernel<kModeFragkon, 9, 0>, (const void *)tally_warp_kernel<kModeBoth, 9, 17>,
-            (const void *)tally_warp_kernel<kModeBoth, 9, 0>, (const void *)tally_warp_kernel<kModeBoth, 16, 0>, (const void *)tally_warp_kernel<kModeBoth, 0, 0> };
-        for (const void *k : wkernels)
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TallyWarpSmem));
-        // which choreography: "warp" = every warp walks its own 32-record tiles (no block barriers), "cta" = 256-record tiles
-        const char *tk = getenv("PSSGPU_TALLY_KERNEL");
-        c->tally_warp = tk ? strcmp(tk, "warp") == 0 : kTallyWarpDefault;
     }
     int occ_p = 0, occ_f = 0;
-    if (c->tally_warp) {
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, tally_warp_kernel<kModePss, 16, 0>, kThreads, sizeof(TallyWarpSmem));
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_f, tally_warp_kernel<kModeFragkon, 9, 0>, kThreads, sizeof(TallyWarpSmem));
-    } else {
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, tally_kernel<kModePss, 16, 0>, kThreads, sizeof(TallySmem));
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_f, tally_kernel<kModeFragkon, 9, 0>, kThreads, sizeof(TallySmem));
-    }
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, tally_kernel<kModePss, 16, 0>, kThreads, sizeof(TallySmem));
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_f, tally_kernel<kModeFragkon, 9, 0>, kThreads, sizeof(TallySmem));
     if (e != cudaSuccess || occ_p < 1 || occ_f < 1) {
         fail(nullptr, PSSGPU_ECUDA, "pssgpu_init: %s (occupancy %d/%d)", cudaGetErrorString(e), occ_p, occ_f);
         if (c->stream) cudaStreamDestroy(c->stream);
@@ -1019,7 +999,7 @@ int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_s
     uint16_t *d_payload = nullptr;
     unsigned long long *d_rad = nullptr;                   // bucket counts | offsets (nb + 1) | cursors
     const uint32_t rad_nb = (k >= 10 && k <= 12) ? (1u << (2 * k - kSpecSmemLog)) : 0u;
-    if (rad_nb && g1 > g0 && !getenv("PSSGPU_SPECTRUM_ATOMICS")) {
+    if (rad_nb && g1 > g0) {
         if (cudaMalloc(&d_payload, (g1 - g0) * 16 * sizeof(uint16_t) + 64) != cudaSuccess) { cudaGetLastError(); d_payload = nullptr; }
         else if (cudaMalloc(&d_rad, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long)) != cudaSuccess) {
             cudaGetLastError(); cudaFree(d_payload); d_payload = nullptr; d_rad = nullptr;
@@ -1047,7 +1027,7 @@ int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_s
             cudaFuncSetAttribute(radix_hist_kernel<unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
             radix_hist_kernel<unsigned long long><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream>>>(d_payload, off, parts, (unsigned long long *)d_counts);
         }
-    } else if (g1 > g0 && k >= 7 && k <= 9 && !getenv("PSSGPU_SPECTRUM_SMEM32")) {
+    } else if (g1 > g0 && k >= 7 && k <= 9) {
         // shared-memory bins, 16-bit counters packed two to a word: 65 536 bins per CTA -- one pass for 4^8 bins, four for 4^9
         const uint32_t n_slices = (uint32_t)std::min<uint64_t>((uint64_t)ctx->sm_count, (g1 - g0 + kSpecSmemThreads - 1) / kSpecSmemThreads);
         const uint32_t passes = (uint32_t)std::max<size_t>(1, bins >> kSpec16Log);
@@ -1065,23 +1045,6 @@ int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_s
             if (k == 7) PSS_SPEC16(7, unsigned long long, w); else if (k == 8) PSS_SPEC16(8, unsigned long long, w); else PSS_SPEC16(9, unsigned long long, w);
         }
 #undef PSS_SPEC16
-    } else if (g1 > g0 && k >= 7 && k <= 9) {    // the first generation (32-bit bins, two passes for 4^8): kept behind PSSGPU_SPECTRUM_SMEM32 for comparison
-        const uint32_t n_slices = (uint32_t)std::min<uint64_t>((uint64_t)ctx->sm_count, (g1 - g0 + kSpecSmemThreads - 1) / kSpecSmemThreads);
-        const uint32_t passes = (uint32_t)std::max<size_t>(1, bins >> kSpecSmemLog);
-        const size_t   smem = std::min<size_t>(bins, kSpecSmemBins) * sizeof(uint32_t);
-        const dim3     sg(n_slices * passes);
-#define PSS_SPEC(K_, CT_, PTR_)                                                                                        \
-        do {                                                                                                           \
-            cudaFuncSetAttribute(spectrum_smem_kernel<K_, CT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-            spectrum_smem_kernel<K_, CT_><<<sg, kSpecSmemThreads, smem, ctx->stream>>>(ctx->d_groups, g0, g1, n_slices, PTR_); \
-        } while (0)
-        if (narrow) {
-            if (k == 7) PSS_SPEC(7, unsigned int, d_narrow); else if (k == 8) PSS_SPEC(8, unsigned int, d_narrow); else PSS_SPEC(9, unsigned int, d_narrow);
-        } else {
-            unsigned long long *w = (unsigned long long *)d_counts;
-            if (k == 7) PSS_SPEC(7, unsigned long long, w); else if (k == 8) PSS_SPEC(8, unsigned long long, w); else PSS_SPEC(9, unsigned long long, w);
-        }
-#undef PSS_SPEC
     } else if (g1 > g0) {
         if (narrow) {
             if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned int><<<grid, 256, 0, ctx->stream>>>(ctx->d_groups, g0, g1, k, d_narrow);

@@ -43,10 +43,7 @@ constexpr uint32_t kBamLocCap    = 2048;          // record starts per block: 65
 constexpr uint32_t kBamMaxRefs   = 1u << 21;
 constexpr uint32_t kBamNone      = 0xffffffffu;
 constexpr int      kBamSlots     = 8;             // batches the host may be ahead of the framing GPU when several GPUs inflate
-#ifndef PSS_INF_WARPS
-#define PSS_INF_WARPS 10
-#endif
-constexpr int      kInfWarps     = PSS_INF_WARPS; // warps per CTA of the inflate kernel: 7.3 KB of tables each, three CTAs per SM
+constexpr int      kInfWarps     = 10;            // warps per CTA of the inflate kernel: 7.3 KB of tables each, three CTAs per SM
 
 enum : unsigned {
     kBamOk = 0, kBamErrInflate = 100 /* + pss_inflate.h code */, kBamErrMagic = 200, kBamErrHeaderTooLarge, kBamErrTooManyRefs,
@@ -95,7 +92,7 @@ struct BamIngest {
     uint32_t *d_crc_tab = nullptr;    // pss_crc32.h tables; null when $PSSGPU_BAM_CRC=0 switches the check off
     bool      check_crc = true;
     int       rg_len = -1;
-    int       inflate_grid = 0, inflate_minb = 3;
+    int       inflate_grid = 0;
     uint64_t  batches = 0;
     // several GPUs (pssgpu_group_feed_bam): this context frames, renders and tallies; `helpers` inflate batches for it
     std::vector<pssgpu_ctx *> helpers;
@@ -120,9 +117,8 @@ __global__ void bam_merge_error_kernel(BamState *st, const unsigned int *remote)
     if (remote[0]) bam_fail(st, remote[0], remote[1]);
 }
 
-// MINB = CTAs per SM the register allocation aims at: 3 (30 warps at the default 10 warps per CTA, 64 registers) or 2
-template <int MINB>
-__global__ void __launch_bounds__(kInfWarps * 32, MINB)
+// the register allocation aims at three CTAs per SM (30 warps, 64 registers): the measured best
+__global__ void __launch_bounds__(kInfWarps * 32, 3)
 bgzf_inflate_kernel(const BamDesc *__restrict__ desc, uint32_t n_blocks, const uint8_t *__restrict__ comp, uint8_t *udata, BamState *st,
                     const uint32_t *__restrict__ crc_tab)
 {
@@ -564,12 +560,9 @@ int bam_ensure(pssgpu_ctx *ctx, bool inflate_only = false)
             CU(cudaMemcpy(B->d_crc_tab, tab.data(), tab.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
         }
         const size_t smem = (size_t)kInfWarps * sizeof(InflateTables);
-        if (const char *e = getenv("PSSGPU_INFLATE_CTAS")) B->inflate_minb = atoi(e) == 2 ? 2 : 3;      // tuning switch
-        CU(cudaFuncSetAttribute(bgzf_inflate_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CU(cudaFuncSetAttribute(bgzf_inflate_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CU(cudaFuncSetAttribute(bgzf_inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int occ = 0;
-        if (B->inflate_minb == 2) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bgzf_inflate_kernel<2>, kInfWarps * 32, smem));
-        else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bgzf_inflate_kernel<3>, kInfWarps * 32, smem));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bgzf_inflate_kernel, kInfWarps * 32, smem));
         if (occ < 1) return fail(ctx, PSSGPU_ECUDA, "BAM ingest: the inflate kernel does not fit an SM");
         B->inflate_grid = occ * ctx->sm_count;
         CU(cudaMemset(B->d_ubuf, 0, kBamCarryCap));
@@ -653,10 +646,7 @@ int bam_stage_and_inflate(pssgpu_ctx *W, const uint8_t *pfx, size_t pfx_len, con
     const size_t   smem = (size_t)kInfWarps * sizeof(InflateTables);
     const unsigned grid = (unsigned)std::min<uint64_t>((n_blocks + kInfWarps - 1) / kInfWarps, (uint64_t)B->inflate_grid);
     time_begin(W, pfx_len + comp_len);
-    if (B->inflate_minb == 2)
-        bgzf_inflate_kernel<2><<<grid, kInfWarps * 32, smem, st>>>(B->d_desc[cur], n_blocks, B->d_comp[cur], B->d_ubuf + kBamCarryCap, B->d_state, B->d_crc_tab);
-    else
-        bgzf_inflate_kernel<3><<<grid, kInfWarps * 32, smem, st>>>(B->d_desc[cur], n_blocks, B->d_comp[cur], B->d_ubuf + kBamCarryCap, B->d_state, B->d_crc_tab);
+    bgzf_inflate_kernel<<<grid, kInfWarps * 32, smem, st>>>(B->d_desc[cur], n_blocks, B->d_comp[cur], B->d_ubuf + kBamCarryCap, B->d_state, B->d_crc_tab);
     time_end(W);
     CU(cudaGetLastError());
     return PSSGPU_OK;

@@ -335,7 +335,7 @@ int pssgpu_group_feed_bam(pssgpu_group *g, const void *bgzf_bytes, size_t len, i
     if (!g || (!bgzf_bytes && len)) return PSSGPU_EINVAL;
     pssgpu_ctx *own = g->ctx[0];
     std::vector<pssgpu_ctx *> helpers;
-    if (g->ctx.size() > 1 && !getenv("PSSGPU_GROUP_BAM_ONE_GPU")) {       // (measurement switch: decode everything on member 0)
+    if (g->ctx.size() > 1) {
         if (!g->bam_self && pssgpu_init(g->dev[0], &g->bam_self) != PSSGPU_OK) {
             g->bam_self = nullptr;
             return gfail(g, PSSGPU_ECUDA, "group_feed_bam: second context on GPU %d: %s", g->dev[0], pssgpu_last_error(nullptr));

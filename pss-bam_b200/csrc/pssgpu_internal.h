@@ -51,7 +51,6 @@ struct pssgpu_ctx {
     size_t    fk_elems = 0;
     unsigned long long *d_stats = nullptr;    // 2 x kStN: outcomes, and fragkon's outcomes in the fused mode
     int       tally_grid_pss = 0, tally_grid_fk = 0;
-    bool      tally_warp = false;             // tally_warp_kernel (warp-autonomous tiles) instead of tally_kernel
     unsigned int *d_range_ctr = nullptr;      // work counter of the tally kernel (zeroed before every launch)
 
     // host feed staging (SAM text pieces; compressed BGZF batches when BAM is fed)

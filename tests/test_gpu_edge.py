@@ -328,7 +328,7 @@ def test_line_longer_than_the_staging_buffer(small):
 def test_spectrum_hot_bins():
     """Low-complexity genome: poly-A, (CA)n and (CAG)n stretches put 10^6 .. 10^7 k-mers into single bins -- far beyond
     the 16-bit shared-memory counters of the k = 7..9 kernel, whose on-the-fly drain must stay exact -- next to N runs
-    and contig ends; the 32-bit-bin first generation (PSSGPU_SPECTRUM_SMEM32) and 64-bit global bins give the same."""
+    and contig ends; 64-bit global bins (PSSGPU_SPECTRUM_WIDE) give the same."""
     import os
     g = Synth.genome(71, [9_000_000, 6_000_000, 1_000_003], n_frac=0.01, lower_frac=0.02)
     for s, (at, n, motif) in zip(g.seqs, [(1_000_000, 5_000_000, b"A"), (500_000, 4_000_000, b"CA"), (1000, 700_000, b"CAG")]):
@@ -342,10 +342,9 @@ def test_spectrum_hot_bins():
         assert int(want.max()) > 3_000_000
         assert np.array_equal(ctx.kmer_spectrum(k), want), k
         assert np.array_equal(sum(ctx.kmer_spectrum(k, s, 5) for s in range(5)), want), k
-        for switch in ("PSSGPU_SPECTRUM_SMEM32", "PSSGPU_SPECTRUM_WIDE"):
-            os.environ[switch] = "1"
-            try:
-                assert np.array_equal(ctx.kmer_spectrum(k), want), (k, switch)
-            finally:
-                del os.environ[switch]
+        os.environ["PSSGPU_SPECTRUM_WIDE"] = "1"
+        try:
+            assert np.array_equal(ctx.kmer_spectrum(k), want), k
+        finally:
+            del os.environ["PSSGPU_SPECTRUM_WIDE"]
     ctx.close()

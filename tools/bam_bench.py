@@ -60,7 +60,6 @@ def main():
     bam_t, bam_tm, bf, br = run(lambda: ctx.feed_bam_ptr(hbam.data_ptr(), nbam, last=True))
     info = ctx.bam_info()
     out = {"reads": a.reads, "sam_bytes": int(nb), "bam_bytes": int(nbam), "zlib_level": a.level, "bam_conversion_s": t_conv,
-           "inflate_ctas_per_sm": os.environ.get("PSSGPU_INFLATE_CTAS", "3"),
            "tables_equal": bool(np.array_equal(sf, bf) and np.array_equal(sr, br)),
            "sam_text": {"s": sam_t, "reads_per_s": a.reads / sam_t, "gb_per_s": nb / sam_t / 1e9, "kernel_ms": sam_tm["kernel_ms"]},
            "bam": {"s": bam_t, "reads_per_s": a.reads / bam_t, "compressed_gb_per_s": nbam / bam_t / 1e9,
