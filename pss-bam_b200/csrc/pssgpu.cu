@@ -35,11 +35,11 @@ int fail(pssgpu_ctx *c, int code, const char *fmt, ...)
     return code;
 }
 
-static cudaEvent_t take_event(pssgpu_ctx *c)
+static Event take_event(pssgpu_ctx *c)
 {
-    cudaEvent_t e = nullptr;
-    if (!c->ev_pool.empty()) { e = c->ev_pool.back(); c->ev_pool.pop_back(); return e; }
-    cudaEventCreate(&e);
+    Event e;
+    if (!c->ev_pool.empty()) { e = std::move(c->ev_pool.back()); c->ev_pool.pop_back(); return e; }
+    create(e, cudaEventDefault);
     return e;
 }
 void time_begin(pssgpu_ctx *c, uint64_t bytes)
@@ -47,52 +47,59 @@ void time_begin(pssgpu_ctx *c, uint64_t bytes)
     c->launches++;
     c->bytes_scanned += bytes;
     if (!c->timing) return;
-    cudaEvent_t a = take_event(c), b = take_event(c);
-    cudaEventRecord(a, c->stream);
-    c->ev.emplace_back(a, b);
+    Event a = take_event(c), b = take_event(c);
+    cudaEventRecord(a.get(), c->stream.get());
+    c->ev.emplace_back(std::move(a), std::move(b));
 }
 void time_end(pssgpu_ctx *c)
 {
     if (!c->timing) return;
-    cudaEventRecord(c->ev.back().second, c->stream);
+    cudaEventRecord(c->ev.back().second.get(), c->stream.get());
 }
 void time_collect(pssgpu_ctx *c)       // stream must be idle
 {
     for (auto &p : c->ev) {
         float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, p.first, p.second) == cudaSuccess) c->kernel_ms += ms;
-        c->ev_pool.push_back(p.first);
-        c->ev_pool.push_back(p.second);
+        if (cudaEventElapsedTime(&ms, p.first.get(), p.second.get()) == cudaSuccess) c->kernel_ms += ms;
+        c->ev_pool.push_back(std::move(p.first));
+        c->ev_pool.push_back(std::move(p.second));
     }
     c->ev.clear();
+}
+
+DevGenome Genome::view() const
+{
+    DevGenome g;
+    g.groups = groups.get();   g.n_groups = n_groups;
+    g.contigs = contigs.get(); g.n_contigs = (uint32_t)n_contigs;
+    g.names = names.get();     g.hash = hash.get(); g.hash_mask = hash_mask;
+    g.exc_pos = exc_pos.get(); g.exc_chr = exc_chr.get(); g.n_exc = n_exc;
+    return g;
+}
+
+uint64_t Genome::hbm_bytes() const
+{
+    return n_groups * sizeof(uint64_t) + kExcCap * 9 + n_contigs * sizeof(DevContig) + names_bytes + ((uint64_t)hash_mask + 1) * 4;
 }
 
 }  // namespace pssgpu
 
 namespace {
 
-void free_genome(pssgpu_ctx *c)
+// the contig table, the names and their hash table -> g (host tables checked or built by the caller)
+cudaError_t put_tables(Genome &g, const DevContig *tab, uint64_t n, const char *names, uint64_t names_bytes, const uint32_t *hash,
+                       uint64_t hash_size)
 {
-    cudaFree(c->d_groups);  c->d_groups = nullptr;
-    cudaFree(c->d_contigs); c->d_contigs = nullptr;
-    cudaFree(c->d_names);   c->d_names = nullptr;
-    cudaFree(c->d_hash);    c->d_hash = nullptr;
-    cudaFree(c->d_exc_pos); c->d_exc_pos = nullptr;
-    cudaFree(c->d_exc_chr); c->d_exc_chr = nullptr;
-    c->n_groups = c->n_bases = c->n_contigs = c->genome_bytes = 0;
-    c->n_exc = 0;
-    c->exc_overflow = false;
-    c->have_genome = false;
-}
-
-DevGenome dev_genome(const pssgpu_ctx *c)
-{
-    DevGenome g;
-    g.groups = c->d_groups;   g.n_groups = c->n_groups;
-    g.contigs = c->d_contigs; g.n_contigs = (uint32_t)c->n_contigs;
-    g.names = c->d_names;     g.hash = c->d_hash; g.hash_mask = c->hash_mask;
-    g.exc_pos = c->d_exc_pos; g.exc_chr = c->d_exc_chr; g.n_exc = c->n_exc;
-    return g;
+    g.n_contigs = n;
+    g.names_bytes = (uint32_t)names_bytes;
+    g.hash_mask = (uint32_t)(hash_size - 1);
+    cudaError_t e = alloc(g.contigs, std::max<size_t>(1, n) * sizeof(DevContig));
+    if (e == cudaSuccess) e = alloc(g.names, names_bytes + 16);                  // + slack: names are also read as whole words
+    if (e == cudaSuccess) e = alloc(g.hash, hash_size * sizeof(uint32_t));
+    if (e == cudaSuccess && n) e = cudaMemcpy(g.contigs.get(), tab, n * sizeof(DevContig), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && names_bytes) e = cudaMemcpy(g.names.get(), names, names_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(g.hash.get(), hash, hash_size * sizeof(uint32_t), cudaMemcpyHostToDevice);
+    return e;
 }
 
 int upload_impl(pssgpu_ctx *ctx, const pssgpu_contig *contigs, uint64_t n, bool src_on_device)
@@ -100,8 +107,8 @@ int upload_impl(pssgpu_ctx *ctx, const pssgpu_contig *contigs, uint64_t n, bool 
     if (!ctx || (!contigs && n)) return fail(ctx, PSSGPU_EINVAL, "genome_upload: null argument");
     if (n > 0x7fffffffull) return fail(ctx, PSSGPU_EUNSUPP, "genome_upload: too many contigs");
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
-    free_genome(ctx);
+    CU(cudaStreamSynchronize(ctx->stream.get()));
+    ctx->genome = Genome();          // the old genome goes first: HBM never holds two, and a failed upload leaves none
 
     // layout + name table
     std::vector<DevContig> tab(n);
@@ -171,29 +178,19 @@ int upload_impl(pssgpu_ctx *ctx, const pssgpu_contig *contigs, uint64_t n, bool 
         }
     }
 
-    uint32_t *d_flags = nullptr;
-    unsigned long long *d_exc_n = nullptr;
-    uint8_t *d_piece = nullptr;
-    auto cleanup = [&]() { cudaFree(d_flags); cudaFree(d_exc_n); cudaFree(d_piece); };
-#define CUX(call)                                                                                  \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess) {                                                                   \
-            cleanup(); free_genome(ctx);                                                           \
-            return fail(ctx, e_ == cudaErrorMemoryAllocation ? PSSGPU_ENOMEM : PSSGPU_ECUDA,       \
-                        "%s: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__);      \
-        }                                                                                          \
-    } while (0)
-
-    CUX(cudaMalloc(&ctx->d_groups, n_groups * sizeof(uint64_t)));
-    CUX(cudaMemsetAsync(ctx->d_groups, 0xff, n_groups * sizeof(uint64_t), ctx->stream));   // everything "other" until packed
-    CUX(cudaMalloc(&ctx->d_exc_pos, kExcCap * sizeof(uint64_t)));
-    CUX(cudaMalloc(&ctx->d_exc_chr, kExcCap));
-    CUX(cudaMalloc(&d_flags, sizeof(uint32_t)));
-    CUX(cudaMalloc(&d_exc_n, sizeof(unsigned long long)));
-    CUX(cudaMemsetAsync(d_flags, 0, sizeof(uint32_t), ctx->stream));
-    CUX(cudaMemsetAsync(d_exc_n, 0, sizeof(unsigned long long), ctx->stream));
-    if (!src_on_device) CUX(cudaMalloc(&d_piece, kPackPiece));
+    Genome g;
+    DevPtr<uint32_t>           d_flags;
+    DevPtr<unsigned long long> d_exc_n;
+    DevPtr<uint8_t>            d_piece;
+    CU(alloc(g.groups, n_groups * sizeof(uint64_t)));
+    CU(cudaMemsetAsync(g.groups.get(), 0xff, n_groups * sizeof(uint64_t), ctx->stream.get()));   // everything "other" until packed
+    CU(alloc(g.exc_pos, kExcCap * sizeof(uint64_t)));
+    CU(alloc(g.exc_chr, kExcCap));
+    CU(alloc(d_flags, sizeof(uint32_t)));
+    CU(alloc(d_exc_n, sizeof(unsigned long long)));
+    CU(cudaMemsetAsync(d_flags.get(), 0, sizeof(uint32_t), ctx->stream.get()));
+    CU(cudaMemsetAsync(d_exc_n.get(), 0, sizeof(unsigned long long), ctx->stream.get()));
+    if (!src_on_device) CU(alloc(d_piece, kPackPiece));
 
     for (uint64_t i = 0; i < n; i++) {
         for (uint64_t off = 0; off < contigs[i].len; off += kPackPiece) {
@@ -202,68 +199,53 @@ int upload_impl(pssgpu_ctx *ctx, const pssgpu_contig *contigs, uint64_t n, bool 
             if (src_on_device) {
                 a.src = reinterpret_cast<const uint8_t *>(contigs[i].seq) + off;
             } else {
-                CUX(cudaMemcpyAsync(d_piece, contigs[i].seq + off, nb, cudaMemcpyHostToDevice, ctx->stream));
+                CU(cudaMemcpyAsync(d_piece.get(), contigs[i].seq + off, nb, cudaMemcpyHostToDevice, ctx->stream.get()));
                 ctx->h2d_bytes += nb;
-                a.src = d_piece;
+                a.src = d_piece.get();
             }
             a.n_bases = nb;
-            a.dst = ctx->d_groups + (tab[i].base_off + off) / 16;
+            a.dst = g.groups.get() + (tab[i].base_off + off) / 16;
             a.gbase = tab[i].base_off + off;
-            a.exc_pos = ctx->d_exc_pos; a.exc_chr = ctx->d_exc_chr; a.exc_n = d_exc_n; a.exc_cap = kExcCap;
-            a.flags = d_flags;
+            a.exc_pos = g.exc_pos.get(); a.exc_chr = g.exc_chr.get(); a.exc_n = d_exc_n.get(); a.exc_cap = kExcCap;
+            a.flags = d_flags.get();
             const uint64_t groups = (nb + 15) / 16;
             const unsigned grid = (unsigned)std::min<uint64_t>((groups + 255) / 256, (uint64_t)ctx->sm_count * 8);
             time_begin(ctx, nb);
-            pack_kernel<<<grid, 256, 0, ctx->stream>>>(a);
+            pack_kernel<<<grid, 256, 0, ctx->stream.get()>>>(a);
             time_end(ctx);
-            CUX(cudaGetLastError());
+            CU(cudaGetLastError());
         }
     }
     uint32_t flags = 0;
     unsigned long long exc_n = 0;
-    CUX(cudaMemcpyAsync(&flags, d_flags, sizeof flags, cudaMemcpyDeviceToHost, ctx->stream));
-    CUX(cudaMemcpyAsync(&exc_n, d_exc_n, sizeof exc_n, cudaMemcpyDeviceToHost, ctx->stream));
-    CUX(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMemcpyAsync(&flags, d_flags.get(), sizeof flags, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaMemcpyAsync(&exc_n, d_exc_n.get(), sizeof exc_n, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     time_collect(ctx);
-    if (flags & 1u) {
-        cleanup(); free_genome(ctx);
-        return fail(ctx, PSSGPU_EUNSUPP, "genome_upload: a contig contains a NUL byte");
-    }
+    if (flags & 1u) return fail(ctx, PSSGPU_EUNSUPP, "genome_upload: a contig contains a NUL byte");
     if (exc_n > kExcCap) {
-        ctx->exc_overflow = true;
-        ctx->n_exc = 0;
+        g.exc_overflow = true;
     } else if (exc_n > 0) {
         std::vector<uint64_t> pos(exc_n);
         std::vector<uint8_t>  chr(exc_n);
-        CUX(cudaMemcpy(pos.data(), ctx->d_exc_pos, exc_n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
-        CUX(cudaMemcpy(chr.data(), ctx->d_exc_chr, exc_n, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(pos.data(), g.exc_pos.get(), exc_n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(chr.data(), g.exc_chr.get(), exc_n, cudaMemcpyDeviceToHost));
         std::vector<uint32_t> order(exc_n);
         for (uint32_t k = 0; k < exc_n; k++) order[k] = k;
         std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return pos[a] < pos[b]; });
         std::vector<uint64_t> spos(exc_n);
         std::vector<uint8_t>  schr(exc_n);
         for (uint32_t k = 0; k < exc_n; k++) { spos[k] = pos[order[k]]; schr[k] = chr[order[k]]; }
-        CUX(cudaMemcpy(ctx->d_exc_pos, spos.data(), exc_n * sizeof(uint64_t), cudaMemcpyHostToDevice));
-        CUX(cudaMemcpy(ctx->d_exc_chr, schr.data(), exc_n, cudaMemcpyHostToDevice));
-        ctx->n_exc = (uint32_t)exc_n;
+        CU(cudaMemcpy(g.exc_pos.get(), spos.data(), exc_n * sizeof(uint64_t), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(g.exc_chr.get(), schr.data(), exc_n, cudaMemcpyHostToDevice));
+        g.n_exc = (uint32_t)exc_n;
     }
-    CUX(cudaMalloc(&ctx->d_contigs, std::max<size_t>(1, n) * sizeof(DevContig)));
-    CUX(cudaMalloc(&ctx->d_names, names.size() + 16));      // + slack: names are also read as whole words
-    CUX(cudaMalloc(&ctx->d_hash, hash_size * sizeof(uint32_t)));
-    if (n) CUX(cudaMemcpy(ctx->d_contigs, tab.data(), n * sizeof(DevContig), cudaMemcpyHostToDevice));
-    if (!names.empty()) CUX(cudaMemcpy(ctx->d_names, names.data(), names.size(), cudaMemcpyHostToDevice));
-    CUX(cudaMemcpy(ctx->d_hash, hash.data(), hash_size * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    cleanup();
-#undef CUX
-    ctx->hash_mask = hash_size - 1;
-    ctx->names_bytes = (uint32_t)names.size();
-    ctx->cc_seed = cc_seed;
-    ctx->cc_ok = cc_ok;
-    ctx->n_groups = n_groups;
-    ctx->n_bases = total;
-    ctx->n_contigs = n;
-    ctx->genome_bytes = n_groups * sizeof(uint64_t) + kExcCap * 9 + n * sizeof(DevContig) + names.size() + hash_size * 4;
-    ctx->have_genome = true;
+    CU(put_tables(g, tab.data(), n, names.data(), names.size(), hash.data(), hash_size));
+    g.cc_seed = cc_seed;
+    g.cc_ok = cc_ok;
+    g.n_groups = n_groups;
+    g.n_bases = total;
+    ctx->genome = std::move(g);
     return PSSGPU_OK;
 }
 
@@ -292,19 +274,19 @@ int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t str
     TallyArgs a;
     a.sam = d_sam; a.len = len; a.stream_off = stream_off;
     a.len_dev = len_dev;
-    a.g = dev_genome(ctx);
+    a.g = ctx->genome.view();
     a.cfg = ctx->cfg;
     a.cfg_fk = ctx->cfg_fk;
-    a.names_bytes = ctx->names_bytes;
-    a.cc_seed = ctx->cc_seed;
-    a.cc_ok = ctx->cc_ok;
-    a.pss_tables = ctx->d_tables;
-    a.fk_hist = ctx->d_fk;
-    a.stats = ctx->d_stats;
-    a.stats_fk = ctx->d_stats + kStN;
-    a.dbg_off = ctx->dbg ? ctx->d_dbg_off : nullptr;
-    a.dbg_code = ctx->dbg ? ctx->d_dbg_code : nullptr;
-    a.dbg_n = ctx->dbg ? ctx->d_dbg_n : nullptr;
+    a.names_bytes = ctx->genome.names_bytes;
+    a.cc_seed = ctx->genome.cc_seed;
+    a.cc_ok = ctx->genome.cc_ok;
+    a.pss_tables = ctx->d_tables.get();
+    a.fk_hist = ctx->d_fk.get();
+    a.stats = ctx->d_stats.get();
+    a.stats_fk = ctx->d_stats.get() + kStN;
+    a.dbg_off = ctx->dbg ? ctx->d_dbg_off.get() : nullptr;
+    a.dbg_code = ctx->dbg ? ctx->d_dbg_code.get() : nullptr;
+    a.dbg_n = ctx->dbg ? ctx->d_dbg_n.get() : nullptr;
     a.dbg_cap = ctx->dbg_cap;
     const int      max_grid = MODE == kModeFragkon ? ctx->tally_grid_fk : ctx->tally_grid_pss;
     // ranges handed out by an atomic counter: about eight per CTA on large inputs, never below 128 KiB
@@ -314,18 +296,18 @@ int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t str
     rb = (rb + 31) & ~31ull;
     const uint64_t n_ranges = (len + rb - 1) / rb;
     a.range_bytes = rb;
-    a.range_ctr = ctx->d_range_ctr;
+    a.range_ctr = ctx->d_range_ctr.get();
     a.one = 1u;
-    CU(cudaMemsetAsync(ctx->d_range_ctr, 0, sizeof(unsigned int), ctx->stream));
+    CU(cudaMemsetAsync(ctx->d_range_ctr.get(), 0, sizeof(unsigned int), ctx->stream.get()));
     time_begin(ctx, len);
     const unsigned grid = (unsigned)std::min<uint64_t>(n_ranges, (uint64_t)max_grid);
     constexpr int PM = MODE == kModeFragkon ? kModePss : MODE;          // (never launched with MODE == kModeFragkon)
     constexpr size_t smem = sizeof(TallySmem);
-    if (MODE == kModeFragkon) tally_kernel<kModeFragkon, 9, 0><<<grid, kThreads, smem, ctx->stream>>>(a);
-    else if (ctx->cfg.R == 15) tally_kernel<PM, 9, 17><<<grid, kThreads, smem, ctx->stream>>>(a);         // the default -r
-    else if (ctx->cfg.R + 2 <= 18) tally_kernel<PM, 9, 0><<<grid, kThreads, smem, ctx->stream>>>(a);
-    else if (ctx->cfg.R <= kMaxRegion) tally_kernel<PM, 16, 0><<<grid, kThreads, smem, ctx->stream>>>(a);
-    else tally_kernel<PM, 0, 0><<<grid, kThreads, smem, ctx->stream>>>(a);                                // any -r: exact, not tuned
+    if (MODE == kModeFragkon) tally_kernel<kModeFragkon, 9, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);
+    else if (ctx->cfg.R == 15) tally_kernel<PM, 9, 17><<<grid, kThreads, smem, ctx->stream.get()>>>(a);         // the default -r
+    else if (ctx->cfg.R + 2 <= 18) tally_kernel<PM, 9, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);
+    else if (ctx->cfg.R <= kMaxRegion) tally_kernel<PM, 16, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);
+    else tally_kernel<PM, 0, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);                                // any -r: exact, not tuned
     time_end(ctx);
     CU(cudaGetLastError());
     return PSSGPU_OK;
@@ -342,13 +324,16 @@ int pssgpu::launch_tally_mode(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len,
 
 namespace {
 
+// after the parameters of a *_begin were accepted: no tally is open until the begin completes (a table it failed to
+// allocate must never be fed)
 int begin_common(pssgpu_ctx *ctx)
 {
-    CU(cudaStreamSynchronize(ctx->stream));
-    if (!ctx->d_stats) CU(cudaMalloc(&ctx->d_stats, 2 * kStN * sizeof(unsigned long long)));
-    if (!ctx->d_range_ctr) CU(cudaMalloc(&ctx->d_range_ctr, sizeof(unsigned int)));
-    CU(cudaMemsetAsync(ctx->d_stats, 0, 2 * kStN * sizeof(unsigned long long), ctx->stream));
-    if (ctx->d_dbg_n) CU(cudaMemsetAsync(ctx->d_dbg_n, 0, sizeof(unsigned long long), ctx->stream));
+    ctx->mode = -1;
+    CU(cudaStreamSynchronize(ctx->stream.get()));
+    if (!ctx->d_stats) CU(alloc(ctx->d_stats, 2 * kStN * sizeof(unsigned long long)));
+    if (!ctx->d_range_ctr) CU(alloc(ctx->d_range_ctr, sizeof(unsigned int)));
+    CU(cudaMemsetAsync(ctx->d_stats.get(), 0, 2 * kStN * sizeof(unsigned long long), ctx->stream.get()));
+    if (ctx->dbg_cap) CU(cudaMemsetAsync(ctx->d_dbg_n.get(), 0, sizeof(unsigned long long), ctx->stream.get()));
     ctx->carry_len = 0;
     ctx->cur = 0;
     ctx->fed_bytes = 0;
@@ -384,15 +369,14 @@ int pssgpu_init(int device, pssgpu_ctx **out)
         return fail(nullptr, PSSGPU_EUNSUPP, "pssgpu_init: device %d is sm_%d%d; this library holds sm_100a code only",
                     device, prop.major, prop.minor);
     CU(cudaSetDevice(device));
-    pssgpu_ctx *c = new pssgpu_ctx();
+    std::unique_ptr<pssgpu_ctx> c(new pssgpu_ctx());       // on failure released here, with its device current
     c->device = device;
     c->sm_count = prop.multiProcessorCount;
-    cudaError_t e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->copy_done, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking);
+    cudaError_t e = create(c->stream);
+    if (e == cudaSuccess) e = create(c->copy_stream);
     for (int i = 0; i < 2; i++) {
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->ev_copied[i], cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->ev_tallied[i], cudaEventDisableTiming);
+        if (e == cudaSuccess) e = create(c->ev_copied[i]);
+        if (e == cudaSuccess) e = create(c->ev_tallied[i]);
     }
     {   // every instantiation needs its dynamic shared memory raised above the 48 KB default
         const void *kernels[] = {
@@ -405,44 +389,26 @@ int pssgpu_init(int device, pssgpu_ctx **out)
     int occ_p = 0, occ_f = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, tally_kernel<kModePss, 16, 0>, kThreads, sizeof(TallySmem));
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_f, tally_kernel<kModeFragkon, 9, 0>, kThreads, sizeof(TallySmem));
-    if (e != cudaSuccess || occ_p < 1 || occ_f < 1) {
-        fail(nullptr, PSSGPU_ECUDA, "pssgpu_init: %s (occupancy %d/%d)", cudaGetErrorString(e), occ_p, occ_f);
-        if (c->stream) cudaStreamDestroy(c->stream);
-        if (c->copy_done) cudaEventDestroy(c->copy_done);
-        if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-        for (int i = 0; i < 2; i++) { if (c->ev_copied[i]) cudaEventDestroy(c->ev_copied[i]); if (c->ev_tallied[i]) cudaEventDestroy(c->ev_tallied[i]); }
-        delete c;
-        return PSSGPU_ECUDA;
-    }
+    if (e != cudaSuccess || occ_p < 1 || occ_f < 1)
+        return fail(nullptr, PSSGPU_ECUDA, "pssgpu_init: %s (occupancy %d/%d)", cudaGetErrorString(e), occ_p, occ_f);
     c->tally_grid_pss = c->sm_count * occ_p;
     c->tally_grid_fk = c->sm_count * occ_f;
 
-    *out = c;
+    *out = c.release();
     return PSSGPU_OK;
 }
 
 void pssgpu_destroy(pssgpu_ctx *ctx)
 {
     if (!ctx) return;
-    Bind bind(ctx);
-    cudaStreamSynchronize(ctx->stream);
-    bam_destroy(ctx);
-    free_genome(ctx);
-    cudaFree(ctx->d_tables); cudaFree(ctx->d_fk); cudaFree(ctx->d_stats); cudaFree(ctx->d_range_ctr);
-    cudaFree(ctx->d_stage[0]); cudaFree(ctx->d_stage[1]);
-    cudaFree(ctx->d_dbg_off); cudaFree(ctx->d_dbg_code); cudaFree(ctx->d_dbg_n);
-    for (auto &p : ctx->ev) { cudaEventDestroy(p.first); cudaEventDestroy(p.second); }
-    for (auto e : ctx->ev_pool) cudaEventDestroy(e);
-    if (ctx->copy_done) cudaEventDestroy(ctx->copy_done);
-    if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    for (int i = 0; i < 2; i++) { if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]); if (ctx->ev_tallied[i]) cudaEventDestroy(ctx->ev_tallied[i]); }
-    cudaStreamDestroy(ctx->stream);
+    Bind bind(ctx);                   // the context's members are released on its device
+    cudaStreamSynchronize(ctx->stream.get());
     delete ctx;
 }
 
 const char *pssgpu_last_error(const pssgpu_ctx *ctx) { return ctx ? ctx->err.c_str() : g_init_error.c_str(); }
 
-void *pssgpu_cuda_stream(pssgpu_ctx *ctx) { return ctx ? (void *)ctx->stream : nullptr; }
+void *pssgpu_cuda_stream(pssgpu_ctx *ctx) { return ctx ? (void *)ctx->stream.get() : nullptr; }
 
 void *pssgpu_host_alloc(size_t bytes)
 {
@@ -495,9 +461,9 @@ bool same_tag(const pssgpu_genome_tag &a, const pssgpu_genome_tag &b)
 int genome_save_impl(pssgpu_ctx *ctx, const char *path, const pssgpu_genome_tag *tag)
 {
     if (!ctx || !path) return fail(ctx, PSSGPU_EINVAL, "genome_save: null argument");
-    if (!ctx->have_genome) return fail(ctx, PSSGPU_ENOGENOME, "genome_save: no genome resident");
+    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "genome_save: no genome resident");
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     // written under a temporary name and renamed: a reader never sees a half-written cache
     const std::string tmp = std::string(path) + ".tmp" + std::to_string((long)getpid());
     FILE *f = fopen(tmp.c_str(), "wb");
@@ -505,18 +471,19 @@ int genome_save_impl(pssgpu_ctx *ctx, const char *path, const pssgpu_genome_tag 
     CacheHeader h;
     memset(&h, 0, sizeof h);
     memcpy(h.magic, kCacheMagic, 8);
-    h.n_contigs = ctx->n_contigs; h.n_groups = ctx->n_groups; h.n_bases = ctx->n_bases; h.names_bytes = ctx->names_bytes;
-    h.n_exc = ctx->n_exc; h.hash_size = (uint64_t)ctx->hash_mask + 1; h.cc_seed = ctx->cc_seed; h.cc_ok = ctx->cc_ok;
-    h.exc_overflow = ctx->exc_overflow ? 1u : 0u; h.pad_bases = (uint32_t)kPadBases;
+    const Genome &G = ctx->genome;
+    h.n_contigs = G.n_contigs; h.n_groups = G.n_groups; h.n_bases = G.n_bases; h.names_bytes = G.names_bytes;
+    h.n_exc = G.n_exc; h.hash_size = (uint64_t)G.hash_mask + 1; h.cc_seed = G.cc_seed; h.cc_ok = G.cc_ok;
+    h.exc_overflow = G.exc_overflow ? 1u : 0u; h.pad_bases = (uint32_t)kPadBases;
     if (tag) h.tag = *tag;
     std::vector<char> buf(kCachePiece);
     bool ok = fwrite(&h, sizeof h, 1, f) == 1
-           && write_dev(f, ctx->d_contigs, h.n_contigs * sizeof(DevContig), buf)
-           && write_dev(f, ctx->d_names, h.names_bytes, buf)
-           && write_dev(f, ctx->d_hash, h.hash_size * sizeof(uint32_t), buf)
-           && write_dev(f, ctx->d_exc_pos, h.n_exc * sizeof(uint64_t), buf)
-           && write_dev(f, ctx->d_exc_chr, h.n_exc, buf)
-           && write_dev(f, ctx->d_groups, h.n_groups * sizeof(uint64_t), buf);
+           && write_dev(f, G.contigs.get(), h.n_contigs * sizeof(DevContig), buf)
+           && write_dev(f, G.names.get(), h.names_bytes, buf)
+           && write_dev(f, G.hash.get(), h.hash_size * sizeof(uint32_t), buf)
+           && write_dev(f, G.exc_pos.get(), h.n_exc * sizeof(uint64_t), buf)
+           && write_dev(f, G.exc_chr.get(), h.n_exc, buf)
+           && write_dev(f, G.groups.get(), h.n_groups * sizeof(uint64_t), buf);
     ok = (fclose(f) == 0) && ok;
     if (ok && rename(tmp.c_str(), path) != 0) ok = false;
     if (!ok) { remove(tmp.c_str()); return fail(ctx, PSSGPU_EINVAL, "genome_save: writing %s failed", path); }
@@ -528,8 +495,8 @@ int genome_load_impl(pssgpu_ctx *ctx, const char *path, const pssgpu_genome_tag 
 {
     if (!ctx || !path) return fail(ctx, PSSGPU_EINVAL, "genome_load: null argument");
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
-    free_genome(ctx);
+    CU(cudaStreamSynchronize(ctx->stream.get()));
+    ctx->genome = Genome();          // as in upload_impl: the old genome goes first, a failed load leaves none
     FILE *f = fopen(path, "rb");
     if (!f) return fail(ctx, PSSGPU_EINVAL, "genome_load: cannot open %s", path);
     CacheHeader h;
@@ -575,32 +542,24 @@ int genome_load_impl(pssgpu_ctx *ctx, const char *path, const pssgpu_genome_tag 
     if (!ok) { fclose(f); return fail(ctx, PSSGPU_EINVAL, "genome_load: %s is damaged (a table entry is out of range)", path); }
 
     std::vector<char> buf(kCachePiece);
-    cudaError_t e = cudaMalloc(&ctx->d_contigs, std::max<size_t>(1, h.n_contigs) * sizeof(DevContig));
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_names, h.names_bytes + 16);
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_hash, h.hash_size * sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_exc_pos, kExcCap * sizeof(uint64_t));
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_exc_chr, kExcCap);
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_groups, h.n_groups * sizeof(uint64_t));
-    if (e == cudaSuccess && h.n_contigs) e = cudaMemcpy(ctx->d_contigs, tab.data(), h.n_contigs * sizeof(DevContig), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && h.names_bytes) e = cudaMemcpy(ctx->d_names, names.data(), h.names_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(ctx->d_hash, hash.data(), h.hash_size * sizeof(uint32_t), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && h.n_exc) e = cudaMemcpy(ctx->d_exc_pos, exc_pos.data(), h.n_exc * sizeof(uint64_t), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && h.n_exc) e = cudaMemcpy(ctx->d_exc_chr, exc_chr.data(), h.n_exc, cudaMemcpyHostToDevice);
-    ok = e == cudaSuccess && read_dev(f, ctx->d_groups, h.n_groups * sizeof(uint64_t), buf);
+    Genome g;
+    cudaError_t e = put_tables(g, tab.data(), h.n_contigs, names.data(), h.names_bytes, hash.data(), h.hash_size);
+    if (e == cudaSuccess) e = alloc(g.exc_pos, kExcCap * sizeof(uint64_t));
+    if (e == cudaSuccess) e = alloc(g.exc_chr, kExcCap);
+    if (e == cudaSuccess) e = alloc(g.groups, h.n_groups * sizeof(uint64_t));
+    if (e == cudaSuccess && h.n_exc) e = cudaMemcpy(g.exc_pos.get(), exc_pos.data(), h.n_exc * sizeof(uint64_t), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && h.n_exc) e = cudaMemcpy(g.exc_chr.get(), exc_chr.data(), h.n_exc, cudaMemcpyHostToDevice);
+    ok = e == cudaSuccess && read_dev(f, g.groups.get(), h.n_groups * sizeof(uint64_t), buf);
     fclose(f);
     if (!ok) {
-        free_genome(ctx);
         cudaGetLastError();
         return fail(ctx, e == cudaErrorMemoryAllocation ? PSSGPU_ENOMEM : PSSGPU_EINVAL, "genome_load: reading %s failed", path);
     }
-    ctx->hash_mask = (uint32_t)(h.hash_size - 1);
-    ctx->names_bytes = (uint32_t)h.names_bytes;
-    ctx->cc_seed = h.cc_seed; ctx->cc_ok = h.cc_ok;
-    ctx->n_groups = h.n_groups; ctx->n_bases = h.n_bases; ctx->n_contigs = h.n_contigs;
-    ctx->n_exc = (uint32_t)h.n_exc; ctx->exc_overflow = h.exc_overflow != 0;
-    ctx->genome_bytes = h.n_groups * sizeof(uint64_t) + kExcCap * 9 + h.n_contigs * sizeof(DevContig) + h.names_bytes + h.hash_size * 4;
+    g.cc_seed = h.cc_seed; g.cc_ok = h.cc_ok;
+    g.n_groups = h.n_groups; g.n_bases = h.n_bases;
+    g.n_exc = (uint32_t)h.n_exc; g.exc_overflow = h.exc_overflow != 0;
+    ctx->genome = std::move(g);
     ctx->h2d_bytes += h.n_groups * sizeof(uint64_t);
-    ctx->have_genome = true;
     return PSSGPU_OK;
 }
 }  // namespace
@@ -620,10 +579,10 @@ int pssgpu_genome_load_tagged(pssgpu_ctx *ctx, const char *path, const pssgpu_ge
 
 int pssgpu_genome_info(const pssgpu_ctx *ctx, uint64_t *n_contigs, uint64_t *n_bases, uint64_t *hbm_bytes)
 {
-    if (!ctx || !ctx->have_genome) return PSSGPU_ENOGENOME;
-    if (n_contigs) *n_contigs = ctx->n_contigs;
-    if (n_bases) *n_bases = ctx->n_bases;
-    if (hbm_bytes) *hbm_bytes = ctx->genome_bytes;
+    if (!ctx || !ctx->genome.resident()) return PSSGPU_ENOGENOME;
+    if (n_contigs) *n_contigs = ctx->genome.n_contigs;
+    if (n_bases) *n_bases = ctx->genome.n_bases;
+    if (hbm_bytes) *hbm_bytes = ctx->genome.hbm_bytes();
     return PSSGPU_OK;
 }
 
@@ -656,7 +615,7 @@ int pss_cfg(pssgpu_ctx *ctx, const pssgpu_pss_params *p, TallyCfg &c)
     int rc;
     if ((rc = ctx_string(ctx, p->up_ctx, &c.up_mask, &c.up_other, c.up_ctx)) != PSSGPU_OK) return rc;
     if ((rc = ctx_string(ctx, p->down_ctx, &c.down_mask, &c.down_other, c.down_ctx)) != PSSGPU_OK) return rc;
-    if ((c.up_other || c.down_other) && ctx->exc_overflow)
+    if ((c.up_other || c.down_other) && ctx->genome.exc_overflow)
         return fail(ctx, PSSGPU_EUNSUPP, "-U/-D name bytes outside " PSSGPU_SYM_CHARS " and the genome holds more than %llu such bytes",
                     (unsigned long long)kExcCap);
     return PSSGPU_OK;
@@ -677,10 +636,9 @@ int fk_cfg(pssgpu_ctx *ctx, const pssgpu_fragkon_params *p, TallyCfg &c)
 
 int alloc_pss_tables(pssgpu_ctx *ctx, int R)
 {
-    cudaFree(ctx->d_tables); ctx->d_tables = nullptr;
     const size_t elems = 2 * (size_t)(R + 2) * 16;
-    CU(cudaMalloc(&ctx->d_tables, elems * sizeof(unsigned long long)));
-    CU(cudaMemsetAsync(ctx->d_tables, 0, elems * sizeof(unsigned long long), ctx->stream));
+    CU(alloc(ctx->d_tables, elems * sizeof(unsigned long long)));
+    CU(cudaMemsetAsync(ctx->d_tables.get(), 0, elems * sizeof(unsigned long long), ctx->stream.get()));
     return PSSGPU_OK;
 }
 
@@ -688,11 +646,11 @@ int alloc_fk_tables(pssgpu_ctx *ctx, int K)
 {
     const size_t elems = 2ull << (2 * K);
     if (elems != ctx->fk_elems) {
-        cudaFree(ctx->d_fk); ctx->d_fk = nullptr; ctx->fk_elems = 0;
-        CU(cudaMalloc(&ctx->d_fk, elems * sizeof(unsigned long long)));
+        ctx->fk_elems = 0;
+        CU(alloc(ctx->d_fk, elems * sizeof(unsigned long long)));
         ctx->fk_elems = elems;
     }
-    CU(cudaMemsetAsync(ctx->d_fk, 0, elems * sizeof(unsigned long long), ctx->stream));
+    CU(cudaMemsetAsync(ctx->d_fk.get(), 0, elems * sizeof(unsigned long long), ctx->stream.get()));
     return PSSGPU_OK;
 }
 
@@ -701,7 +659,7 @@ int alloc_fk_tables(pssgpu_ctx *ctx, int K)
 int pssgpu_pss_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p)
 {
     if (!ctx || !p) return fail(ctx, PSSGPU_EINVAL, "pss_begin: null argument");
-    if (!ctx->have_genome) return fail(ctx, PSSGPU_ENOGENOME, "pss_begin: no genome resident");
+    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "pss_begin: no genome resident");
     Bind bind(ctx);
     TallyCfg c;
     int rc;
@@ -716,7 +674,7 @@ int pssgpu_pss_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p)
 int pssgpu_both_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p, const pssgpu_fragkon_params *f)
 {
     if (!ctx || !p || !f) return fail(ctx, PSSGPU_EINVAL, "both_begin: null argument");
-    if (!ctx->have_genome) return fail(ctx, PSSGPU_ENOGENOME, "both_begin: no genome resident");
+    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "both_begin: no genome resident");
     Bind bind(ctx);
     TallyCfg c, cf;
     int rc;
@@ -738,20 +696,20 @@ namespace {
 int stage_launch(pssgpu_ctx *ctx, size_t klen, uint64_t soff)
 {
     const int cur = ctx->cur;
-    CU(cudaEventRecord(ctx->ev_copied[cur], ctx->copy_stream));
-    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[cur], 0));
-    int rc = launch_tally_mode(ctx, ctx->d_stage[cur], klen, soff);
+    CU(cudaEventRecord(ctx->ev_copied[cur].get(), ctx->copy_stream.get()));
+    CU(cudaStreamWaitEvent(ctx->stream.get(), ctx->ev_copied[cur].get(), 0));
+    int rc = launch_tally_mode(ctx, ctx->d_stage[cur].get(), klen, soff);
     if (rc != PSSGPU_OK) return rc;
-    CU(cudaEventRecord(ctx->ev_tallied[cur], ctx->stream));
+    CU(cudaEventRecord(ctx->ev_tallied[cur].get(), ctx->stream.get()));
     ctx->cur ^= 1;
-    CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_tallied[ctx->cur], 0));
+    CU(cudaStreamWaitEvent(ctx->copy_stream.get(), ctx->ev_tallied[ctx->cur].get(), 0));
     return PSSGPU_OK;
 }
 
 int feed_impl(pssgpu_ctx *ctx, const char *sam, size_t len, int last)
 {
     for (int s = 0; s < 2; s++)
-        if (!ctx->d_stage[s]) CU(cudaMalloc(&ctx->d_stage[s], kStageCap + 64));
+        if (!ctx->d_stage[s]) CU(alloc(ctx->d_stage[s], kStageCap + 64));
     // Two staging buffers, two streams: the copies queue up on copy_stream, the tallies on the context's stream; a
     // tally waits for its copy (ev_copied), a copy into a buffer waits for the tally that last read it (ev_tallied).
     // The PCIe link then never idles behind a kernel launch.
@@ -763,27 +721,27 @@ int feed_impl(pssgpu_ctx *ctx, const char *sam, size_t len, int last)
             // the stretches before the cut are tallied now (the kernel's long_record path), the rest stays carried.
             const size_t   cut = (kStageCap / (size_t)kMaxLine) * (size_t)kMaxLine, tail = kStageCap - cut;
             const uint64_t soff = ctx->fed_bytes + off - ctx->carry_len;
-            uint8_t       *from = ctx->d_stage[ctx->cur];
+            uint8_t       *from = ctx->d_stage[ctx->cur].get();
             int rc = stage_launch(ctx, cut, soff);
             if (rc != PSSGPU_OK) return rc;
-            CU(cudaMemcpyAsync(ctx->d_stage[ctx->cur], from + cut, tail, cudaMemcpyDeviceToDevice, ctx->copy_stream));
+            CU(cudaMemcpyAsync(ctx->d_stage[ctx->cur].get(), from + cut, tail, cudaMemcpyDeviceToDevice, ctx->copy_stream.get()));
             ctx->carry_len = tail;
         }
         const size_t room = kStageCap - ctx->carry_len;
         const size_t plen = std::min(std::min(len - off, kFeedPiece), room);
         const char  *piece = sam + off;
         const char  *nl = (const char *)memrchr(piece, '\n', plen);
-        uint8_t     *slot = ctx->d_stage[ctx->cur];
+        uint8_t     *slot = ctx->d_stage[ctx->cur].get();
         if (!nl) {                       // no line ends in this piece: it only grows the carry
-            CU(cudaMemcpyAsync(slot + ctx->carry_len, piece, plen, cudaMemcpyHostToDevice, ctx->copy_stream));
+            CU(cudaMemcpyAsync(slot + ctx->carry_len, piece, plen, cudaMemcpyHostToDevice, ctx->copy_stream.get()));
             ctx->carry_len += plen;
         } else {
             const size_t cut = (size_t)(nl - piece) + 1, tail = plen - cut;
-            CU(cudaMemcpyAsync(slot + ctx->carry_len, piece, cut, cudaMemcpyHostToDevice, ctx->copy_stream));
+            CU(cudaMemcpyAsync(slot + ctx->carry_len, piece, cut, cudaMemcpyHostToDevice, ctx->copy_stream.get()));
             int rc = stage_launch(ctx, ctx->carry_len + cut, ctx->fed_bytes + off - ctx->carry_len);
             if (rc != PSSGPU_OK) return rc;
             // (the other buffer is free once the tally that read it, two pieces ago, is done: stage_launch queued the wait)
-            if (tail) CU(cudaMemcpyAsync(ctx->d_stage[ctx->cur], piece + cut, tail, cudaMemcpyHostToDevice, ctx->copy_stream));
+            if (tail) CU(cudaMemcpyAsync(ctx->d_stage[ctx->cur].get(), piece + cut, tail, cudaMemcpyHostToDevice, ctx->copy_stream.get()));
             ctx->carry_len = tail;
         }
         ctx->h2d_bytes += plen;
@@ -809,7 +767,7 @@ int pssgpu_feed(pssgpu_ctx *ctx, const char *sam, size_t len, int last)
     // that read it are waited for.  The tallies are not: they drain at pssgpu_sync / *_finish / get_stats, which is
     // where a kernel fault would surface.  A caller that alternates two pinned buffers (host/pss_host.c) thus
     // overlaps its own reading of the next chunk with the tally of this one.
-    const cudaError_t e = cudaStreamSynchronize(ctx->copy_stream);
+    const cudaError_t e = cudaStreamSynchronize(ctx->copy_stream.get());
     if (rc != PSSGPU_OK) return rc;
     if (e != cudaSuccess) return fail(ctx, PSSGPU_ECUDA, "feed: %s", cudaGetErrorString(e));
     return PSSGPU_OK;
@@ -821,7 +779,7 @@ int pssgpu_feed_async(pssgpu_ctx *ctx, const char *sam, size_t len, int last)
     if (ctx->mode < 0) return fail(ctx, PSSGPU_EINVAL, "feed_async: no tally open (call *_begin first)");
     Bind bind(ctx);
     const int rc = feed_impl(ctx, sam, len, last);
-    if (rc != PSSGPU_OK) cudaStreamSynchronize(ctx->copy_stream);      // after an error nothing reads `sam` any more
+    if (rc != PSSGPU_OK) cudaStreamSynchronize(ctx->copy_stream.get());      // after an error nothing reads `sam` any more
     return rc;
 }
 
@@ -829,7 +787,7 @@ int pssgpu_feed_wait(pssgpu_ctx *ctx)
 {
     if (!ctx) return PSSGPU_EINVAL;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->copy_stream));
+    CU(cudaStreamSynchronize(ctx->copy_stream.get()));
     return PSSGPU_OK;
 }
 
@@ -849,7 +807,7 @@ int pssgpu_sync(pssgpu_ctx *ctx)
 {
     if (!ctx) return PSSGPU_EINVAL;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, false); if (brc != PSSGPU_OK) return brc; }
     time_collect(ctx);
     return PSSGPU_OK;
@@ -862,9 +820,9 @@ int pssgpu_pss_finish(pssgpu_ctx *ctx, uint64_t *fwd, uint64_t *rev)
     if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "pss_finish: %zu bytes of an unterminated line pending (feed with last=1)", ctx->carry_len);
     Bind bind(ctx);
     const size_t half = (size_t)(ctx->cfg.R + 2) * 16 * sizeof(uint64_t);
-    CU(cudaMemcpyAsync(fwd, ctx->d_tables, half, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(rev, (const char *)ctx->d_tables + half, half, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMemcpyAsync(fwd, ctx->d_tables.get(), half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaMemcpyAsync(rev, (const char *)ctx->d_tables.get() + half, half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
     ctx->d2h_bytes += 2 * half;
     time_collect(ctx);
@@ -878,8 +836,8 @@ int pssgpu_pss_finish_device(pssgpu_ctx *ctx, void *d_tables)
     if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "pss_finish_device: unterminated line pending");
     Bind bind(ctx);
     const size_t bytes = 2 * (size_t)(ctx->cfg.R + 2) * 16 * sizeof(uint64_t);
-    CU(cudaMemcpyAsync(d_tables, ctx->d_tables, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMemcpyAsync(d_tables, ctx->d_tables.get(), bytes, cudaMemcpyDeviceToDevice, ctx->stream.get()));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
     time_collect(ctx);
     return PSSGPU_OK;
@@ -892,8 +850,8 @@ int read_stats(pssgpu_ctx *ctx, pssgpu_stats *out, int which)
     if (!ctx->d_stats) return fail(ctx, PSSGPU_EINVAL, "get_stats: no tally was opened");
     Bind bind(ctx);
     unsigned long long h[kStN];
-    CU(cudaMemcpyAsync(h, ctx->d_stats + which * kStN, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMemcpyAsync(h, ctx->d_stats.get() + which * kStN, sizeof h, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, false); if (brc != PSSGPU_OK) return brc; }
     time_collect(ctx);
     out->lines = h[kStLines];
@@ -928,7 +886,7 @@ void pssgpu_fragkon_default_params(pssgpu_fragkon_params *p)
 int pssgpu_fragkon_begin(pssgpu_ctx *ctx, const pssgpu_fragkon_params *p)
 {
     if (!ctx || !p) return fail(ctx, PSSGPU_EINVAL, "fragkon_begin: null argument");
-    if (!ctx->have_genome) return fail(ctx, PSSGPU_ENOGENOME, "fragkon_begin: no genome resident");
+    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "fragkon_begin: no genome resident");
     Bind bind(ctx);
     TallyCfg c;
     int rc;
@@ -947,9 +905,9 @@ int pssgpu_fragkon_finish(pssgpu_ctx *ctx, uint64_t *fp, uint64_t *tp)
     if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish: unterminated line pending (feed with last=1)");
     Bind bind(ctx);
     const size_t half = (ctx->fk_elems / 2) * sizeof(uint64_t);
-    CU(cudaMemcpyAsync(fp, ctx->d_fk, half, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(tp, (const char *)ctx->d_fk + half, half, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMemcpyAsync(fp, ctx->d_fk.get(), half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaMemcpyAsync(tp, (const char *)ctx->d_fk.get() + half, half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
     ctx->d2h_bytes += 2 * half;
     time_collect(ctx);
@@ -962,8 +920,8 @@ int pssgpu_fragkon_finish_device(pssgpu_ctx *ctx, void *d_out)
     if (ctx->mode != kModeFragkon && ctx->mode != kModeBoth) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish_device: no fragkon tally open");
     if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish_device: unterminated line pending");
     Bind bind(ctx);
-    CU(cudaMemcpyAsync(d_out, ctx->d_fk, ctx->fk_elems * sizeof(uint64_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMemcpyAsync(d_out, ctx->d_fk.get(), ctx->fk_elems * sizeof(uint64_t), cudaMemcpyDeviceToDevice, ctx->stream.get()));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
     time_collect(ctx);
     return PSSGPU_OK;
@@ -973,59 +931,63 @@ int pssgpu_fragkon_finish_device(pssgpu_ctx *ctx, void *d_out)
 int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_shards, void *d_counts)
 {
     if (!ctx || !d_counts) return fail(ctx, PSSGPU_EINVAL, "kmer_spectrum: null argument");
-    if (!ctx->have_genome) return fail(ctx, PSSGPU_ENOGENOME, "kmer_spectrum: no genome resident");
+    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "kmer_spectrum: no genome resident");
     if (k < 1 || k > kMaxFragK) return fail(ctx, PSSGPU_EUNSUPP, "kmer_spectrum: k %d outside [1,%d]", k, kMaxFragK);
     if (n_shards < 1 || shard < 0 || shard >= n_shards) return fail(ctx, PSSGPU_EINVAL, "kmer_spectrum: shard %d of %d", shard, n_shards);
     Bind bind(ctx);
     const size_t bins = 1ull << (2 * k);
     // k-mers are attributed to the group holding their first base; the last
     // two groups are slack/padding and start no k-mer
-    const uint64_t usable = ctx->n_groups - 2;
+    const uint64_t *d_groups = ctx->genome.groups.get();
+    const uint64_t usable = ctx->genome.n_groups - 2;
     const uint64_t g0 = usable * (uint64_t)shard / (uint64_t)n_shards;
     const uint64_t g1 = usable * (uint64_t)(shard + 1) / (uint64_t)n_shards;
     const unsigned grid = (unsigned)std::min<uint64_t>(std::max<uint64_t>(1, (g1 - g0 + 255) / 256), (uint64_t)ctx->sm_count * 8);
     // 32-bit bins while no bin can overflow them (fewer than 2^32 positions in the shard)
     // (PSSGPU_SPECTRUM_WIDE: test switch -- run the 64-bit-bin instantiations on a genome that would not need them)
     const bool narrow = (g1 - g0) * 16 < 0xffffffffull && !getenv("PSSGPU_SPECTRUM_WIDE");
-    unsigned int *d_narrow = nullptr;
+    // the scratch buffers of this call are released when it returns, after the stream synchronisation that follows the
+    // last launch
+    DevPtr<unsigned int> d_narrow;
     if (narrow) {
-        CU(cudaMalloc(&d_narrow, bins * sizeof(unsigned int)));
-        cudaError_t e = cudaMemsetAsync(d_narrow, 0, bins * sizeof(unsigned int), ctx->stream);
-        if (e != cudaSuccess) { cudaFree(d_narrow); return fail(ctx, PSSGPU_ECUDA, "kmer_spectrum: %s", cudaGetErrorString(e)); }
+        CU(alloc(d_narrow, bins * sizeof(unsigned int)));
+        cudaError_t e = cudaMemsetAsync(d_narrow.get(), 0, bins * sizeof(unsigned int), ctx->stream.get());
+        if (e != cudaSuccess) return fail(ctx, PSSGPU_ECUDA, "kmer_spectrum: %s", cudaGetErrorString(e));
     } else {
-        CU(cudaMemsetAsync(d_counts, 0, bins * sizeof(uint64_t), ctx->stream));
+        CU(cudaMemsetAsync(d_counts, 0, bins * sizeof(uint64_t), ctx->stream.get()));
     }
     // k = 10 .. 12: radix partition through a scratch buffer (32 bytes per group); without the memory for it, L2 atomics
-    uint16_t *d_payload = nullptr;
-    unsigned long long *d_rad = nullptr;                   // bucket counts | offsets (nb + 1) | cursors
+    DevPtr<uint16_t> d_payload;
+    DevPtr<unsigned long long> d_rad;                      // bucket counts | offsets (nb + 1) | cursors
     const uint32_t rad_nb = (k >= 10 && k <= 12) ? (1u << (2 * k - kSpecSmemLog)) : 0u;
     if (rad_nb && g1 > g0) {
-        if (cudaMalloc(&d_payload, (g1 - g0) * 16 * sizeof(uint16_t) + 64) != cudaSuccess) { cudaGetLastError(); d_payload = nullptr; }
-        else if (cudaMalloc(&d_rad, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long)) != cudaSuccess) {
-            cudaGetLastError(); cudaFree(d_payload); d_payload = nullptr; d_rad = nullptr;
+        if (alloc(d_payload, (g1 - g0) * 16 * sizeof(uint16_t) + 64) != cudaSuccess
+            || alloc(d_rad, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long)) != cudaSuccess) {
+            cudaGetLastError();
+            d_payload.reset();
         }
     }
     time_begin(ctx, (g1 - g0) * sizeof(uint64_t));
     if (d_payload) {
-        unsigned long long *cnt = d_rad, *off = d_rad + rad_nb, *cur = d_rad + 2 * (size_t)rad_nb + 1;
-        cudaMemsetAsync(d_rad, 0, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long), ctx->stream);
+        unsigned long long *cnt = d_rad.get(), *off = cnt + rad_nb, *cur = cnt + 2 * (size_t)rad_nb + 1;
+        cudaMemsetAsync(cnt, 0, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long), ctx->stream.get());
         const unsigned rgrid = (unsigned)std::min<uint64_t>((g1 - g0 + kRadixThreads - 1) / kRadixThreads, (uint64_t)ctx->sm_count * 4);
         const uint32_t parts = std::max<uint32_t>(1u, (2u * (uint32_t)ctx->sm_count + rad_nb - 1) / rad_nb);
         const size_t   hsmem = (size_t)kSpecSmemBins * sizeof(uint32_t);
 #define PSS_RADIX(K_)                                                                                                  \
         do {                                                                                                           \
-            radix_count_kernel<K_><<<rgrid, kRadixThreads, 0, ctx->stream>>>(ctx->d_groups, g0, g1, cnt);             \
-            radix_scan_kernel<<<1, kRadixThreads, 0, ctx->stream>>>(cnt, off, cur, rad_nb);                           \
-            radix_scatter_kernel<K_><<<rgrid, kRadixThreads, 0, ctx->stream>>>(ctx->d_groups, g0, g1, cur, d_payload); \
+            radix_count_kernel<K_><<<rgrid, kRadixThreads, 0, ctx->stream.get()>>>(d_groups, g0, g1, cnt);                  \
+            radix_scan_kernel<<<1, kRadixThreads, 0, ctx->stream.get()>>>(cnt, off, cur, rad_nb);                           \
+            radix_scatter_kernel<K_><<<rgrid, kRadixThreads, 0, ctx->stream.get()>>>(d_groups, g0, g1, cur, d_payload.get()); \
         } while (0)
         if (k == 10) PSS_RADIX(10); else if (k == 11) PSS_RADIX(11); else PSS_RADIX(12);
 #undef PSS_RADIX
         if (narrow) {
             cudaFuncSetAttribute(radix_hist_kernel<unsigned int>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
-            radix_hist_kernel<unsigned int><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream>>>(d_payload, off, parts, d_narrow);
+            radix_hist_kernel<unsigned int><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream.get()>>>(d_payload.get(), off, parts, d_narrow.get());
         } else {
             cudaFuncSetAttribute(radix_hist_kernel<unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
-            radix_hist_kernel<unsigned long long><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream>>>(d_payload, off, parts, (unsigned long long *)d_counts);
+            radix_hist_kernel<unsigned long long><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream.get()>>>(d_payload.get(), off, parts, (unsigned long long *)d_counts);
         }
     } else if (g1 > g0 && k >= 7 && k <= 9) {
         // shared-memory bins, 16-bit counters packed two to a word: 65 536 bins per CTA -- one pass for 4^8 bins, four for 4^9
@@ -1036,10 +998,10 @@ int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_s
 #define PSS_SPEC16(K_, CT_, PTR_)                                                                                      \
         do {                                                                                                           \
             cudaFuncSetAttribute(spectrum_smem16_kernel<K_, CT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-            spectrum_smem16_kernel<K_, CT_><<<sg, kSpecSmemThreads, smem, ctx->stream>>>(ctx->d_groups, g0, g1, n_slices, PTR_); \
+            spectrum_smem16_kernel<K_, CT_><<<sg, kSpecSmemThreads, smem, ctx->stream.get()>>>(d_groups, g0, g1, n_slices, PTR_); \
         } while (0)
         if (narrow) {
-            if (k == 7) PSS_SPEC16(7, unsigned int, d_narrow); else if (k == 8) PSS_SPEC16(8, unsigned int, d_narrow); else PSS_SPEC16(9, unsigned int, d_narrow);
+            if (k == 7) PSS_SPEC16(7, unsigned int, d_narrow.get()); else if (k == 8) PSS_SPEC16(8, unsigned int, d_narrow.get()); else PSS_SPEC16(9, unsigned int, d_narrow.get());
         } else {
             unsigned long long *w = (unsigned long long *)d_counts;
             if (k == 7) PSS_SPEC16(7, unsigned long long, w); else if (k == 8) PSS_SPEC16(8, unsigned long long, w); else PSS_SPEC16(9, unsigned long long, w);
@@ -1047,23 +1009,20 @@ int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_s
 #undef PSS_SPEC16
     } else if (g1 > g0) {
         if (narrow) {
-            if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned int><<<grid, 256, 0, ctx->stream>>>(ctx->d_groups, g0, g1, k, d_narrow);
-            else spectrum_kernel<false, unsigned int><<<grid, 256, 0, ctx->stream>>>(ctx->d_groups, g0, g1, k, d_narrow);
+            if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned int><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, d_narrow.get());
+            else spectrum_kernel<false, unsigned int><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, d_narrow.get());
         } else {
-            if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned long long><<<grid, 256, 0, ctx->stream>>>(ctx->d_groups, g0, g1, k, (unsigned long long *)d_counts);
-            else spectrum_kernel<false, unsigned long long><<<grid, 256, 0, ctx->stream>>>(ctx->d_groups, g0, g1, k, (unsigned long long *)d_counts);
+            if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned long long><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, (unsigned long long *)d_counts);
+            else spectrum_kernel<false, unsigned long long><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, (unsigned long long *)d_counts);
         }
     }
     if (narrow) {
         const unsigned wgrid = (unsigned)std::min<uint64_t>((bins + 255) / 256, (uint64_t)ctx->sm_count * 8);
-        widen_kernel<<<wgrid, 256, 0, ctx->stream>>>(d_narrow, (unsigned long long *)d_counts, bins);
+        widen_kernel<<<wgrid, 256, 0, ctx->stream.get()>>>(d_narrow.get(), (unsigned long long *)d_counts, bins);
     }
     time_end(ctx);
     cudaError_t le = cudaGetLastError();
-    cudaError_t se = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d_narrow);
-    cudaFree(d_payload);
-    cudaFree(d_rad);
+    cudaError_t se = cudaStreamSynchronize(ctx->stream.get());
     if (le != cudaSuccess || se != cudaSuccess)
         return fail(ctx, PSSGPU_ECUDA, "kmer_spectrum: %s", cudaGetErrorString(le != cudaSuccess ? le : se));
     time_collect(ctx);
@@ -1076,15 +1035,14 @@ int pssgpu_kmer_spectrum_shard(pssgpu_ctx *ctx, int k, int shard, int n_shards, 
     if (k < 1 || k > kMaxFragK) return fail(ctx, PSSGPU_EUNSUPP, "kmer_spectrum: k %d outside [1,%d]", k, kMaxFragK);
     Bind bind(ctx);
     const size_t bins = 1ull << (2 * k);
-    void *d = nullptr;
-    CU(cudaMalloc(&d, bins * sizeof(uint64_t)));
-    int rc = pssgpu_kmer_spectrum_shard_device(ctx, k, shard, n_shards, d);
+    DevPtr<uint64_t> d;
+    CU(alloc(d, bins * sizeof(uint64_t)));
+    int rc = pssgpu_kmer_spectrum_shard_device(ctx, k, shard, n_shards, d.get());
     if (rc == PSSGPU_OK) {
-        cudaError_t e = cudaMemcpy(counts, d, bins * sizeof(uint64_t), cudaMemcpyDeviceToHost);
+        cudaError_t e = cudaMemcpy(counts, d.get(), bins * sizeof(uint64_t), cudaMemcpyDeviceToHost);
         if (e != cudaSuccess) rc = fail(ctx, PSSGPU_ECUDA, "kmer_spectrum: D2H: %s", cudaGetErrorString(e));
         else ctx->d2h_bytes += bins * sizeof(uint64_t);
     }
-    cudaFree(d);
     return rc;
 }
 
@@ -1095,7 +1053,7 @@ int pssgpu_timing_reset(pssgpu_ctx *ctx, int enable)
 {
     if (!ctx) return PSSGPU_EINVAL;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     time_collect(ctx);
     ctx->timing = enable != 0;
     ctx->launches = ctx->bytes_scanned = ctx->h2d_bytes = ctx->d2h_bytes = 0;
@@ -1107,7 +1065,7 @@ int pssgpu_timing_get(pssgpu_ctx *ctx, pssgpu_timing *out)
 {
     if (!ctx || !out) return PSSGPU_EINVAL;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     time_collect(ctx);
     out->launches = ctx->launches;
     out->kernel_ms = ctx->kernel_ms;
@@ -1122,13 +1080,14 @@ int pssgpu_debug_status(pssgpu_ctx *ctx, int enable)
 {
     if (!ctx) return PSSGPU_EINVAL;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
-    if (enable && !ctx->d_dbg_n) {
-        ctx->dbg_cap = 8ull << 20;
-        CU(cudaMalloc(&ctx->d_dbg_off, ctx->dbg_cap * sizeof(uint64_t)));
-        CU(cudaMalloc(&ctx->d_dbg_code, ctx->dbg_cap));
-        CU(cudaMalloc(&ctx->d_dbg_n, sizeof(unsigned long long)));
-        CU(cudaMemset(ctx->d_dbg_n, 0, sizeof(unsigned long long)));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
+    if (enable && !ctx->dbg_cap) {               // (after a call that failed half way, everything is allocated again)
+        const uint64_t cap = 8ull << 20;
+        CU(alloc(ctx->d_dbg_off, cap * sizeof(uint64_t)));
+        CU(alloc(ctx->d_dbg_code, cap));
+        CU(alloc(ctx->d_dbg_n, sizeof(unsigned long long)));
+        CU(cudaMemset(ctx->d_dbg_n.get(), 0, sizeof(unsigned long long)));
+        ctx->dbg_cap = cap;
     }
     ctx->dbg = enable != 0;
     return PSSGPU_OK;
@@ -1138,15 +1097,15 @@ int pssgpu_debug_fetch(pssgpu_ctx *ctx, uint64_t *offsets, int8_t *codes, uint64
 {
     if (!ctx || !n) return PSSGPU_EINVAL;
     *n = 0;
-    if (!ctx->d_dbg_n) return PSSGPU_OK;
+    if (!ctx->dbg_cap) return PSSGPU_OK;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     unsigned long long have = 0;
-    CU(cudaMemcpy(&have, ctx->d_dbg_n, sizeof have, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&have, ctx->d_dbg_n.get(), sizeof have, cudaMemcpyDeviceToHost));
     if (have > ctx->dbg_cap) have = ctx->dbg_cap;
     const uint64_t take = std::min<uint64_t>(have, cap);
-    if (take && offsets) CU(cudaMemcpy(offsets, ctx->d_dbg_off, take * sizeof(uint64_t), cudaMemcpyDeviceToHost));
-    if (take && codes) CU(cudaMemcpy(codes, ctx->d_dbg_code, take, cudaMemcpyDeviceToHost));
+    if (take && offsets) CU(cudaMemcpy(offsets, ctx->d_dbg_off.get(), take * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    if (take && codes) CU(cudaMemcpy(codes, ctx->d_dbg_code.get(), take, cudaMemcpyDeviceToHost));
     *n = take;
     return PSSGPU_OK;
 }

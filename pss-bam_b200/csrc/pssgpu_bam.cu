@@ -70,38 +70,39 @@ struct BamIngest {
     bool      finished = false;       // `last` seen
     std::string read_group;
     bool      use_rg = false;
-    // device
-    BamState *d_state = nullptr;
-    uint8_t  *d_ubuf = nullptr;       // [0, kBamCarryCap) carry, then the inflated batch
-    uint8_t  *d_text = nullptr;
+    // device, allocated by bam_ensure in two stages: what inflating needs, then what framing needs
+    bool      inflate_ready = false, framing_ready = false;
+    DevPtr<BamState> d_state;
+    DevPtr<uint8_t>  d_ubuf;          // [0, kBamCarryCap) carry, then the inflated batch
+    DevPtr<uint8_t>  d_text;
     size_t    text_cap = 0;
     size_t    batch_comp = 0, batch_u = 0;                       // limits of one batch: compressed / inflated bytes
-    uint8_t  *d_comp[2] = { nullptr, nullptr };                  // compressed staging, double buffered
-    uint32_t *d_loc = nullptr;        // kBamMaxBlocks x kBamLocCap record starts (offsets in ubuf)
-    uint32_t *d_s = nullptr, *d_e = nullptr, *d_n = nullptr;     // per block: guessed start, chain exit, records
+    DevPtr<uint8_t>  d_comp[2];                                  // compressed staging, double buffered
+    DevPtr<uint32_t> d_loc;           // kBamMaxBlocks x kBamLocCap record starts (offsets in ubuf)
+    DevPtr<uint32_t> d_s, d_e, d_n;                              // per block: guessed start, chain exit, records
     // descriptor slots: two when this context inflates its own batches (slot = the staging buffer, ctx->cur), a ring of
     // kBamSlots when helpers inflate for it -- the host must be able to deal as many batches ahead as the helpers can hold
-    BamDesc  *d_desc[kBamSlots] = {};
-    BamDesc  *h_desc[kBamSlots] = {};                            // pinned
-    uint8_t  *h_pfx[kBamSlots] = {};                             // pinned: a BGZF block that arrived in two feed calls
-    cudaEvent_t ev_ring_copied[kBamSlots] = {}, ev_ring_done[kBamSlots] = {};    // ring mode: descriptors copied / batch processed
+    DevPtr<BamDesc>  d_desc[kBamSlots];
+    HostPtr<BamDesc> h_desc[kBamSlots];
+    HostPtr<uint8_t> h_pfx[kBamSlots];                           // a BGZF block that arrived in two feed calls
+    Event     ev_ring_copied[kBamSlots], ev_ring_done[kBamSlots];        // ring mode: descriptors copied / batch processed
     int       ring_slot = 0;
-    uint8_t  *d_hdr = nullptr;        // copy of the BAM header (reference names)
-    uint32_t *d_ref_off = nullptr, *d_ref_len = nullptr;
-    char     *d_rg = nullptr;
-    uint32_t *d_crc_tab = nullptr;    // pss_crc32.h tables; null when $PSSGPU_BAM_CRC=0 switches the check off
+    DevPtr<uint8_t>  d_hdr;           // copy of the BAM header (reference names)
+    DevPtr<uint32_t> d_ref_off, d_ref_len;
+    DevPtr<char>     d_rg;
+    DevPtr<uint32_t> d_crc_tab;       // pss_crc32.h tables; null when $PSSGPU_BAM_CRC=0 switches the check off
     bool      check_crc = true;
     int       rg_len = -1;
     int       inflate_grid = 0;
     uint64_t  batches = 0;
     // several GPUs (pssgpu_group_feed_bam): this context frames, renders and tallies; `helpers` inflate batches for it
     std::vector<pssgpu_ctx *> helpers;
-    std::vector<cudaEvent_t>  ev_fetched;        // per helper: its inflated batch has been copied over (its buffer is free)
+    std::vector<Event>        ev_fetched;        // per helper: its inflated batch has been copied over (its buffer is free)
     std::vector<uint64_t>     helper_batches;
     std::vector<std::array<bool, 2>> helper_busy;  // per helper and staging buffer: a batch dealt there has not been inflated yet
     size_t        deal_start = 0;
     cudaEvent_t   desc_reader[kBamSlots] = {};             // a helper's copy that also reads h_desc[i] (its ev_copied)
-    unsigned int *d_remote_err = nullptr;        // error / error_arg of the helper whose batch was fetched last
+    DevPtr<unsigned int> d_remote_err;           // error / error_arg of the helper whose batch was fetched last
     uint64_t      dealt = 0, own_batches = 0;
 };
 
@@ -459,9 +460,11 @@ static const char *bam_error_text(unsigned code)
     }
 }
 
+void BamDelete::operator()(BamIngest *b) const { delete b; }
+
 void bam_reset(pssgpu_ctx *ctx)
 {
-    BamIngest *B = ctx->bam;
+    BamIngest *B = ctx->bam.get();
     if (!B) return;
     Bind bind(ctx);
     B->carry.clear();
@@ -472,45 +475,26 @@ void bam_reset(pssgpu_ctx *ctx)
     B->ring_slot = 0;
     for (uint64_t &h : B->helper_batches) h = 0;
     for (auto &b : B->helper_busy) b = { false, false };
-    if (B->d_state) {
+    if (B->inflate_ready) {
         BamState z;
         memset(&z, 0, sizeof z);
         z.entry = kBamCarryCap;
-        cudaMemcpyAsync(B->d_state, &z, sizeof z, cudaMemcpyHostToDevice, ctx->stream);
-        cudaStreamSynchronize(ctx->stream);
+        cudaMemcpyAsync(B->d_state.get(), &z, sizeof z, cudaMemcpyHostToDevice, ctx->stream.get());
+        cudaStreamSynchronize(ctx->stream.get());
     }
     for (pssgpu_ctx *h : B->helpers) bam_reset(h);       // their error flags (a helper need not be a member that *_begin reaches)
 }
 
-void bam_destroy(pssgpu_ctx *ctx)
-{
-    BamIngest *B = ctx->bam;
-    if (!B) return;
-    cudaFree(B->d_state); cudaFree(B->d_ubuf); cudaFree(B->d_text); cudaFree(B->d_loc); cudaFree(B->d_comp[0]); cudaFree(B->d_comp[1]);
-    cudaFree(B->d_s); cudaFree(B->d_e); cudaFree(B->d_n);
-    for (int i = 0; i < kBamSlots; i++) {
-        cudaFree(B->d_desc[i]);
-        if (B->h_desc[i]) cudaFreeHost(B->h_desc[i]);
-        if (B->h_pfx[i]) cudaFreeHost(B->h_pfx[i]);
-        if (B->ev_ring_copied[i]) cudaEventDestroy(B->ev_ring_copied[i]);
-        if (B->ev_ring_done[i]) cudaEventDestroy(B->ev_ring_done[i]);
-    }
-    cudaFree(B->d_hdr); cudaFree(B->d_ref_off); cudaFree(B->d_ref_len); cudaFree(B->d_rg); cudaFree(B->d_crc_tab); cudaFree(B->d_remote_err);
-    for (cudaEvent_t e : B->ev_fetched) cudaEventDestroy(e);
-    delete B;
-    ctx->bam = nullptr;
-}
-
 int bam_check(pssgpu_ctx *ctx, bool finishing)
 {
-    BamIngest *B = ctx->bam;
-    if (!B || !B->d_state || B->batches == 0) {
+    BamIngest *B = ctx->bam.get();
+    if (!B || !B->inflate_ready || B->batches == 0) {
         if (B && finishing && !B->carry.empty())
             return fail(ctx, PSSGPU_EINVAL, "BAM ingest: %zu bytes of an incomplete BGZF block pending (feed with last=1)", B->carry.size());
         return PSSGPU_OK;
     }
     BamState s;
-    if (cudaMemcpy(&s, B->d_state, sizeof s, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    if (cudaMemcpy(&s, B->d_state.get(), sizeof s, cudaMemcpyDeviceToHost) != cudaSuccess) {
         cudaGetLastError();
         return fail(ctx, PSSGPU_ECUDA, "BAM ingest: cannot read the device state");
     }
@@ -535,29 +519,30 @@ namespace {
 // batch size) are allocated when the context is first fed a BAM itself
 int bam_ensure(pssgpu_ctx *ctx, bool inflate_only = false)
 {
-    if (!ctx->bam) ctx->bam = new BamIngest();
-    BamIngest *B = ctx->bam;
-    if (!B->d_state) {
+    if (!ctx->bam) ctx->bam.reset(new BamIngest());
+    BamIngest *B = ctx->bam.get();
+    // a stage that failed half way is allocated again from its start: alloc() and create() release what they replace
+    if (!B->inflate_ready) {
         size_t mb = kBamBatchCompDefault >> 20;
         if (const char *e = getenv("PSSGPU_BAM_BATCH_MB")) mb = std::min<size_t>(std::max<size_t>(1, strtoull(e, nullptr, 10)), 512);
         B->batch_comp = mb << 20;
         B->batch_u = 6 * B->batch_comp;                        // a batch also closes when its inflated size reaches this
         B->text_cap = 3 * B->batch_u + (64ull << 20);          // lines are ~1.3 x the record bytes; beyond the cap: error, never silence
-        CU(cudaMalloc(&B->d_ubuf, kBamCarryCap + B->batch_u + (1u << 20)));
-        for (int i = 0; i < 2; i++) CU(cudaMalloc(&B->d_comp[i], B->batch_comp + (128u << 10)));
+        CU(alloc(B->d_ubuf, kBamCarryCap + B->batch_u + (1u << 20)));
+        for (int i = 0; i < 2; i++) CU(alloc(B->d_comp[i], B->batch_comp + (128u << 10)));
         for (int i = 0; i < kBamSlots; i++) {
-            CU(cudaMalloc(&B->d_desc[i], kBamMaxBlocks * sizeof(BamDesc)));
-            CU(cudaMallocHost(&B->h_desc[i], kBamMaxBlocks * sizeof(BamDesc)));
-            CU(cudaMallocHost(&B->h_pfx[i], 65536 + 64));
-            CU(cudaEventCreateWithFlags(&B->ev_ring_copied[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&B->ev_ring_done[i], cudaEventDisableTiming));
+            CU(alloc(B->d_desc[i], kBamMaxBlocks * sizeof(BamDesc)));
+            CU(alloc(B->h_desc[i], kBamMaxBlocks * sizeof(BamDesc)));
+            CU(alloc(B->h_pfx[i], 65536 + 64));
+            CU(create(B->ev_ring_copied[i]));
+            CU(create(B->ev_ring_done[i]));
         }
         if (const char *e = getenv("PSSGPU_BAM_CRC")) B->check_crc = atoi(e) != 0;
         if (B->check_crc) {
             std::vector<uint32_t> tab(kCrcTableWords);
             crc32_build_tables(tab.data());
-            CU(cudaMalloc(&B->d_crc_tab, tab.size() * sizeof(uint32_t)));
-            CU(cudaMemcpy(B->d_crc_tab, tab.data(), tab.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+            CU(alloc(B->d_crc_tab, tab.size() * sizeof(uint32_t)));
+            CU(cudaMemcpy(B->d_crc_tab.get(), tab.data(), tab.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
         }
         const size_t smem = (size_t)kInfWarps * sizeof(InflateTables);
         CU(cudaFuncSetAttribute(bgzf_inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -565,25 +550,27 @@ int bam_ensure(pssgpu_ctx *ctx, bool inflate_only = false)
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bgzf_inflate_kernel, kInfWarps * 32, smem));
         if (occ < 1) return fail(ctx, PSSGPU_ECUDA, "BAM ingest: the inflate kernel does not fit an SM");
         B->inflate_grid = occ * ctx->sm_count;
-        CU(cudaMemset(B->d_ubuf, 0, kBamCarryCap));
+        CU(cudaMemset(B->d_ubuf.get(), 0, kBamCarryCap));
         BamState z;
         memset(&z, 0, sizeof z);
         z.entry = kBamCarryCap;
-        CU(cudaMalloc(&B->d_state, sizeof(BamState)));         // last: d_state != nullptr <=> the inflate part is complete
-        CU(cudaMemcpy(B->d_state, &z, sizeof z, cudaMemcpyHostToDevice));
+        CU(alloc(B->d_state, sizeof(BamState)));
+        CU(cudaMemcpy(B->d_state.get(), &z, sizeof z, cudaMemcpyHostToDevice));
+        B->inflate_ready = true;
     }
-    if (inflate_only || B->d_rg) return PSSGPU_OK;
-    CU(cudaMalloc(&B->d_text, B->text_cap + 4096));
-    CU(cudaMalloc(&B->d_loc, (size_t)kBamMaxBlocks * kBamLocCap * sizeof(uint32_t)));
-    CU(cudaMalloc(&B->d_s, kBamMaxBlocks * sizeof(uint32_t)));
-    CU(cudaMalloc(&B->d_e, kBamMaxBlocks * sizeof(uint32_t)));
-    CU(cudaMalloc(&B->d_n, kBamMaxBlocks * sizeof(uint32_t)));
-    CU(cudaMalloc(&B->d_hdr, kBamCarryCap + 64));
-    CU(cudaMalloc(&B->d_ref_off, (size_t)kBamMaxRefs * sizeof(uint32_t)));
-    CU(cudaMalloc(&B->d_ref_len, (size_t)kBamMaxRefs * sizeof(uint32_t)));
-    CU(cudaMalloc(&B->d_remote_err, 2 * sizeof(unsigned int)));
-    CU(cudaMalloc(&B->d_rg, 256));                             // last: d_rg != nullptr <=> the framing part is complete
-    if (B->use_rg && B->rg_len > 0) CU(cudaMemcpy(B->d_rg, B->read_group.data(), (size_t)B->rg_len, cudaMemcpyHostToDevice));
+    if (inflate_only || B->framing_ready) return PSSGPU_OK;
+    CU(alloc(B->d_text, B->text_cap + 4096));
+    CU(alloc(B->d_loc, (size_t)kBamMaxBlocks * kBamLocCap * sizeof(uint32_t)));
+    CU(alloc(B->d_s, kBamMaxBlocks * sizeof(uint32_t)));
+    CU(alloc(B->d_e, kBamMaxBlocks * sizeof(uint32_t)));
+    CU(alloc(B->d_n, kBamMaxBlocks * sizeof(uint32_t)));
+    CU(alloc(B->d_hdr, kBamCarryCap + 64));
+    CU(alloc(B->d_ref_off, (size_t)kBamMaxRefs * sizeof(uint32_t)));
+    CU(alloc(B->d_ref_len, (size_t)kBamMaxRefs * sizeof(uint32_t)));
+    CU(alloc(B->d_remote_err, 2 * sizeof(unsigned int)));
+    CU(alloc(B->d_rg, 256));
+    if (B->use_rg && B->rg_len > 0) CU(cudaMemcpy(B->d_rg.get(), B->read_group.data(), (size_t)B->rg_len, cudaMemcpyHostToDevice));
+    B->framing_ready = true;
     return PSSGPU_OK;
 }
 
@@ -621,9 +608,9 @@ int bgzf_frame(const uint8_t *p, size_t n, uint32_t *total, uint32_t *pay_off, u
 struct BamSlot { int i; cudaEvent_t copied, done; };
 BamSlot bam_slot(pssgpu_ctx *ctx)
 {
-    BamIngest *B = ctx->bam;
-    if (B->helpers.empty()) return BamSlot{ ctx->cur, ctx->ev_copied[ctx->cur], ctx->ev_tallied[ctx->cur] };
-    return BamSlot{ B->ring_slot, B->ev_ring_copied[B->ring_slot], B->ev_ring_done[B->ring_slot] };
+    BamIngest *B = ctx->bam.get();
+    if (B->helpers.empty()) return BamSlot{ ctx->cur, ctx->ev_copied[ctx->cur].get(), ctx->ev_tallied[ctx->cur].get() };
+    return BamSlot{ B->ring_slot, B->ev_ring_copied[B->ring_slot].get(), B->ev_ring_done[B->ring_slot].get() };
 }
 
 // compressed bytes + block descriptors -> W's staging buffers, inflate on W's stream into W's inflated buffer; `desc` is
@@ -632,21 +619,21 @@ int bam_stage_and_inflate(pssgpu_ctx *W, const uint8_t *pfx, size_t pfx_len, con
                           uint32_t n_blocks)
 {
     pssgpu_ctx *ctx = W;                                   // (the CU macro reports through `ctx`)
-    BamIngest  *B = W->bam;
+    BamIngest  *B = W->bam.get();
     const int   cur = W->cur;
     // pfx: a block that arrived in two feed calls (pinned copy), in front of the blocks that lie in the caller's buffer
-    if (pfx_len) CU(cudaMemcpyAsync(B->d_comp[cur], pfx, pfx_len, cudaMemcpyHostToDevice, W->copy_stream));
-    if (comp_len) CU(cudaMemcpyAsync(B->d_comp[cur] + pfx_len, src, comp_len, cudaMemcpyHostToDevice, W->copy_stream));
-    CU(cudaMemcpyAsync(B->d_desc[cur], desc, n_blocks * sizeof(BamDesc), cudaMemcpyHostToDevice, W->copy_stream));
+    if (pfx_len) CU(cudaMemcpyAsync(B->d_comp[cur].get(), pfx, pfx_len, cudaMemcpyHostToDevice, W->copy_stream.get()));
+    if (comp_len) CU(cudaMemcpyAsync(B->d_comp[cur].get() + pfx_len, src, comp_len, cudaMemcpyHostToDevice, W->copy_stream.get()));
+    CU(cudaMemcpyAsync(B->d_desc[cur].get(), desc, n_blocks * sizeof(BamDesc), cudaMemcpyHostToDevice, W->copy_stream.get()));
     W->h2d_bytes += pfx_len + comp_len;
-    CU(cudaEventRecord(W->ev_copied[cur], W->copy_stream));
-    CU(cudaStreamWaitEvent(W->stream, W->ev_copied[cur], 0));
-    cudaStream_t st = W->stream;
+    CU(cudaEventRecord(W->ev_copied[cur].get(), W->copy_stream.get()));
+    CU(cudaStreamWaitEvent(W->stream.get(), W->ev_copied[cur].get(), 0));
+    cudaStream_t st = W->stream.get();
     CU(cudaMemsetAsync(&B->d_state->work_ctr, 0, sizeof(unsigned int), st));
     const size_t   smem = (size_t)kInfWarps * sizeof(InflateTables);
     const unsigned grid = (unsigned)std::min<uint64_t>((n_blocks + kInfWarps - 1) / kInfWarps, (uint64_t)B->inflate_grid);
     time_begin(W, pfx_len + comp_len);
-    bgzf_inflate_kernel<<<grid, kInfWarps * 32, smem, st>>>(B->d_desc[cur], n_blocks, B->d_comp[cur], B->d_ubuf + kBamCarryCap, B->d_state, B->d_crc_tab);
+    bgzf_inflate_kernel<<<grid, kInfWarps * 32, smem, st>>>(B->d_desc[cur].get(), n_blocks, B->d_comp[cur].get(), B->d_ubuf.get() + kBamCarryCap, B->d_state.get(), B->d_crc_tab.get());
     time_end(W);
     CU(cudaGetLastError());
     return PSSGPU_OK;
@@ -658,12 +645,12 @@ int bam_stage_and_inflate(pssgpu_ctx *W, const uint8_t *pfx, size_t pfx_len, con
 int bam_submit(pssgpu_ctx *ctx, const uint8_t *pfx, size_t pfx_len, const uint8_t *src, size_t comp_len, uint32_t n_blocks, uint64_t total_u,
                int is_last, bool may_deal = false)
 {
-    BamIngest *B = ctx->bam;
+    BamIngest *B = ctx->bam.get();
     const bool    ring = !B->helpers.empty();
     const BamSlot slot = bam_slot(ctx);
     const int     cur = slot.i;
-    cudaStream_t st = ctx->stream;
-    BamState    *S = B->d_state;
+    cudaStream_t st = ctx->stream.get();
+    BamState    *S = B->d_state.get();
     int          hi = -1;                                  // helper that inflates this batch
     if (n_blocks && may_deal && !B->helpers.empty()) {
         // the helper with the fewest batches in flight (staged or inflating: at most two, its staging is double buffered);
@@ -676,7 +663,7 @@ int bam_submit(pssgpu_ctx *ctx, const uint8_t *pfx, size_t pfx_len, const uint8_
             pssgpu_ctx  *W = B->helpers[h];
             int          fl = 0;
             for (int b = 0; b < 2; b++) {
-                if (B->helper_busy[h][b] && cudaEventQuery(W->ev_tallied[b]) == cudaSuccess) B->helper_busy[h][b] = false;
+                if (B->helper_busy[h][b] && cudaEventQuery(W->ev_tallied[b].get()) == cudaSuccess) B->helper_busy[h][b] = false;
                 fl += B->helper_busy[h][b] ? 1 : 0;
             }
             cudaGetLastError();                            // (cudaErrorNotReady is an answer, not an error)
@@ -690,78 +677,78 @@ int bam_submit(pssgpu_ctx *ctx, const uint8_t *pfx, size_t pfx_len, const uint8_
     B->desc_reader[cur] = nullptr;
     if (hi < 0) {
         if (n_blocks) {
-            int rc = bam_stage_and_inflate(ctx, pfx, pfx_len, src, comp_len, B->h_desc[cur], n_blocks);
+            int rc = bam_stage_and_inflate(ctx, pfx, pfx_len, src, comp_len, B->h_desc[cur].get(), n_blocks);
             if (rc != PSSGPU_OK) return rc;
             B->own_batches++;
         } else {
-            CU(cudaEventRecord(slot.copied, ctx->copy_stream));
+            CU(cudaEventRecord(slot.copied, ctx->copy_stream.get()));
             CU(cudaStreamWaitEvent(st, slot.copied, 0));
         }
     } else {
         pssgpu_ctx *W = B->helpers[hi];
-        BamIngest  *Bw = W->bam;
+        BamIngest  *Bw = W->bam.get();
         const int   wc = W->cur;
         {
             Bind bind(W);
             // the helper's inflated buffer is free once its previous batch has been fetched
             if (B->helper_batches[hi]) {
-                if (cudaStreamWaitEvent(W->stream, B->ev_fetched[hi], 0) != cudaSuccess)
+                if (cudaStreamWaitEvent(W->stream.get(), B->ev_fetched[hi].get(), 0) != cudaSuccess)
                     return fail(ctx, PSSGPU_ECUDA, "feed_bam: GPU %d cannot wait for GPU %d", W->device, ctx->device);
             }
-            int rc = bam_stage_and_inflate(W, pfx, pfx_len, src, comp_len, B->h_desc[cur], n_blocks);
-            if (rc == PSSGPU_OK && cudaEventRecord(W->ev_tallied[wc], W->stream) != cudaSuccess) rc = PSSGPU_ECUDA;      // "inflated"
+            int rc = bam_stage_and_inflate(W, pfx, pfx_len, src, comp_len, B->h_desc[cur].get(), n_blocks);
+            if (rc == PSSGPU_OK && cudaEventRecord(W->ev_tallied[wc].get(), W->stream.get()) != cudaSuccess) rc = PSSGPU_ECUDA;      // "inflated"
             W->cur ^= 1;
             // its other staging buffer is free once the batch that used it has been inflated
-            if (rc == PSSGPU_OK && cudaStreamWaitEvent(W->copy_stream, W->ev_tallied[W->cur], 0) != cudaSuccess) rc = PSSGPU_ECUDA;
+            if (rc == PSSGPU_OK && cudaStreamWaitEvent(W->copy_stream.get(), W->ev_tallied[W->cur].get(), 0) != cudaSuccess) rc = PSSGPU_ECUDA;
             if (rc != PSSGPU_OK) return fail(ctx, rc, "feed_bam: inflate on GPU %d: %s", W->device, pssgpu_last_error(W));
         }
-        B->desc_reader[cur] = W->ev_copied[wc];
+        B->desc_reader[cur] = W->ev_copied[wc].get();
         B->helper_busy[hi][wc] = true;
         B->helper_batches[hi]++;
         // this GPU: the descriptors, then -- once the helper is done -- the inflated bytes and its error flag over NVLink
-        CU(cudaMemcpyAsync(B->d_desc[cur], B->h_desc[cur], n_blocks * sizeof(BamDesc), cudaMemcpyHostToDevice, ctx->copy_stream));
-        CU(cudaEventRecord(slot.copied, ctx->copy_stream));
+        CU(cudaMemcpyAsync(B->d_desc[cur].get(), B->h_desc[cur].get(), n_blocks * sizeof(BamDesc), cudaMemcpyHostToDevice, ctx->copy_stream.get()));
+        CU(cudaEventRecord(slot.copied, ctx->copy_stream.get()));
         CU(cudaStreamWaitEvent(st, slot.copied, 0));
-        CU(cudaStreamWaitEvent(st, W->ev_tallied[wc], 0));
-        CU(cudaMemcpyPeerAsync(B->d_ubuf + kBamCarryCap, ctx->device, Bw->d_ubuf + kBamCarryCap, W->device, total_u, st));
-        CU(cudaMemcpyPeerAsync(B->d_remote_err, ctx->device, &Bw->d_state->error, W->device, 2 * sizeof(unsigned int), st));
-        CU(cudaEventRecord(B->ev_fetched[hi], st));
-        bam_merge_error_kernel<<<1, 1, 0, st>>>(S, B->d_remote_err);
+        CU(cudaStreamWaitEvent(st, W->ev_tallied[wc].get(), 0));
+        CU(cudaMemcpyPeerAsync(B->d_ubuf.get() + kBamCarryCap, ctx->device, Bw->d_ubuf.get() + kBamCarryCap, W->device, total_u, st));
+        CU(cudaMemcpyPeerAsync(B->d_remote_err.get(), ctx->device, &Bw->d_state->error, W->device, 2 * sizeof(unsigned int), st));
+        CU(cudaEventRecord(B->ev_fetched[hi].get(), st));
+        bam_merge_error_kernel<<<1, 1, 0, st>>>(S, B->d_remote_err.get());
     }
-    bam_prepare_kernel<<<1, 32, 0, st>>>(S, B->d_ubuf, total_u, B->d_hdr, B->d_ref_off, B->d_ref_len);
+    bam_prepare_kernel<<<1, 32, 0, st>>>(S, B->d_ubuf.get(), total_u, B->d_hdr.get(), B->d_ref_off.get(), B->d_ref_len.get());
     if (n_blocks) {
-        bam_guess_kernel<<<(n_blocks + 3) / 4, 128, 0, st>>>(B->d_desc[cur], n_blocks, B->d_ubuf, S, B->d_loc, B->d_s, B->d_e, B->d_n);
+        bam_guess_kernel<<<(n_blocks + 3) / 4, 128, 0, st>>>(B->d_desc[cur].get(), n_blocks, B->d_ubuf.get(), S, B->d_loc.get(), B->d_s.get(), B->d_e.get(), B->d_n.get());
     }
-    bam_fix_kernel<<<1, 32, 0, st>>>(B->d_desc[cur], n_blocks, B->d_ubuf, S, B->d_loc, B->d_s, B->d_e, B->d_n, is_last);
+    bam_fix_kernel<<<1, 32, 0, st>>>(B->d_desc[cur].get(), n_blocks, B->d_ubuf.get(), S, B->d_loc.get(), B->d_s.get(), B->d_e.get(), B->d_n.get(), is_last);
     if (n_blocks) {
         BamRefs refs;
-        refs.blob = B->d_hdr; refs.name_off = B->d_ref_off; refs.name_len = B->d_ref_len; refs.n_ref = 0;
+        refs.blob = B->d_hdr.get(); refs.name_off = B->d_ref_off.get(); refs.name_len = B->d_ref_len.get(); refs.n_ref = 0;
         time_begin(ctx, total_u);
-        bam_render_kernel<<<n_blocks, 128, 0, st>>>(B->d_ubuf, S, B->d_loc, B->d_n, refs, B->d_rg, B->use_rg ? B->rg_len : -1,
-                                                    B->d_text, B->text_cap);
+        bam_render_kernel<<<n_blocks, 128, 0, st>>>(B->d_ubuf.get(), S, B->d_loc.get(), B->d_n.get(), refs, B->d_rg.get(), B->use_rg ? B->rg_len : -1,
+                                                    B->d_text.get(), B->text_cap);
         time_end(ctx);
     }
-    bam_carry_kernel<<<1, 256, 0, st>>>(B->d_ubuf, S);
+    bam_carry_kernel<<<1, 256, 0, st>>>(B->d_ubuf.get(), S);
     CU(cudaGetLastError());
     if (n_blocks) {
         // the text of this batch: at most text_cap bytes, the real length is in the device state
         const size_t bound = std::min<size_t>(B->text_cap, (size_t)(total_u + (1u << 20)) * 3 / 2);
-        int rc = launch_tally_mode(ctx, B->d_text, bound, ctx->fed_bytes, &S->text_len);
+        int rc = launch_tally_mode(ctx, B->d_text.get(), bound, ctx->fed_bytes, &S->text_len);
         if (rc != PSSGPU_OK) return rc;
     }
-    CU(cudaEventRecord(slot.done, ctx->stream));
+    CU(cudaEventRecord(slot.done, ctx->stream.get()));
     if (ring) B->ring_slot = (cur + 1) % kBamSlots;
     else ctx->cur ^= 1;
     // the next staging buffer / descriptor slot is free once the batch that used it has been inflated; the simple,
     // sufficient condition: that whole batch is done
-    CU(cudaStreamWaitEvent(ctx->copy_stream, bam_slot(ctx).done, 0));
+    CU(cudaStreamWaitEvent(ctx->copy_stream.get(), bam_slot(ctx).done, 0));
     B->batches++;
     return PSSGPU_OK;
 }
 
 int feed_bam_impl(pssgpu_ctx *ctx, const uint8_t *data, size_t len, int last)
 {
-    BamIngest *B = ctx->bam;
+    BamIngest *B = ctx->bam.get();
     if (B->finished && len) return fail(ctx, PSSGPU_EINVAL, "feed_bam: data after last=1");
     size_t off = 0;
     // a block left incomplete by the previous call is completed in the carry buffer
@@ -796,13 +783,13 @@ int feed_bam_impl(pssgpu_ctx *ctx, const uint8_t *data, size_t len, int last)
         const int     cur = slot.i;
         CU(cudaEventSynchronize(slot.copied));                      // h_desc[cur] / h_pfx[cur] are free again
         if (B->desc_reader[cur]) CU(cudaEventSynchronize(B->desc_reader[cur]));      // ... also on the GPU that inflated that batch
-        BamDesc *desc = B->h_desc[cur];
+        BamDesc *desc = B->h_desc[cur].get();
         const size_t start = off;
         uint32_t n_blocks = 0, pfx_len = 0;
         uint64_t total_u = 0;
         bool     more = true;
         if (pfx_pending) {
-            memcpy(B->h_pfx[cur], B->carry.data(), pfx_total);
+            memcpy(B->h_pfx[cur].get(), B->carry.data(), pfx_total);
             B->carry.clear();
             desc[n_blocks++] = BamDesc{ pfx_po, pfx_pl, 0u, pfx_isz };
             total_u = pfx_isz;
@@ -822,7 +809,7 @@ int feed_bam_impl(pssgpu_ctx *ctx, const uint8_t *data, size_t len, int last)
             off += total;
         }
         if (n_blocks) {
-            int rc = bam_submit(ctx, B->h_pfx[cur], pfx_len, data + start, off - start, n_blocks, total_u, 0, true);
+            int rc = bam_submit(ctx, B->h_pfx[cur].get(), pfx_len, data + start, off - start, n_blocks, total_u, 0, true);
             if (rc != PSSGPU_OK) return rc;
         }
         if (!more) {                                     // an incomplete block at the end of this call
@@ -851,7 +838,7 @@ int bam_set_helpers(pssgpu_ctx *ctx, const std::vector<pssgpu_ctx *> &helpers)
         int  rc = bam_ensure(ctx);
         if (rc != PSSGPU_OK) return rc;
     }
-    BamIngest *B = ctx->bam;
+    BamIngest *B = ctx->bam.get();
     if (B->helpers == helpers) return PSSGPU_OK;
     if (B->batches) return fail(ctx, PSSGPU_EINVAL, "feed_bam: the GPUs of a stream cannot change while it is fed");
     for (pssgpu_ctx *h : helpers) {
@@ -872,9 +859,9 @@ int bam_set_helpers(pssgpu_ctx *ctx, const std::vector<pssgpu_ctx *> &helpers)
             if (cudaDeviceCanAccessPeer(&can, ctx->device, h->device) == cudaSuccess && can) cudaDeviceEnablePeerAccess(h->device, 0);
             cudaGetLastError();
         }
-    for (cudaEvent_t e : B->ev_fetched) cudaEventDestroy(e);
-    B->ev_fetched.assign(helpers.size(), nullptr);
-    for (cudaEvent_t &e : B->ev_fetched) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    B->ev_fetched.clear();
+    B->ev_fetched.resize(helpers.size());
+    for (Event &e : B->ev_fetched) CU(create(e));
     B->helper_batches.assign(helpers.size(), 0);
     B->helper_busy.assign(helpers.size(), std::array<bool, 2>{ false, false });
     B->deal_start = 0;
@@ -885,7 +872,7 @@ int bam_set_helpers(pssgpu_ctx *ctx, const std::vector<pssgpu_ctx *> &helpers)
 // batches inflated on the context's own GPU, and on every helper, since *_begin
 void bam_dealing(pssgpu_ctx *ctx, uint64_t *own, std::vector<uint64_t> *per_helper)
 {
-    BamIngest *B = ctx->bam;
+    BamIngest *B = ctx->bam.get();
     *own = B ? B->own_batches : 0;
     if (B) *per_helper = B->helper_batches; else per_helper->clear();
 }
@@ -902,15 +889,15 @@ int pssgpu_bam_read_group(pssgpu_ctx *ctx, const char *read_group)
     Bind bind(ctx);
     int rc = bam_ensure(ctx);
     if (rc != PSSGPU_OK) return rc;
-    BamIngest *B = ctx->bam;
-    CU(cudaStreamSynchronize(ctx->stream));
+    BamIngest *B = ctx->bam.get();
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     if (!read_group) { B->use_rg = false; B->read_group.clear(); B->rg_len = -1; return PSSGPU_OK; }
     const size_t n = strlen(read_group);
     if (n > 255) return fail(ctx, PSSGPU_EUNSUPP, "read group name longer than 255 bytes");
     B->read_group = read_group;
     B->use_rg = true;
     B->rg_len = (int)n;
-    if (n) CU(cudaMemcpy(B->d_rg, read_group, n, cudaMemcpyHostToDevice));
+    if (n) CU(cudaMemcpy(B->d_rg.get(), read_group, n, cudaMemcpyHostToDevice));
     return PSSGPU_OK;
 }
 
@@ -923,9 +910,9 @@ int pssgpu_feed_bam(pssgpu_ctx *ctx, const void *bgzf_bytes, size_t len, int las
     int rc = bam_ensure(ctx);
     if (rc == PSSGPU_OK) rc = feed_bam_impl(ctx, (const uint8_t *)bgzf_bytes, len, last);
     // like pssgpu_feed: the caller's bytes have been copied when we return, the kernels may still run
-    cudaError_t e = cudaStreamSynchronize(ctx->copy_stream);
+    cudaError_t e = cudaStreamSynchronize(ctx->copy_stream.get());
     for (pssgpu_ctx *h : ctx->bam ? ctx->bam->helpers : std::vector<pssgpu_ctx *>()) {
-        const cudaError_t eh = cudaStreamSynchronize(h->copy_stream);
+        const cudaError_t eh = cudaStreamSynchronize(h->copy_stream.get());
         if (e == cudaSuccess) e = eh;
     }
     if (rc != PSSGPU_OK) return rc;
@@ -937,12 +924,12 @@ int pssgpu_bam_info(pssgpu_ctx *ctx, pssgpu_bam_stats *out)
 {
     if (!ctx || !out) return PSSGPU_EINVAL;
     memset(out, 0, sizeof *out);
-    BamIngest *B = ctx->bam;
-    if (!B || !B->d_state) return PSSGPU_OK;
+    BamIngest *B = ctx->bam.get();
+    if (!B || !B->inflate_ready) return PSSGPU_OK;
     Bind bind(ctx);
-    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream.get()));
     BamState s;
-    CU(cudaMemcpy(&s, B->d_state, sizeof s, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&s, B->d_state.get(), sizeof s, cudaMemcpyDeviceToHost));
     out->records = s.n_records;
     out->dropped_by_read_group = s.n_dropped;
     out->references = s.hdr_done ? (uint64_t)s.n_ref : 0;

@@ -49,6 +49,9 @@ struct Nccl {
 };
 constexpr int kNcclUint64 = 5, kNcclSum = 0;      // nccl.h: ncclUint64, ncclSum
 
+struct CtxDestroy { void operator()(pssgpu_ctx *c) const { pssgpu_destroy(c); } };
+using CtxPtr = std::unique_ptr<pssgpu_ctx, CtxDestroy>;
+
 __global__ void add_u64_kernel(unsigned long long *__restrict__ acc, const unsigned long long *__restrict__ x, size_t n)
 {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) acc[i] += x[i];
@@ -57,16 +60,16 @@ __global__ void add_u64_kernel(unsigned long long *__restrict__ acc, const unsig
 }  // namespace
 
 struct pssgpu_group {
-    std::vector<pssgpu_ctx *> ctx;
+    std::vector<CtxPtr>       ctx;
     std::vector<int>          dev;
     std::vector<ncclComm_t>   comm;
-    std::vector<unsigned long long *> d_red;       // per GPU: reduction buffer
+    std::vector<DevPtr<unsigned long long>> d_red;  // per GPU: reduction buffer (released under its member's Bind)
     size_t      red_cap = 0;                        // elements
     Nccl        nccl;
     bool        use_nccl = false;
     std::string err;
     size_t      next = 0;                           // round-robin cursor of pssgpu_group_feed
-    pssgpu_ctx *bam_self = nullptr;                 // pssgpu_group_feed_bam: a second context on the first GPU that only inflates
+    CtxPtr      bam_self;                           // pssgpu_group_feed_bam: a second context on the first GPU that only inflates
     double      last_reduce_ms = 0.0;
 };
 
@@ -84,17 +87,15 @@ int gfail(pssgpu_group *g, int code, const char *fmt, ...)
 }
 int member_fail(pssgpu_group *g, int i, int rc)
 {
-    return gfail(g, rc, "GPU %d: %s", g->dev[i], pssgpu_last_error(g->ctx[i]));
+    return gfail(g, rc, "GPU %d: %s", g->dev[i], pssgpu_last_error(g->ctx[i].get()));
 }
 
 int ensure_red(pssgpu_group *g, size_t elems)
 {
     if (elems <= g->red_cap) return PSSGPU_OK;
     for (size_t i = 0; i < g->ctx.size(); i++) {
-        Bind bind(g->ctx[i]);
-        cudaFree(g->d_red[i]);
-        g->d_red[i] = nullptr;
-        if (cudaMalloc(&g->d_red[i], elems * sizeof(unsigned long long)) != cudaSuccess) {
+        Bind bind(g->ctx[i].get());
+        if (alloc(g->d_red[i], elems * sizeof(unsigned long long)) != cudaSuccess) {
             cudaGetLastError();
             g->red_cap = 0;
             return gfail(g, PSSGPU_ENOMEM, "group: cannot allocate the reduction buffer on GPU %d", g->dev[i]);
@@ -109,53 +110,46 @@ int reduce_sum(pssgpu_group *g, size_t elems)
 {
     const size_t n = g->ctx.size();
     if (n == 1) return PSSGPU_OK;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    {
-        Bind bind(g->ctx[0]);
-        cudaEventCreate(&e0); cudaEventCreate(&e1);
-        cudaEventRecord(e0, g->ctx[0]->stream);
-    }
+    Bind bind0(g->ctx[0].get());                    // the timing events and the peer scratch live on the first GPU
+    Event e0, e1;
+    create(e0, cudaEventDefault);
+    create(e1, cudaEventDefault);
+    cudaEventRecord(e0.get(), g->ctx[0]->stream.get());
     int rc = PSSGPU_OK;
     if (g->use_nccl) {
         int r = g->nccl.GroupStart();
         for (size_t i = 0; i < n && r == 0; i++) {
-            Bind bind(g->ctx[i]);
-            r = g->nccl.AllReduce(g->d_red[i], g->d_red[i], elems, kNcclUint64, kNcclSum, g->comm[i], g->ctx[i]->stream);
+            Bind bind(g->ctx[i].get());
+            r = g->nccl.AllReduce(g->d_red[i].get(), g->d_red[i].get(), elems, kNcclUint64, kNcclSum, g->comm[i], g->ctx[i]->stream.get());
         }
         const int r2 = g->nccl.GroupEnd();
         if (r == 0) r = r2;
         if (r != 0) rc = gfail(g, PSSGPU_ECUDA, "group: ncclAllReduce: %s", g->nccl.GetErrorString(r));
     } else {
         // peer copies into a scratch area behind the first GPU's own table, added there one by one
-        Bind bind(g->ctx[0]);
-        unsigned long long *tmp = nullptr;
-        if (cudaMalloc(&tmp, elems * sizeof(unsigned long long)) != cudaSuccess) { cudaGetLastError(); rc = gfail(g, PSSGPU_ENOMEM, "group: scratch for the peer reduction"); }
+        DevPtr<unsigned long long> tmp;
+        if (alloc(tmp, elems * sizeof(unsigned long long)) != cudaSuccess) { cudaGetLastError(); rc = gfail(g, PSSGPU_ENOMEM, "group: scratch for the peer reduction"); }
         for (size_t i = 1; i < n && rc == PSSGPU_OK; i++) {
-            cudaStreamSynchronize(g->ctx[i]->stream);
-            cudaError_t e = cudaMemcpyPeerAsync(tmp, g->dev[0], g->d_red[i], g->dev[i], elems * sizeof(unsigned long long), g->ctx[0]->stream);
+            cudaStreamSynchronize(g->ctx[i]->stream.get());
+            cudaError_t e = cudaMemcpyPeerAsync(tmp.get(), g->dev[0], g->d_red[i].get(), g->dev[i], elems * sizeof(unsigned long long), g->ctx[0]->stream.get());
             if (e == cudaSuccess) {
                 const unsigned grid = (unsigned)std::min<size_t>((elems + 255) / 256, (size_t)g->ctx[0]->sm_count * 8);
-                add_u64_kernel<<<grid, 256, 0, g->ctx[0]->stream>>>(g->d_red[0], tmp, elems);
+                add_u64_kernel<<<grid, 256, 0, g->ctx[0]->stream.get()>>>(g->d_red[0].get(), tmp.get(), elems);
                 e = cudaGetLastError();
             }
             if (e != cudaSuccess) rc = gfail(g, PSSGPU_ECUDA, "group: peer reduction: %s", cudaGetErrorString(e));
         }
-        cudaStreamSynchronize(g->ctx[0]->stream);
-        cudaFree(tmp);
+        cudaStreamSynchronize(g->ctx[0]->stream.get());      // before tmp is released
     }
     for (size_t i = 0; i < n; i++) {
-        Bind bind(g->ctx[i]);
-        if (cudaStreamSynchronize(g->ctx[i]->stream) != cudaSuccess && rc == PSSGPU_OK)
+        Bind bind(g->ctx[i].get());
+        if (cudaStreamSynchronize(g->ctx[i]->stream.get()) != cudaSuccess && rc == PSSGPU_OK)
             rc = gfail(g, PSSGPU_ECUDA, "group: reduction failed on GPU %d: %s", g->dev[i], cudaGetErrorString(cudaGetLastError()));
     }
-    {
-        Bind bind(g->ctx[0]);
-        cudaEventRecord(e1, g->ctx[0]->stream);
-        cudaEventSynchronize(e1);
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, e0, e1) == cudaSuccess) g->last_reduce_ms = ms;
-        cudaEventDestroy(e0); cudaEventDestroy(e1);
-    }
+    cudaEventRecord(e1.get(), g->ctx[0]->stream.get());
+    cudaEventSynchronize(e1.get());
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, e0.get(), e1.get()) == cudaSuccess) g->last_reduce_ms = ms;
     return rc;
 }
 
@@ -169,13 +163,13 @@ int gather_sum(pssgpu_group *g, size_t elems, Fill fill, uint64_t *host_out)
     int rc = ensure_red(g, elems);
     if (rc != PSSGPU_OK) return rc;
     for (size_t i = 0; i < g->ctx.size(); i++) {
-        rc = fill(g->ctx[i], g->d_red[i]);
+        rc = fill(g->ctx[i].get(), g->d_red[i].get());
         if (rc != PSSGPU_OK) return member_fail(g, (int)i, rc);
     }
     rc = reduce_sum(g, elems);
     if (rc != PSSGPU_OK) return rc;
-    Bind bind(g->ctx[0]);
-    if (cudaMemcpy(host_out, g->d_red[0], elems * sizeof(uint64_t), cudaMemcpyDeviceToHost) != cudaSuccess)
+    Bind bind(g->ctx[0].get());
+    if (cudaMemcpy(host_out, g->d_red[0].get(), elems * sizeof(uint64_t), cudaMemcpyDeviceToHost) != cudaSuccess)
         return gfail(g, PSSGPU_ECUDA, "group: D2H of the summed tables: %s", cudaGetErrorString(cudaGetLastError()));
     return PSSGPU_OK;
 }
@@ -203,19 +197,15 @@ int pssgpu_group_init(const int *devices, int n, pssgpu_group **out)
                 if (!allow_dup) return fail(nullptr, PSSGPU_EINVAL, "pssgpu_group_init: device %d listed twice", dev[i]);
                 has_dup = true;
             }
-    pssgpu_group *g = new pssgpu_group();
+    std::unique_ptr<pssgpu_group> g(new pssgpu_group());      // on failure its members are destroyed with it
     g->dev = dev;
     for (int d : dev) {
         pssgpu_ctx *c = nullptr;
         const int rc = pssgpu_init(d, &c);
-        if (rc != PSSGPU_OK) {                       // pssgpu_last_error(NULL) holds the reason
-            for (pssgpu_ctx *m : g->ctx) pssgpu_destroy(m);
-            delete g;
-            return rc;
-        }
-        g->ctx.push_back(c);
+        if (rc != PSSGPU_OK) return rc;              // pssgpu_last_error(NULL) holds the reason
+        g->ctx.emplace_back(c);
     }
-    g->d_red.assign(dev.size(), nullptr);
+    g->d_red.resize(dev.size());
     const char *mode = getenv("PSSGPU_GROUP_REDUCE");
     if (dev.size() > 1 && !has_dup && !(mode && strcmp(mode, "peer") == 0) && g->nccl.load()) {
         g->comm.assign(dev.size(), nullptr);
@@ -232,14 +222,14 @@ int pssgpu_group_init(const int *devices, int n, pssgpu_group **out)
     }
     if (dev.size() > 1 && !g->use_nccl) {
         // the peer path: the first GPU reads the others' tables
-        Bind bind(g->ctx[0]);
+        Bind bind(g->ctx[0].get());
         for (size_t i = 1; i < dev.size(); i++) {
             int can = 0;
             if (dev[i] != dev[0]) cudaDeviceCanAccessPeer(&can, dev[0], dev[i]);
             if (can && cudaDeviceEnablePeerAccess(dev[i], 0) != cudaSuccess) cudaGetLastError();      // (already enabled is fine; without it the copy is staged)
         }
     }
-    *out = g;
+    *out = g.release();
     return PSSGPU_OK;
 }
 
@@ -247,19 +237,18 @@ void pssgpu_group_destroy(pssgpu_group *g)
 {
     if (!g) return;
     if (g->bam_self) {
-        for (pssgpu_ctx *c : g->ctx) { Bind bind(c); cudaStreamSynchronize(c->stream); }      // (they may wait on its events)
-        pssgpu_destroy(g->bam_self);
+        for (CtxPtr &c : g->ctx) { Bind bind(c.get()); cudaStreamSynchronize(c->stream.get()); }      // (they may wait on its events)
+        g->bam_self.reset();
     }
     for (size_t i = 0; i < g->ctx.size(); i++) {
-        { Bind bind(g->ctx[i]); cudaStreamSynchronize(g->ctx[i]->stream); cudaFree(g->d_red[i]); }
+        { Bind bind(g->ctx[i].get()); cudaStreamSynchronize(g->ctx[i]->stream.get()); g->d_red[i].reset(); }
         if (g->use_nccl && g->comm[i]) g->nccl.CommDestroy(g->comm[i]);
     }
-    for (pssgpu_ctx *c : g->ctx) pssgpu_destroy(c);
-    delete g;
+    delete g;                                        // then the member contexts
 }
 
 int         pssgpu_group_size(const pssgpu_group *g) { return g ? (int)g->ctx.size() : 0; }
-pssgpu_ctx *pssgpu_group_ctx(pssgpu_group *g, int i) { return (g && i >= 0 && (size_t)i < g->ctx.size()) ? g->ctx[i] : nullptr; }
+pssgpu_ctx *pssgpu_group_ctx(pssgpu_group *g, int i) { return (g && i >= 0 && (size_t)i < g->ctx.size()) ? g->ctx[i].get() : nullptr; }
 const char *pssgpu_group_last_error(const pssgpu_group *g) { return g ? g->err.c_str() : pssgpu_last_error(nullptr); }
 const char *pssgpu_group_reduce_backend(const pssgpu_group *g)
 {
@@ -274,7 +263,7 @@ int pssgpu_group_genome_upload(pssgpu_group *g, const pssgpu_contig *contigs, ui
     std::vector<int> rc(g->ctx.size(), PSSGPU_OK);
     std::vector<std::thread> th;
     for (size_t i = 0; i < g->ctx.size(); i++)
-        th.emplace_back([&, i]() { rc[i] = pssgpu_genome_upload(g->ctx[i], contigs, n_contigs); });
+        th.emplace_back([&, i]() { rc[i] = pssgpu_genome_upload(g->ctx[i].get(), contigs, n_contigs); });
     for (auto &t : th) t.join();
     for (size_t i = 0; i < rc.size(); i++)
         if (rc[i] != PSSGPU_OK) return member_fail(g, (int)i, rc[i]);
@@ -285,7 +274,7 @@ int pssgpu_group_genome_load_tagged(pssgpu_group *g, const char *path, const pss
 {
     if (!g) return PSSGPU_EINVAL;
     for (size_t i = 0; i < g->ctx.size(); i++) {
-        const int rc = pssgpu_genome_load_tagged(g->ctx[i], path, expect);
+        const int rc = pssgpu_genome_load_tagged(g->ctx[i].get(), path, expect);
         if (rc != PSSGPU_OK) return member_fail(g, (int)i, rc);
     }
     return PSSGPU_OK;
@@ -295,7 +284,7 @@ int pssgpu_group_genome_load_tagged(pssgpu_group *g, const char *path, const pss
     do {                                                                            \
         if (!g) return PSSGPU_EINVAL;                                               \
         for (size_t i_ = 0; i_ < g->ctx.size(); i_++) {                             \
-            pssgpu_ctx *c = g->ctx[i_];                                             \
+            pssgpu_ctx *c = g->ctx[i_].get();                                       \
             const int rc_ = (call);                                                 \
             if (rc_ != PSSGPU_OK) return member_fail(g, (int)i_, rc_);              \
         }                                                                           \
@@ -319,7 +308,7 @@ int pssgpu_group_feed(pssgpu_group *g, const char *sam, size_t len, int last)
     if (!g || (!sam && len)) return PSSGPU_EINVAL;
     if (len && !last && sam[len - 1] != '\n') return gfail(g, PSSGPU_EINVAL, "group_feed: a piece must end with a newline (lines are dealt whole)");
     const size_t i = g->next++ % g->ctx.size();
-    int rc = pssgpu_feed(g->ctx[i], sam, len, 1);          // every piece is a complete text for its member
+    int rc = pssgpu_feed(g->ctx[i].get(), sam, len, 1);          // every piece is a complete text for its member
     if (rc != PSSGPU_OK) return member_fail(g, (int)i, rc);
     return PSSGPU_OK;
 }
@@ -333,15 +322,17 @@ int pssgpu_group_feed(pssgpu_group *g, const char *sam, size_t len, int last)
 int pssgpu_group_feed_bam(pssgpu_group *g, const void *bgzf_bytes, size_t len, int last)
 {
     if (!g || (!bgzf_bytes && len)) return PSSGPU_EINVAL;
-    pssgpu_ctx *own = g->ctx[0];
+    pssgpu_ctx *own = g->ctx[0].get();
     std::vector<pssgpu_ctx *> helpers;
     if (g->ctx.size() > 1) {
-        if (!g->bam_self && pssgpu_init(g->dev[0], &g->bam_self) != PSSGPU_OK) {
-            g->bam_self = nullptr;
-            return gfail(g, PSSGPU_ECUDA, "group_feed_bam: second context on GPU %d: %s", g->dev[0], pssgpu_last_error(nullptr));
+        if (!g->bam_self) {
+            pssgpu_ctx *c = nullptr;
+            if (pssgpu_init(g->dev[0], &c) != PSSGPU_OK)
+                return gfail(g, PSSGPU_ECUDA, "group_feed_bam: second context on GPU %d: %s", g->dev[0], pssgpu_last_error(nullptr));
+            g->bam_self.reset(c);
         }
-        helpers.assign(g->ctx.begin() + 1, g->ctx.end());
-        helpers.push_back(g->bam_self);
+        for (size_t i = 1; i < g->ctx.size(); i++) helpers.push_back(g->ctx[i].get());
+        helpers.push_back(g->bam_self.get());
     }
     int rc = bam_set_helpers(own, helpers);
     if (rc == PSSGPU_OK) rc = pssgpu_feed_bam(own, bgzf_bytes, len, last);
@@ -352,7 +343,7 @@ int pssgpu_group_feed_bam(pssgpu_group *g, const void *bgzf_bytes, size_t len, i
 int pssgpu_group_bam_read_group(pssgpu_group *g, const char *read_group)
 {
     if (!g) return PSSGPU_EINVAL;
-    const int rc = pssgpu_bam_read_group(g->ctx[0], read_group);
+    const int rc = pssgpu_bam_read_group(g->ctx[0].get(), read_group);
     return rc == PSSGPU_OK ? rc : member_fail(g, 0, rc);
 }
 
@@ -361,12 +352,12 @@ int pssgpu_group_bam_read_group(pssgpu_group *g, const char *read_group)
 int pssgpu_group_bam_info(pssgpu_group *g, pssgpu_bam_stats *out, uint64_t *batches_per_member)
 {
     if (!g || !out) return PSSGPU_EINVAL;
-    const int rc = pssgpu_bam_info(g->ctx[0], out);
+    const int rc = pssgpu_bam_info(g->ctx[0].get(), out);
     if (rc != PSSGPU_OK) return member_fail(g, 0, rc);
     if (batches_per_member) {
         uint64_t own = 0;
         std::vector<uint64_t> per;
-        bam_dealing(g->ctx[0], &own, &per);
+        bam_dealing(g->ctx[0].get(), &own, &per);
         // helpers = members 1 .. n-1, then the second context on the first GPU
         const size_t n = g->ctx.size();
         for (size_t i = 0; i < n; i++) batches_per_member[i] = i == 0 ? own + (per.size() == n ? per[n - 1] : 0) : (i - 1 < per.size() ? per[i - 1] : 0);
@@ -405,7 +396,7 @@ int pssgpu_group_get_stats(pssgpu_group *g, pssgpu_stats *out, int fragkon)
     memset(out, 0, sizeof *out);
     for (size_t i = 0; i < g->ctx.size(); i++) {
         pssgpu_stats s;
-        const int rc = fragkon ? pssgpu_get_fragkon_stats(g->ctx[i], &s) : pssgpu_get_stats(g->ctx[i], &s);
+        const int rc = fragkon ? pssgpu_get_fragkon_stats(g->ctx[i].get(), &s) : pssgpu_get_stats(g->ctx[i].get(), &s);
         if (rc != PSSGPU_OK) return member_fail(g, (int)i, rc);
         out->lines += s.lines; out->counted += s.counted; out->no_contig += s.no_contig; out->filtered += s.filtered;
         out->parse_fail += s.parse_fail; out->undefined += s.undefined;
@@ -426,14 +417,14 @@ int pssgpu_group_kmer_spectrum(pssgpu_group *g, int k, uint64_t *counts)
     std::vector<int> rcs(n, PSSGPU_OK);
     std::vector<std::thread> th;
     for (int i = 0; i < n; i++)                         // the shard call is synchronous: one host thread per GPU
-        th.emplace_back([&, i]() { rcs[i] = pssgpu_kmer_spectrum_shard_device(g->ctx[i], k, i, n, g->d_red[i]); });
+        th.emplace_back([&, i]() { rcs[i] = pssgpu_kmer_spectrum_shard_device(g->ctx[i].get(), k, i, n, g->d_red[i].get()); });
     for (auto &t : th) t.join();
     for (int i = 0; i < n; i++)
         if (rcs[i] != PSSGPU_OK) return member_fail(g, i, rcs[i]);
     rc = reduce_sum(g, elems);
     if (rc != PSSGPU_OK) return rc;
-    Bind bind(g->ctx[0]);
-    if (cudaMemcpy(counts, g->d_red[0], elems * sizeof(uint64_t), cudaMemcpyDeviceToHost) != cudaSuccess)
+    Bind bind(g->ctx[0].get());
+    if (cudaMemcpy(counts, g->d_red[0].get(), elems * sizeof(uint64_t), cudaMemcpyDeviceToHost) != cudaSuccess)
         return gfail(g, PSSGPU_ECUDA, "group: D2H of the spectrum: %s", cudaGetErrorString(cudaGetLastError()));
     return PSSGPU_OK;
 }
