@@ -244,6 +244,37 @@ def _host_view(buf):
     return a.ctypes.data, a.size, a
 
 
+def _contig_array(contigs, device=False):
+    """(id, seq) pairs with seq in host memory, or with device=True (id, device_ptr, len) triples ->
+    (_Contig array, count, keepalive)."""
+    contigs = list(contigs)
+    arr = (_Contig * max(1, len(contigs)))()
+    keep = []
+    for i, c in enumerate(contigs):
+        if device:
+            (cid, addr, n), ka = c, None
+        else:
+            cid, seq = c
+            addr, n, ka = _host_view(seq)
+        cid = cid.encode("latin1") if isinstance(cid, str) else bytes(cid)
+        keep.append((cid, ka))
+        arr[i] = _Contig(cid, addr, n)
+    return arr, len(contigs), keep
+
+
+def _pss_params(o: PssOptions):
+    return _PssParams(o.region_len, o.min_len, o.max_len, o.min_mq, bytes(o.up_ctx), bytes(o.down_ctx), o.merged_only)
+
+
+def _fk_params(o: FragkonOptions):
+    return _FkParams(o.klen, o.min_len, o.max_len, o.min_mq, o.merged_only)
+
+
+def _table_pair(shape):
+    """The two tables a *_finish call fills: pss forward / reverse, or fragkon's two histograms."""
+    return np.zeros(shape, dtype=np.uint64), np.zeros(shape, dtype=np.uint64)
+
+
 class Context:
     """One GPU.  Mirrors the call order of the reference mains: load genome, tally a SAM stream, read tables."""
 
@@ -281,26 +312,13 @@ class Context:
     # ---- genome (init_genome's result, fasta-genome-io.c:221-238)
     def upload_genome(self, contigs):
         """contigs: iterable of (id, seq) with seq bytes / np.uint8 (host) -- any order."""
-        contigs = list(contigs)
-        arr = (_Contig * max(1, len(contigs)))()
-        keep = []
-        for i, (cid, seq) in enumerate(contigs):
-            cid = cid.encode("latin1") if isinstance(cid, str) else bytes(cid)
-            addr, n, ka = _host_view(seq)
-            keep.append((cid, ka))
-            arr[i] = _Contig(cid, addr, n)
-        self._ck(self.lib.pssgpu_genome_upload(self.h, arr, len(contigs)))
+        arr, n, keep = _contig_array(contigs)
+        self._ck(self.lib.pssgpu_genome_upload(self.h, arr, n))
 
     def upload_genome_device(self, contigs):
         """contigs: iterable of (id, device_ptr, len)."""
-        contigs = list(contigs)
-        arr = (_Contig * max(1, len(contigs)))()
-        keep = []
-        for i, (cid, ptr, n) in enumerate(contigs):
-            cid = cid.encode("latin1") if isinstance(cid, str) else bytes(cid)
-            keep.append(cid)
-            arr[i] = _Contig(cid, ptr, n)
-        self._ck(self.lib.pssgpu_genome_upload_device(self.h, arr, len(contigs)))
+        arr, n, keep = _contig_array(contigs, device=True)
+        self._ck(self.lib.pssgpu_genome_upload_device(self.h, arr, n))
 
     def save_genome(self, path, tag=None):
         """Write the resident packed genome to `path` (pssgpu_genome_save[_tagged]); tag = (size, mtime_ns, path_hash, user)."""
@@ -325,22 +343,16 @@ class Context:
 
     # ---- tallies
     def pss_begin(self, o: PssOptions = PssOptions()):
-        self._up, self._down = bytes(o.up_ctx), bytes(o.down_ctx)
-        p = _PssParams(o.region_len, o.min_len, o.max_len, o.min_mq, self._up, self._down, o.merged_only)
-        self._ck(self.lib.pssgpu_pss_begin(self.h, C.byref(p)))
+        self._ck(self.lib.pssgpu_pss_begin(self.h, C.byref(_pss_params(o))))
         self._mode, self._R = "pss", o.region_len
 
     def fragkon_begin(self, o: FragkonOptions = FragkonOptions()):
-        p = _FkParams(o.klen, o.min_len, o.max_len, o.min_mq, o.merged_only)
-        self._ck(self.lib.pssgpu_fragkon_begin(self.h, C.byref(p)))
+        self._ck(self.lib.pssgpu_fragkon_begin(self.h, C.byref(_fk_params(o))))
         self._mode, self._K = "fragkon", o.klen
 
     def both_begin(self, o: PssOptions = PssOptions(), f: FragkonOptions = FragkonOptions()):
         """pss-bam and fragkon tallies from one scan of the text."""
-        self._up, self._down = bytes(o.up_ctx), bytes(o.down_ctx)
-        p = _PssParams(o.region_len, o.min_len, o.max_len, o.min_mq, self._up, self._down, o.merged_only)
-        q = _FkParams(f.klen, f.min_len, f.max_len, f.min_mq, f.merged_only)
-        self._ck(self.lib.pssgpu_both_begin(self.h, C.byref(p), C.byref(q)))
+        self._ck(self.lib.pssgpu_both_begin(self.h, C.byref(_pss_params(o)), C.byref(_fk_params(f))))
         self._mode, self._R, self._K = "both", o.region_len, f.klen
 
     def fragkon_stats(self):
@@ -381,9 +393,7 @@ class Context:
         self._ck(self.lib.pssgpu_sync(self.h))
 
     def pss_finish(self):
-        R = self._R
-        fwd = np.zeros((R + 2, 16), dtype=np.uint64)
-        rev = np.zeros((R + 2, 16), dtype=np.uint64)
+        fwd, rev = _table_pair((self._R + 2, 16))
         self._ck(self.lib.pssgpu_pss_finish(self.h, fwd.ctypes.data, rev.ctypes.data))
         return fwd, rev
 
@@ -391,9 +401,7 @@ class Context:
         self._ck(self.lib.pssgpu_pss_finish_device(self.h, dev_ptr))
 
     def fragkon_finish(self):
-        nb = 1 << (2 * self._K)
-        fp = np.zeros(nb, dtype=np.uint64)
-        tp = np.zeros(nb, dtype=np.uint64)
+        fp, tp = _table_pair(1 << (2 * self._K))
         self._ck(self.lib.pssgpu_fragkon_finish(self.h, fp.ctypes.data, tp.ctypes.data))
         return fp, tp
 
@@ -491,25 +499,15 @@ class Group:
         return float(self.lib.pssgpu_group_last_reduce_ms(self.h))
 
     def upload_genome(self, contigs):
-        contigs = list(contigs)
-        arr = (_Contig * max(1, len(contigs)))()
-        keep = []
-        for i, (cid, seq) in enumerate(contigs):
-            cid = cid.encode("latin1") if isinstance(cid, str) else bytes(cid)
-            addr, n, ka = _host_view(seq)
-            keep.append((cid, ka))
-            arr[i] = _Contig(cid, addr, n)
-        self._ck(self.lib.pssgpu_group_genome_upload(self.h, arr, len(contigs)))
+        arr, n, keep = _contig_array(contigs)
+        self._ck(self.lib.pssgpu_group_genome_upload(self.h, arr, n))
 
     def pss_begin(self, o: PssOptions = PssOptions()):
-        self._up, self._down = bytes(o.up_ctx), bytes(o.down_ctx)
-        p = _PssParams(o.region_len, o.min_len, o.max_len, o.min_mq, self._up, self._down, o.merged_only)
-        self._ck(self.lib.pssgpu_group_pss_begin(self.h, C.byref(p)))
+        self._ck(self.lib.pssgpu_group_pss_begin(self.h, C.byref(_pss_params(o))))
         self._R = o.region_len
 
     def fragkon_begin(self, o: FragkonOptions = FragkonOptions()):
-        p = _FkParams(o.klen, o.min_len, o.max_len, o.min_mq, o.merged_only)
-        self._ck(self.lib.pssgpu_group_fragkon_begin(self.h, C.byref(p)))
+        self._ck(self.lib.pssgpu_group_fragkon_begin(self.h, C.byref(_fk_params(o))))
         self._K = o.klen
 
     def feed(self, sam, last=False):
@@ -541,16 +539,12 @@ class Group:
         self._ck(self.lib.pssgpu_group_sync(self.h))
 
     def pss_finish(self):
-        R = self._R
-        fwd = np.zeros((R + 2, 16), dtype=np.uint64)
-        rev = np.zeros((R + 2, 16), dtype=np.uint64)
+        fwd, rev = _table_pair((self._R + 2, 16))
         self._ck(self.lib.pssgpu_group_pss_finish(self.h, fwd.ctypes.data, rev.ctypes.data))
         return fwd, rev
 
     def fragkon_finish(self):
-        nb = 1 << (2 * self._K)
-        fp = np.zeros(nb, dtype=np.uint64)
-        tp = np.zeros(nb, dtype=np.uint64)
+        fp, tp = _table_pair(1 << (2 * self._K))
         self._ck(self.lib.pssgpu_group_fragkon_finish(self.h, fp.ctypes.data, tp.ctypes.data))
         return fp, tp
 

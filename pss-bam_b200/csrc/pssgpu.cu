@@ -267,8 +267,27 @@ int ctx_string(pssgpu_ctx *ctx, const char *s, uint32_t *mask, uint32_t *other, 
     return PSSGPU_OK;
 }
 
+// The one rule that picks the tally_kernel instantiation for a mode and -r (R is not read in fragkon mode).
+// pssgpu_init prepares what it returns for every mode and R; launch_tally_mode launches it.
+using TallyKernel = void (*)(TallyArgs);
 template <int MODE>
-int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t stream_off, const unsigned long long *len_dev)
+TallyKernel tally_kernel_for_r(int R)
+{
+    if (R == 15) return tally_kernel<MODE, 9, 17>;              // the default -r
+    if (R <= 16) return tally_kernel<MODE, 9, 0>;
+    if (R <= kMaxRegion) return tally_kernel<MODE, 16, 0>;
+    return tally_kernel<MODE, 0, 0>;                            // any -r: exact, not tuned
+}
+TallyKernel tally_kernel_for(int mode, int R)
+{
+    return mode == kModeFragkon ? tally_kernel<kModeFragkon, 9, 0>
+         : mode == kModeBoth    ? tally_kernel_for_r<kModeBoth>(R)
+                                : tally_kernel_for_r<kModePss>(R);
+}
+
+}  // namespace
+
+int pssgpu::launch_tally_mode(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t stream_off, const unsigned long long *len_dev)
 {
     if (len == 0) return PSSGPU_OK;
     TallyArgs a;
@@ -288,7 +307,7 @@ int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t str
     a.dbg_code = ctx->dbg ? ctx->d_dbg_code.get() : nullptr;
     a.dbg_n = ctx->dbg ? ctx->d_dbg_n.get() : nullptr;
     a.dbg_cap = ctx->dbg_cap;
-    const int      max_grid = MODE == kModeFragkon ? ctx->tally_grid_fk : ctx->tally_grid_pss;
+    const int      max_grid = ctx->mode == kModeFragkon ? ctx->tally_grid_fk : ctx->tally_grid_pss;
     // ranges handed out by an atomic counter: about eight per CTA on large inputs, never below 128 KiB
     uint64_t rb = len / ((uint64_t)max_grid * 8u);
     if (const char *e = getenv("PSSGPU_RANGE_KB")) rb = std::max<uint64_t>(1, strtoull(e, nullptr, 10)) << 10;   // developer / test switch
@@ -301,47 +320,11 @@ int launch_tally(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t str
     CU(cudaMemsetAsync(ctx->d_range_ctr.get(), 0, sizeof(unsigned int), ctx->stream.get()));
     time_begin(ctx, len);
     const unsigned grid = (unsigned)std::min<uint64_t>(n_ranges, (uint64_t)max_grid);
-    constexpr int PM = MODE == kModeFragkon ? kModePss : MODE;          // (never launched with MODE == kModeFragkon)
-    constexpr size_t smem = sizeof(TallySmem);
-    if (MODE == kModeFragkon) tally_kernel<kModeFragkon, 9, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);
-    else if (ctx->cfg.R == 15) tally_kernel<PM, 9, 17><<<grid, kThreads, smem, ctx->stream.get()>>>(a);         // the default -r
-    else if (ctx->cfg.R + 2 <= 18) tally_kernel<PM, 9, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);
-    else if (ctx->cfg.R <= kMaxRegion) tally_kernel<PM, 16, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);
-    else tally_kernel<PM, 0, 0><<<grid, kThreads, smem, ctx->stream.get()>>>(a);                                // any -r: exact, not tuned
+    tally_kernel_for(ctx->mode, ctx->cfg.R)<<<grid, kThreads, sizeof(TallySmem), ctx->stream.get()>>>(a);
     time_end(ctx);
     CU(cudaGetLastError());
     return PSSGPU_OK;
 }
-
-}  // namespace
-
-int pssgpu::launch_tally_mode(pssgpu_ctx *ctx, const uint8_t *d_sam, size_t len, uint64_t stream_off, const unsigned long long *len_dev)
-{
-    return ctx->mode == kModePss  ? launch_tally<kModePss>(ctx, d_sam, len, stream_off, len_dev)
-         : ctx->mode == kModeBoth ? launch_tally<kModeBoth>(ctx, d_sam, len, stream_off, len_dev)
-                                  : launch_tally<kModeFragkon>(ctx, d_sam, len, stream_off, len_dev);
-}
-
-namespace {
-
-// after the parameters of a *_begin were accepted: no tally is open until the begin completes (a table it failed to
-// allocate must never be fed)
-int begin_common(pssgpu_ctx *ctx)
-{
-    ctx->mode = -1;
-    CU(cudaStreamSynchronize(ctx->stream.get()));
-    if (!ctx->d_stats) CU(alloc(ctx->d_stats, 2 * kStN * sizeof(unsigned long long)));
-    if (!ctx->d_range_ctr) CU(alloc(ctx->d_range_ctr, sizeof(unsigned int)));
-    CU(cudaMemsetAsync(ctx->d_stats.get(), 0, 2 * kStN * sizeof(unsigned long long), ctx->stream.get()));
-    if (ctx->dbg_cap) CU(cudaMemsetAsync(ctx->d_dbg_n.get(), 0, sizeof(unsigned long long), ctx->stream.get()));
-    ctx->carry_len = 0;
-    ctx->cur = 0;
-    ctx->fed_bytes = 0;
-    bam_reset(ctx);
-    return PSSGPU_OK;
-}
-
-}  // namespace
 
 // ===========================================================================
 extern "C" {
@@ -378,17 +361,19 @@ int pssgpu_init(int device, pssgpu_ctx **out)
         if (e == cudaSuccess) e = create(c->ev_copied[i]);
         if (e == cudaSuccess) e = create(c->ev_tallied[i]);
     }
-    {   // every instantiation needs its dynamic shared memory raised above the 48 KB default
-        const void *kernels[] = {
-            (const void *)tally_kernel<kModePss, 9, 17>, (const void *)tally_kernel<kModePss, 9, 0>, (const void *)tally_kernel<kModePss, 16, 0>,
-            (const void *)tally_kernel<kModePss, 0, 0>, (const void *)tally_kernel<kModeFragkon, 9, 0>, (const void *)tally_kernel<kModeBoth, 9, 17>,
-            (const void *)tally_kernel<kModeBoth, 9, 0>, (const void *)tally_kernel<kModeBoth, 16, 0>, (const void *)tally_kernel<kModeBoth, 0, 0> };
-        for (const void *k : kernels)
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TallySmem));
+    // every instantiation tally_kernel_for() returns for an accepted -r needs its dynamic shared memory raised above
+    // the 48 KB default
+    for (int mode : { kModePss, kModeFragkon, kModeBoth }) {
+        TallyKernel prev = nullptr;
+        for (int R = 0; R <= kMaxRegionWide && e == cudaSuccess; R++) {
+            const TallyKernel k = tally_kernel_for(mode, R);
+            if (k != prev) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TallySmem));
+            prev = k;
+        }
     }
     int occ_p = 0, occ_f = 0;
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, tally_kernel<kModePss, 16, 0>, kThreads, sizeof(TallySmem));
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_f, tally_kernel<kModeFragkon, 9, 0>, kThreads, sizeof(TallySmem));
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, tally_kernel_for(kModePss, kMaxRegion), kThreads, sizeof(TallySmem));
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_f, tally_kernel_for(kModeFragkon, 0), kThreads, sizeof(TallySmem));
     if (e != cudaSuccess || occ_p < 1 || occ_f < 1)
         return fail(nullptr, PSSGPU_ECUDA, "pssgpu_init: %s (occupancy %d/%d)", cudaGetErrorString(e), occ_p, occ_f);
     c->tally_grid_pss = c->sm_count * occ_p;
@@ -654,40 +639,49 @@ int alloc_fk_tables(pssgpu_ctx *ctx, int K)
     return PSSGPU_OK;
 }
 
-}  // namespace
-
-int pssgpu_pss_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p)
+// A new tally: pss (p), fragkon (f) or both from one scan (mode); `fn` names the entry point in messages.  The fused
+// mode keeps the pss options in cfg (with cfg.mode == kModeBoth) and the fragkon ones in cfg_fk; fragkon alone keeps
+// its options in cfg.
+int begin_tally(pssgpu_ctx *ctx, const char *fn, int mode, const pssgpu_pss_params *p, const pssgpu_fragkon_params *f)
 {
-    if (!ctx || !p) return fail(ctx, PSSGPU_EINVAL, "pss_begin: null argument");
-    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "pss_begin: no genome resident");
-    Bind bind(ctx);
-    TallyCfg c;
-    int rc;
-    if ((rc = pss_cfg(ctx, p, c)) != PSSGPU_OK) return rc;
-    if ((rc = begin_common(ctx)) != PSSGPU_OK) return rc;
-    if ((rc = alloc_pss_tables(ctx, c.R)) != PSSGPU_OK) return rc;
-    ctx->cfg = c;
-    ctx->mode = kModePss;
-    return PSSGPU_OK;
-}
-
-int pssgpu_both_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p, const pssgpu_fragkon_params *f)
-{
-    if (!ctx || !p || !f) return fail(ctx, PSSGPU_EINVAL, "both_begin: null argument");
-    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "both_begin: no genome resident");
+    const bool pss = mode != kModeFragkon, fk = mode != kModePss;
+    if (!ctx || (pss && !p) || (fk && !f)) return fail(ctx, PSSGPU_EINVAL, "%s: null argument", fn);
+    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "%s: no genome resident", fn);
     Bind bind(ctx);
     TallyCfg c, cf;
     int rc;
-    if ((rc = pss_cfg(ctx, p, c)) != PSSGPU_OK) return rc;
-    if ((rc = fk_cfg(ctx, f, cf)) != PSSGPU_OK) return rc;
-    if ((rc = begin_common(ctx)) != PSSGPU_OK) return rc;
-    if ((rc = alloc_pss_tables(ctx, c.R)) != PSSGPU_OK) return rc;
-    if ((rc = alloc_fk_tables(ctx, cf.K)) != PSSGPU_OK) return rc;
-    c.mode = kModeBoth;
-    ctx->cfg = c;
-    ctx->cfg_fk = cf;
-    ctx->mode = kModeBoth;
+    if (pss && (rc = pss_cfg(ctx, p, c)) != PSSGPU_OK) return rc;
+    if (fk && (rc = fk_cfg(ctx, f, cf)) != PSSGPU_OK) return rc;
+    // the parameters were accepted: no tally is open until the begin completes (a table it failed to allocate must
+    // never be fed)
+    ctx->mode = -1;
+    CU(cudaStreamSynchronize(ctx->stream.get()));
+    if (!ctx->d_stats) CU(alloc(ctx->d_stats, 2 * kStN * sizeof(unsigned long long)));
+    if (!ctx->d_range_ctr) CU(alloc(ctx->d_range_ctr, sizeof(unsigned int)));
+    CU(cudaMemsetAsync(ctx->d_stats.get(), 0, 2 * kStN * sizeof(unsigned long long), ctx->stream.get()));
+    if (ctx->dbg_cap) CU(cudaMemsetAsync(ctx->d_dbg_n.get(), 0, sizeof(unsigned long long), ctx->stream.get()));
+    ctx->carry_len = 0;
+    ctx->cur = 0;
+    ctx->fed_bytes = 0;
+    bam_reset(ctx);
+    if (pss && (rc = alloc_pss_tables(ctx, c.R)) != PSSGPU_OK) return rc;
+    if (fk && (rc = alloc_fk_tables(ctx, cf.K)) != PSSGPU_OK) return rc;
+    if (mode == kModeBoth) {
+        c.mode = kModeBoth;
+        ctx->cfg_fk = cf;
+    }
+    ctx->cfg = pss ? c : cf;
+    ctx->mode = mode;
     return PSSGPU_OK;
+}
+
+}  // namespace
+
+int pssgpu_pss_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p) { return begin_tally(ctx, "pss_begin", kModePss, p, nullptr); }
+int pssgpu_fragkon_begin(pssgpu_ctx *ctx, const pssgpu_fragkon_params *p) { return begin_tally(ctx, "fragkon_begin", kModeFragkon, nullptr, p); }
+int pssgpu_both_begin(pssgpu_ctx *ctx, const pssgpu_pss_params *p, const pssgpu_fragkon_params *f)
+{
+    return begin_tally(ctx, "both_begin", kModeBoth, p, f);
 }
 
 namespace {
@@ -813,34 +807,39 @@ int pssgpu_sync(pssgpu_ctx *ctx)
     return PSSGPU_OK;
 }
 
-int pssgpu_pss_finish(pssgpu_ctx *ctx, uint64_t *fwd, uint64_t *rev)
+namespace {
+// The open tally's pss (which == kModePss) or fragkon table: to the host, its halves to `lo` and `hi`, or, with
+// to_device, whole to the device buffer `lo`.
+int finish_tally(pssgpu_ctx *ctx, const char *fn, int which, bool to_device, void *lo, void *hi)
 {
-    if (!ctx || !fwd || !rev) return fail(ctx, PSSGPU_EINVAL, "pss_finish: null argument");
-    if (ctx->mode != kModePss && ctx->mode != kModeBoth) return fail(ctx, PSSGPU_EINVAL, "pss_finish: no pss tally open");
-    if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "pss_finish: %zu bytes of an unterminated line pending (feed with last=1)", ctx->carry_len);
+    if (!ctx || !lo || (!to_device && !hi)) return fail(ctx, PSSGPU_EINVAL, "%s: null argument", fn);
+    const bool fk = which == kModeFragkon;
+    if (ctx->mode != which && ctx->mode != kModeBoth) return fail(ctx, PSSGPU_EINVAL, "%s: no %s tally open", fn, fk ? "fragkon" : "pss");
+    if (ctx->carry_len)
+        return fail(ctx, PSSGPU_EINVAL, "%s: %zu bytes of an unterminated line pending (feed with last=1)", fn, ctx->carry_len);
     Bind bind(ctx);
-    const size_t half = (size_t)(ctx->cfg.R + 2) * 16 * sizeof(uint64_t);
-    CU(cudaMemcpyAsync(fwd, ctx->d_tables.get(), half, cudaMemcpyDeviceToHost, ctx->stream.get()));
-    CU(cudaMemcpyAsync(rev, (const char *)ctx->d_tables.get() + half, half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    const size_t half = (fk ? ctx->fk_elems / 2 : (size_t)(ctx->cfg.R + 2) * 16) * sizeof(uint64_t);
+    const char  *table = fk ? (const char *)ctx->d_fk.get() : (const char *)ctx->d_tables.get();
+    if (to_device) {
+        CU(cudaMemcpyAsync(lo, table, 2 * half, cudaMemcpyDeviceToDevice, ctx->stream.get()));
+    } else {
+        CU(cudaMemcpyAsync(lo, table, half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+        CU(cudaMemcpyAsync(hi, table + half, half, cudaMemcpyDeviceToHost, ctx->stream.get()));
+    }
     CU(cudaStreamSynchronize(ctx->stream.get()));
     { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
-    ctx->d2h_bytes += 2 * half;
+    if (!to_device) ctx->d2h_bytes += 2 * half;
     time_collect(ctx);
     return PSSGPU_OK;
 }
+}  // namespace
 
-int pssgpu_pss_finish_device(pssgpu_ctx *ctx, void *d_tables)
+int pssgpu_pss_finish(pssgpu_ctx *ctx, uint64_t *fwd, uint64_t *rev) { return finish_tally(ctx, "pss_finish", kModePss, false, fwd, rev); }
+int pssgpu_pss_finish_device(pssgpu_ctx *ctx, void *d_tables) { return finish_tally(ctx, "pss_finish_device", kModePss, true, d_tables, nullptr); }
+int pssgpu_fragkon_finish(pssgpu_ctx *ctx, uint64_t *fp, uint64_t *tp) { return finish_tally(ctx, "fragkon_finish", kModeFragkon, false, fp, tp); }
+int pssgpu_fragkon_finish_device(pssgpu_ctx *ctx, void *d_out)
 {
-    if (!ctx || !d_tables) return fail(ctx, PSSGPU_EINVAL, "pss_finish_device: null argument");
-    if (ctx->mode != kModePss && ctx->mode != kModeBoth) return fail(ctx, PSSGPU_EINVAL, "pss_finish_device: no pss tally open");
-    if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "pss_finish_device: unterminated line pending");
-    Bind bind(ctx);
-    const size_t bytes = 2 * (size_t)(ctx->cfg.R + 2) * 16 * sizeof(uint64_t);
-    CU(cudaMemcpyAsync(d_tables, ctx->d_tables.get(), bytes, cudaMemcpyDeviceToDevice, ctx->stream.get()));
-    CU(cudaStreamSynchronize(ctx->stream.get()));
-    { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
-    time_collect(ctx);
-    return PSSGPU_OK;
+    return finish_tally(ctx, "fragkon_finish_device", kModeFragkon, true, d_out, nullptr);
 }
 
 namespace {
@@ -881,50 +880,6 @@ void pssgpu_fragkon_default_params(pssgpu_fragkon_params *p)
     p->min_len = 0;              // :16
     p->max_len = 250000000UL;    // :17
     p->merged_only = 0;          // :18
-}
-
-int pssgpu_fragkon_begin(pssgpu_ctx *ctx, const pssgpu_fragkon_params *p)
-{
-    if (!ctx || !p) return fail(ctx, PSSGPU_EINVAL, "fragkon_begin: null argument");
-    if (!ctx->genome.resident()) return fail(ctx, PSSGPU_ENOGENOME, "fragkon_begin: no genome resident");
-    Bind bind(ctx);
-    TallyCfg c;
-    int rc;
-    if ((rc = fk_cfg(ctx, p, c)) != PSSGPU_OK) return rc;
-    if ((rc = begin_common(ctx)) != PSSGPU_OK) return rc;
-    if ((rc = alloc_fk_tables(ctx, c.K)) != PSSGPU_OK) return rc;
-    ctx->cfg = c;
-    ctx->mode = kModeFragkon;
-    return PSSGPU_OK;
-}
-
-int pssgpu_fragkon_finish(pssgpu_ctx *ctx, uint64_t *fp, uint64_t *tp)
-{
-    if (!ctx || !fp || !tp) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish: null argument");
-    if (ctx->mode != kModeFragkon && ctx->mode != kModeBoth) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish: no fragkon tally open");
-    if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish: unterminated line pending (feed with last=1)");
-    Bind bind(ctx);
-    const size_t half = (ctx->fk_elems / 2) * sizeof(uint64_t);
-    CU(cudaMemcpyAsync(fp, ctx->d_fk.get(), half, cudaMemcpyDeviceToHost, ctx->stream.get()));
-    CU(cudaMemcpyAsync(tp, (const char *)ctx->d_fk.get() + half, half, cudaMemcpyDeviceToHost, ctx->stream.get()));
-    CU(cudaStreamSynchronize(ctx->stream.get()));
-    { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
-    ctx->d2h_bytes += 2 * half;
-    time_collect(ctx);
-    return PSSGPU_OK;
-}
-
-int pssgpu_fragkon_finish_device(pssgpu_ctx *ctx, void *d_out)
-{
-    if (!ctx || !d_out) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish_device: null argument");
-    if (ctx->mode != kModeFragkon && ctx->mode != kModeBoth) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish_device: no fragkon tally open");
-    if (ctx->carry_len) return fail(ctx, PSSGPU_EINVAL, "fragkon_finish_device: unterminated line pending");
-    Bind bind(ctx);
-    CU(cudaMemcpyAsync(d_out, ctx->d_fk.get(), ctx->fk_elems * sizeof(uint64_t), cudaMemcpyDeviceToDevice, ctx->stream.get()));
-    CU(cudaStreamSynchronize(ctx->stream.get()));
-    { const int brc = bam_check(ctx, true); if (brc != PSSGPU_OK) return brc; }
-    time_collect(ctx);
-    return PSSGPU_OK;
 }
 
 // ---- genome-kmer-count ----------------------------------------------------------
@@ -968,57 +923,51 @@ int pssgpu_kmer_spectrum_shard_device(pssgpu_ctx *ctx, int k, int shard, int n_s
         }
     }
     time_begin(ctx, (g1 - g0) * sizeof(uint64_t));
-    if (d_payload) {
-        unsigned long long *cnt = d_rad.get(), *off = cnt + rad_nb, *cur = cnt + 2 * (size_t)rad_nb + 1;
-        cudaMemsetAsync(cnt, 0, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long), ctx->stream.get());
-        const unsigned rgrid = (unsigned)std::min<uint64_t>((g1 - g0 + kRadixThreads - 1) / kRadixThreads, (uint64_t)ctx->sm_count * 4);
-        const uint32_t parts = std::max<uint32_t>(1u, (2u * (uint32_t)ctx->sm_count + rad_nb - 1) / rad_nb);
-        const size_t   hsmem = (size_t)kSpecSmemBins * sizeof(uint32_t);
-#define PSS_RADIX(K_)                                                                                                  \
-        do {                                                                                                           \
-            radix_count_kernel<K_><<<rgrid, kRadixThreads, 0, ctx->stream.get()>>>(d_groups, g0, g1, cnt);                  \
-            radix_scan_kernel<<<1, kRadixThreads, 0, ctx->stream.get()>>>(cnt, off, cur, rad_nb);                           \
-            radix_scatter_kernel<K_><<<rgrid, kRadixThreads, 0, ctx->stream.get()>>>(d_groups, g0, g1, cur, d_payload.get()); \
-        } while (0)
-        if (k == 10) PSS_RADIX(10); else if (k == 11) PSS_RADIX(11); else PSS_RADIX(12);
-#undef PSS_RADIX
-        if (narrow) {
-            cudaFuncSetAttribute(radix_hist_kernel<unsigned int>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
-            radix_hist_kernel<unsigned int><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream.get()>>>(d_payload.get(), off, parts, d_narrow.get());
-        } else {
-            cudaFuncSetAttribute(radix_hist_kernel<unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
-            radix_hist_kernel<unsigned long long><<<rad_nb * parts, kSpecSmemThreads, hsmem, ctx->stream.get()>>>(d_payload.get(), off, parts, (unsigned long long *)d_counts);
+    // the counting launches, into 32-bit scratch bins or into the caller's 64-bit counters
+    auto launch = [&](auto *counts) {
+        using CT = std::remove_pointer_t<decltype(counts)>;
+        cudaStream_t st = ctx->stream.get();
+        if (d_payload) {
+            unsigned long long *cnt = d_rad.get(), *off = cnt + rad_nb, *cur = cnt + 2 * (size_t)rad_nb + 1;
+            cudaMemsetAsync(cnt, 0, (3 * (size_t)rad_nb + 2) * sizeof(unsigned long long), st);
+            const unsigned rgrid = (unsigned)std::min<uint64_t>((g1 - g0 + kRadixThreads - 1) / kRadixThreads, (uint64_t)ctx->sm_count * 4);
+            const uint32_t parts = std::max<uint32_t>(1u, (2u * (uint32_t)ctx->sm_count + rad_nb - 1) / rad_nb);
+            const size_t   hsmem = (size_t)kSpecSmemBins * sizeof(uint32_t);
+            decltype(&radix_count_kernel<10>)   count;
+            decltype(&radix_scatter_kernel<10>) scatter;
+            switch (k) {
+            case 10: count = radix_count_kernel<10>; scatter = radix_scatter_kernel<10>; break;
+            case 11: count = radix_count_kernel<11>; scatter = radix_scatter_kernel<11>; break;
+            default: count = radix_count_kernel<12>; scatter = radix_scatter_kernel<12>; break;
+            }
+            count<<<rgrid, kRadixThreads, 0, st>>>(d_groups, g0, g1, cnt);
+            radix_scan_kernel<<<1, kRadixThreads, 0, st>>>(cnt, off, cur, rad_nb);
+            scatter<<<rgrid, kRadixThreads, 0, st>>>(d_groups, g0, g1, cur, d_payload.get());
+            cudaFuncSetAttribute(radix_hist_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
+            radix_hist_kernel<CT><<<rad_nb * parts, kSpecSmemThreads, hsmem, st>>>(d_payload.get(), off, parts, counts);
+        } else if (g1 > g0 && k >= 7 && k <= 9) {
+            // shared-memory bins, 16-bit counters packed two to a word: 65 536 bins per CTA -- one pass for 4^8 bins, four for 4^9
+            const uint32_t n_slices = (uint32_t)std::min<uint64_t>((uint64_t)ctx->sm_count, (g1 - g0 + kSpecSmemThreads - 1) / kSpecSmemThreads);
+            const uint32_t passes = (uint32_t)std::max<size_t>(1, bins >> kSpec16Log);
+            const size_t   smem = std::min<size_t>(std::max<size_t>(bins / 2, std::min<size_t>(bins, 32768)), kSpec16Words) * sizeof(uint32_t);
+            decltype(&spectrum_smem16_kernel<7, CT>) spec16;
+            switch (k) {
+            case 7:  spec16 = spectrum_smem16_kernel<7, CT>; break;
+            case 8:  spec16 = spectrum_smem16_kernel<8, CT>; break;
+            default: spec16 = spectrum_smem16_kernel<9, CT>; break;
+            }
+            cudaFuncSetAttribute(spec16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            spec16<<<n_slices * passes, kSpecSmemThreads, smem, st>>>(d_groups, g0, g1, n_slices, counts);
+        } else if (g1 > g0) {
+            (k <= kSpectrumSmemK ? spectrum_kernel<true, CT> : spectrum_kernel<false, CT>)<<<grid, 256, 0, st>>>(d_groups, g0, g1, k, counts);
         }
-    } else if (g1 > g0 && k >= 7 && k <= 9) {
-        // shared-memory bins, 16-bit counters packed two to a word: 65 536 bins per CTA -- one pass for 4^8 bins, four for 4^9
-        const uint32_t n_slices = (uint32_t)std::min<uint64_t>((uint64_t)ctx->sm_count, (g1 - g0 + kSpecSmemThreads - 1) / kSpecSmemThreads);
-        const uint32_t passes = (uint32_t)std::max<size_t>(1, bins >> kSpec16Log);
-        const size_t   smem = std::min<size_t>(std::max<size_t>(bins / 2, std::min<size_t>(bins, 32768)), kSpec16Words) * sizeof(uint32_t);
-        const dim3     sg(n_slices * passes);
-#define PSS_SPEC16(K_, CT_, PTR_)                                                                                      \
-        do {                                                                                                           \
-            cudaFuncSetAttribute(spectrum_smem16_kernel<K_, CT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-            spectrum_smem16_kernel<K_, CT_><<<sg, kSpecSmemThreads, smem, ctx->stream.get()>>>(d_groups, g0, g1, n_slices, PTR_); \
-        } while (0)
-        if (narrow) {
-            if (k == 7) PSS_SPEC16(7, unsigned int, d_narrow.get()); else if (k == 8) PSS_SPEC16(8, unsigned int, d_narrow.get()); else PSS_SPEC16(9, unsigned int, d_narrow.get());
-        } else {
-            unsigned long long *w = (unsigned long long *)d_counts;
-            if (k == 7) PSS_SPEC16(7, unsigned long long, w); else if (k == 8) PSS_SPEC16(8, unsigned long long, w); else PSS_SPEC16(9, unsigned long long, w);
-        }
-#undef PSS_SPEC16
-    } else if (g1 > g0) {
-        if (narrow) {
-            if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned int><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, d_narrow.get());
-            else spectrum_kernel<false, unsigned int><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, d_narrow.get());
-        } else {
-            if (k <= kSpectrumSmemK) spectrum_kernel<true, unsigned long long><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, (unsigned long long *)d_counts);
-            else spectrum_kernel<false, unsigned long long><<<grid, 256, 0, ctx->stream.get()>>>(d_groups, g0, g1, k, (unsigned long long *)d_counts);
-        }
-    }
+    };
     if (narrow) {
+        launch(d_narrow.get());
         const unsigned wgrid = (unsigned)std::min<uint64_t>((bins + 255) / 256, (uint64_t)ctx->sm_count * 8);
         widen_kernel<<<wgrid, 256, 0, ctx->stream.get()>>>(d_narrow.get(), (unsigned long long *)d_counts, bins);
+    } else {
+        launch((unsigned long long *)d_counts);
     }
     time_end(ctx);
     cudaError_t le = cudaGetLastError();

@@ -156,21 +156,33 @@ int reduce_sum(pssgpu_group *g, size_t elems)
 }  // namespace
 
 namespace {
-// tables of every member -> d_red, summed, to the host
+// fill(member context, its reduction buffer, its index) of every member -> d_red, summed; the sum to the host: whole
+// to `lo`, or with `hi`, its halves to `lo` and `hi`.  threaded: the fills are synchronous calls that each keep their
+// GPU busy, so they run on one host thread per member.
 template <class Fill>
-int gather_sum(pssgpu_group *g, size_t elems, Fill fill, uint64_t *host_out)
+int gather_sum(pssgpu_group *g, size_t elems, bool threaded, Fill fill, uint64_t *lo, uint64_t *hi = nullptr)
 {
     int rc = ensure_red(g, elems);
     if (rc != PSSGPU_OK) return rc;
-    for (size_t i = 0; i < g->ctx.size(); i++) {
-        rc = fill(g->ctx[i].get(), g->d_red[i].get());
-        if (rc != PSSGPU_OK) return member_fail(g, (int)i, rc);
+    const int n = (int)g->ctx.size();
+    std::vector<int> rcs(n, PSSGPU_OK);
+    if (threaded) {
+        std::vector<std::thread> th;
+        for (int i = 0; i < n; i++) th.emplace_back([&, i]() { rcs[i] = fill(g->ctx[i].get(), g->d_red[i].get(), i); });
+        for (auto &t : th) t.join();
+    } else {
+        for (int i = 0; i < n; i++)
+            if ((rcs[i] = fill(g->ctx[i].get(), g->d_red[i].get(), i)) != PSSGPU_OK) break;
     }
+    for (int i = 0; i < n; i++)
+        if (rcs[i] != PSSGPU_OK) return member_fail(g, i, rcs[i]);
     rc = reduce_sum(g, elems);
     if (rc != PSSGPU_OK) return rc;
     Bind bind(g->ctx[0].get());
-    if (cudaMemcpy(host_out, g->d_red[0].get(), elems * sizeof(uint64_t), cudaMemcpyDeviceToHost) != cudaSuccess)
-        return gfail(g, PSSGPU_ECUDA, "group: D2H of the summed tables: %s", cudaGetErrorString(cudaGetLastError()));
+    const size_t part = (hi ? elems / 2 : elems) * sizeof(uint64_t);
+    cudaError_t e = cudaMemcpy(lo, g->d_red[0].get(), part, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && hi) e = cudaMemcpy(hi, g->d_red[0].get() + elems / 2, part, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return gfail(g, PSSGPU_ECUDA, "group: D2H of the summed tables: %s", cudaGetErrorString(cudaGetLastError()));
     return PSSGPU_OK;
 }
 }  // namespace
@@ -368,26 +380,16 @@ int pssgpu_group_bam_info(pssgpu_group *g, pssgpu_bam_stats *out, uint64_t *batc
 int pssgpu_group_pss_finish(pssgpu_group *g, uint64_t *fwd, uint64_t *rev)
 {
     if (!g || !fwd || !rev) return PSSGPU_EINVAL;
-    const size_t half = (size_t)(g->ctx[0]->cfg.R + 2) * 16;
-    std::vector<uint64_t> both(2 * half);
-    const int rc = gather_sum(g, 2 * half, [](pssgpu_ctx *c, unsigned long long *d) { return pssgpu_pss_finish_device(c, d); }, both.data());
-    if (rc != PSSGPU_OK) return rc;
-    memcpy(fwd, both.data(), half * sizeof(uint64_t));
-    memcpy(rev, both.data() + half, half * sizeof(uint64_t));
-    return PSSGPU_OK;
+    const size_t elems = 2 * (size_t)(g->ctx[0]->cfg.R + 2) * 16;
+    return gather_sum(g, elems, false, [](pssgpu_ctx *c, unsigned long long *d, int) { return pssgpu_pss_finish_device(c, d); }, fwd, rev);
 }
 
 int pssgpu_group_fragkon_finish(pssgpu_group *g, uint64_t *fp, uint64_t *tp)
 {
     if (!g || !fp || !tp) return PSSGPU_EINVAL;
-    const size_t elems = g->ctx[0]->fk_elems, half = elems / 2;
+    const size_t elems = g->ctx[0]->fk_elems;
     if (!elems) return gfail(g, PSSGPU_EINVAL, "group_fragkon_finish: no fragkon tally open");
-    std::vector<uint64_t> both(elems);
-    const int rc = gather_sum(g, elems, [](pssgpu_ctx *c, unsigned long long *d) { return pssgpu_fragkon_finish_device(c, d); }, both.data());
-    if (rc != PSSGPU_OK) return rc;
-    memcpy(fp, both.data(), half * sizeof(uint64_t));
-    memcpy(tp, both.data() + half, half * sizeof(uint64_t));
-    return PSSGPU_OK;
+    return gather_sum(g, elems, false, [](pssgpu_ctx *c, unsigned long long *d, int) { return pssgpu_fragkon_finish_device(c, d); }, fp, tp);
 }
 
 int pssgpu_group_get_stats(pssgpu_group *g, pssgpu_stats *out, int fragkon)
@@ -410,23 +412,9 @@ int pssgpu_group_kmer_spectrum(pssgpu_group *g, int k, uint64_t *counts)
 {
     if (!g || !counts) return PSSGPU_EINVAL;
     if (k < 1 || k > kMaxFragK) return gfail(g, PSSGPU_EUNSUPP, "kmer_spectrum: k %d outside [1,%d]", k, kMaxFragK);
-    const size_t elems = (size_t)1 << (2 * k);
-    int rc = ensure_red(g, elems);
-    if (rc != PSSGPU_OK) return rc;
     const int n = (int)g->ctx.size();
-    std::vector<int> rcs(n, PSSGPU_OK);
-    std::vector<std::thread> th;
-    for (int i = 0; i < n; i++)                         // the shard call is synchronous: one host thread per GPU
-        th.emplace_back([&, i]() { rcs[i] = pssgpu_kmer_spectrum_shard_device(g->ctx[i].get(), k, i, n, g->d_red[i].get()); });
-    for (auto &t : th) t.join();
-    for (int i = 0; i < n; i++)
-        if (rcs[i] != PSSGPU_OK) return member_fail(g, i, rcs[i]);
-    rc = reduce_sum(g, elems);
-    if (rc != PSSGPU_OK) return rc;
-    Bind bind(g->ctx[0].get());
-    if (cudaMemcpy(counts, g->d_red[0].get(), elems * sizeof(uint64_t), cudaMemcpyDeviceToHost) != cudaSuccess)
-        return gfail(g, PSSGPU_ECUDA, "group: D2H of the spectrum: %s", cudaGetErrorString(cudaGetLastError()));
-    return PSSGPU_OK;
+    return gather_sum(g, (size_t)1 << (2 * k), true,
+                      [&](pssgpu_ctx *c, unsigned long long *d, int i) { return pssgpu_kmer_spectrum_shard_device(c, k, i, n, d); }, counts);
 }
 
 }  // extern "C"

@@ -292,7 +292,9 @@ def test_fused_pss_and_fragkon_pass(small):
     lines.insert(100, good[0] + b"\tXX:Z:" + b"t" * 5000)                   # a record longer than the look-ahead
     sam = b"\n".join(lines) + b"\n"
     for p, fk in ((PssParams(), FkParams(klen=8)),
-                  (PssParams(region_len=20, min_len=30, max_len=80, min_mq=20, merged_only=1), FkParams(klen=5, min_len=25, min_mq=7))):
+                  (PssParams(region_len=20, min_len=30, max_len=80, min_mq=20, merged_only=1), FkParams(klen=5, min_len=25, min_mq=7)),
+                  (PssParams(region_len=5), FkParams(klen=3)),
+                  (PssParams(region_len=40), FkParams(klen=10))):
         f, r, st = ora.pss(sam, p)
         fp, tp, fst = ora.fragkon(sam, fk)
         ctx.both_begin(_opts(p), pkg.FragkonOptions(fk.klen, fk.min_len, fk.max_len, fk.min_mq, fk.merged_only))
