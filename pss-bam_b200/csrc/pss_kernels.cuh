@@ -58,6 +58,16 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
                  ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
+// one arrival at a counter in shared memory; returns the count before it.  Release: after a __syncwarp, the warp's
+// earlier shared-memory accesses are ordered before the arrival; acquire: those of the earlier arrivals are ordered
+// before what follows it.
+__device__ __forceinline__ uint32_t arrive_count(uint32_t *ctr)
+{
+    uint32_t old;
+    asm volatile("atom.acq_rel.cta.shared::cta.add.u32 %0, [%1], 1;" : "=r"(old) : "r"(smem_u32(ctr)) : "memory");
+    return old;
+}
+
 // L2 prefetch of [src, src + bytes): size multiple of 16, address 16-byte aligned
 __device__ __forceinline__ void bulk_prefetch_l2(const void *src_gmem, uint32_t bytes)
 {
@@ -509,6 +519,8 @@ struct TallySmem {
     uint32_t nlpos[kThreads + 4];                             // positions of the first kThreads + 1 newlines
     uint32_t warp_sum[kWarps];                                // generic newline listing only
     uint32_t ctl[2];                                          // range handed to this CTA
+    uint32_t text_done;                                       // warps done reading a tile's text (a multiple of kWarps
+                                                              // between tiles that copy the next one early)
     unsigned long long long_end;                              // where a record longer than the tile ends
     TallyShared sh;
     alignas(8) uint64_t bar;
@@ -1021,12 +1033,12 @@ __device__ __noinline__ uint32_t list_newlines_generic(TallySmem *Sp, int n_vali
 // One warp-load of records: this lane's record is [start, pe) with its
 // terminator at pe (has == false: no record for the lane).  Parses, filters,
 // gathers, tallies, counts outcomes.  All 32 lanes of the warp must call it
-// together.
-template <int MODE, int NACC, int ROWS>
+// together.  text_done() is called by all of them once none reads bytes or le any more.
+template <int MODE, int NACC, int ROWS, class TextDone>
 __device__ __forceinline__ void process_batch(const TallyArgs &A, TallyShared &T, const uint8_t *bytes, const uint32_t *le,
                                               bool has, int start, int pe, uint64_t goff,
                                               uint32_t lane, uint32_t (&acc)[NACC ? NACC : 1], int &acc_iters, int rows,
-                                              uint32_t &st_acc, uint32_t &st_acc_fk)
+                                              uint32_t &st_acc, uint32_t &st_acc_fk, const TextDone &text_done)
 {
     const uint32_t full = 0xffffffffu;
     int            code = has ? (int)kNeedSlow : 99;                    // 99 = no record for this lane
@@ -1074,6 +1086,7 @@ __device__ __forceinline__ void process_batch(const TallyArgs &A, TallyShared &T
     }
     if (code != 99) log_outcome(A, goff, code);
     __syncwarp();
+    text_done();
     if (MODE != kModeFragkon && NACC > 0) {
         tally_rows<NACC, ROWS>(st, acc, rows, lane, A.one);
         if (++acc_iters >= kFlushEvery) { flush_acc<NACC>(acc, rows, lane, T.table); acc_iters = 0; }
@@ -1101,6 +1114,23 @@ __device__ __forceinline__ void process_batch(const TallyArgs &A, TallyShared &T
     }
 }
 
+// The copy that stages the tile beginning at pos: its 16-byte aligned source (gsrc) and its size, `want` bytes rounded
+// so that kPrefix + size is whole 64-byte slots, at most kStageMax, or the rest of the text if that is less.
+__device__ __forceinline__ int stage_size(uint64_t pos, int want, uint64_t len16, uint64_t &gsrc)
+{
+    gsrc = pos ? ((pos - 1) & ~15ull) : 0;
+    want = (want + 16) & ~63; want -= 16;
+    if (want > kStageMax) want = kStageMax;
+    const uint64_t left = len16 - gsrc;
+    return left <= (uint64_t)want ? (int)left : want;
+}
+__device__ __forceinline__ void stage_copy(TallySmem &S, const uint8_t *src, int nb)
+{
+    fence_proxy_async();                              // the generic-proxy accesses of the old tile come first
+    mbar_expect_tx(&S.bar, (uint32_t)nb);
+    bulk_g2s(S.bytes + kPrefix, src, (uint32_t)nb, &S.bar);
+}
+
 // ---------------------------------------------------------------------------
 // tally kernel.
 //
@@ -1112,6 +1142,7 @@ __device__ __forceinline__ void process_batch(const TallyArgs &A, TallyShared &T
 // idle).  Per tile:
 //   stage     one cp.async.bulk (TMA engine) of as many bytes as kThreads
 //             records are expected to take (running estimate), on an mbarrier
+//             that every warp waits on
 //   pass A    a 64-byte slot per thread and step (bank-conflict free quad
 //             order): SWAR classification into the "<= 0x20" mask words
 //             (stored, the record phase walks them) and newline candidates
@@ -1120,7 +1151,13 @@ __device__ __forceinline__ void process_batch(const TallyArgs &A, TallyShared &T
 //             two candidates in a slot or a false one: exact listing
 //   pass B    scan of the kSegs ballot counts (two shuffles deep), newline
 //             positions of ordinals 0..kThreads to shared memory
-//   records   one thread per record (process_batch)
+//   records   one thread per record (process_batch).  When the next tile
+//             starts in the same range, each warp arrives at a counter as
+//             soon as it has read the last byte of this tile's text, and the
+//             last one to arrive issues the next copy while the other warps
+//             still tally: the tile needs no block barrier at its end.  Else
+//             (first record not found yet, a record longer than the tile, the
+//             range ends) a block barrier ends the tile and thread 0 copies.
 // ---------------------------------------------------------------------------
 // NACC = registers of packed partial sums per lane: 9 cover -r <= 16 (the default is 15), 16 cover -r <= 30;
 // 0 = any -r, through pss_record_wide() and global atomics (exact, not tuned).  ROWS = R + 2 as a compile-time
@@ -1136,7 +1173,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) tally_kernel(const __gri
 
     for (uint32_t i = tid; i < 8; i += kThreads) S.le[kChunks + i] = ~0u;
     if (tid < kPrefix) S.bytes[tid] = 'x';                    // never written by a copy; byte 15 becomes '\n' at offset 0
-    if (tid == 0) { mbar_init(&S.bar, 1); fence_mbar_init(); }
+    if (tid == 0) { S.text_done = 0; mbar_init(&S.bar, 1); fence_mbar_init(); }
     cta_prologue(S.sh, A, tid, kThreads);
 
     const int      rows = A.cfg.R + 2;
@@ -1161,30 +1198,19 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) tally_kernel(const __gri
         const uint64_t range_end = (range_begin + A.range_bytes < text_len) ? range_begin + A.range_bytes : text_len;
         uint64_t       pos = range_begin;                     // everything that starts before pos is somebody's business
         bool           want_full = false;
+        bool           staged = false;                        // the copy of the tile at pos is already under way
 
         while (pos < range_end) {
             // ---- stage ----
-            const uint64_t gsrc = pos ? ((pos - 1) & ~15ull) : 0;                 // 16-byte aligned source
+            uint64_t       gsrc;                                                  // 16-byte aligned source
+            const int      nb = stage_size(pos, want_full ? kStageMax : est, len16, gsrc);
             const int64_t  gbase = (int64_t)gsrc - kPrefix;                       // global offset of bytes[0]
             const int      head = (int)((int64_t)pos - 1 - gbase);                // position of the byte before pos: 15..31
-            int            want = want_full ? kStageMax : est;
-            want = (want + 16) & ~63; want -= 16;                                 // kPrefix + want is a multiple of 64: whole slots
-            if (want > kStageMax) want = kStageMax;
-            const uint64_t left = len16 - gsrc;
-            const bool     sees_end = left <= (uint64_t)want;                     // the copy reaches the end of the text
-            const int      nb = sees_end ? (int)left : want;
-            const bool     is_full = sees_end || want >= kStageMax;
+            const bool     sees_end = (uint64_t)nb == len16 - gsrc;               // the copy reaches the end of the text
+            const bool     is_full = sees_end || nb >= kStageMax;
             const int      data_end = sees_end ? (int)((int64_t)text_len - gbase) : kPrefix + nb;
-            if (tid == 0) {
-                fence_proxy_async();
-                mbar_expect_tx(&S.bar, (uint32_t)nb);
-                bulk_g2s(S.bytes + kPrefix, A.sam + gsrc, (uint32_t)nb, &S.bar);
-            }
-            // one warp sleeps on the mbarrier; the others wait at the block barrier without spending issue slots,
-            // then take their own (immediately successful) acquire of the completed phase
-            if (warp == 0) mbar_wait(&S.bar, phase);
-            __syncthreads();
-            if (warp != 0) mbar_wait(&S.bar, phase);
+            if (tid == 0 && !staged) stage_copy(S, A.sam + gsrc, nb);
+            mbar_wait(&S.bar, phase);
             phase ^= 1u;
 
             // bytes before the record start / after the end of the text are neutralised by the thread that scans them
@@ -1305,6 +1331,14 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) tally_kernel(const __gri
                 }
             }
             // ---- records ----
+            const bool early = n_take > 0 && next < range_end;                   // block uniform
+            const auto text_done = [&]() {                    // every lane of the warp is past its last read of bytes and le
+                if (early && lane == 0 && arrive_count(&S.text_done) % kWarps == kWarps - 1) {
+                    uint64_t nsrc;                                                // the last warp: the next tile, as the stage above will see it
+                    const int nnb = stage_size(next, est, len16, nsrc);
+                    stage_copy(S, A.sam + nsrc, nnb);
+                }
+            };
             {
                 const bool     in = (int)tid < n_take;
                 const int      start = in ? (int)S.nlpos[tid] + 1 : kPrefix;
@@ -1312,12 +1346,18 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) tally_kernel(const __gri
                 const uint64_t goff = (uint64_t)(gbase + start);
                 const bool     has = in && start < data_end && goff < range_end;
                 if (__any_sync(full, has))
-                    process_batch<MODE, NACC, ROWS>(A, S.sh, S.bytes, S.le, has, start, pe, goff, lane, acc, acc_iters, rows, st_acc, st_acc_fk);
+                    process_batch<MODE, NACC, ROWS>(A, S.sh, S.bytes, S.le, has, start, pe, goff, lane, acc, acc_iters, rows, st_acc, st_acc_fk,
+                                                    text_done);
+                else
+                    text_done();
             }
 
             want_full = next_full;
             pos = next;
-            __syncthreads();                                  // tile (and nlpos) fully consumed before it is overwritten
+            staged = early;
+            // the next tile's copy, pass A and pass B overwrite bytes, le and nlpos only once the copy has landed, i.e.
+            // after every warp arrived; without an early copy this barrier orders them after the last reads instead
+            if (!early) __syncthreads();
         }
     }
 

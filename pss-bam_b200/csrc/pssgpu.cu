@@ -619,23 +619,17 @@ int fk_cfg(pssgpu_ctx *ctx, const pssgpu_fragkon_params *p, TallyCfg &c)
     return PSSGPU_OK;
 }
 
-int alloc_pss_tables(pssgpu_ctx *ctx, int R)
+// A zeroed count table of `elems` u64 in buf (of `have` elements), queued on the context's stream.  The buffer is
+// replaced only when its size changes; a launch still queued may read the old one, so the stream drains first.
+int zero_table(pssgpu_ctx *ctx, DevPtr<unsigned long long> &buf, size_t &have, size_t elems)
 {
-    const size_t elems = 2 * (size_t)(R + 2) * 16;
-    CU(alloc(ctx->d_tables, elems * sizeof(unsigned long long)));
-    CU(cudaMemsetAsync(ctx->d_tables.get(), 0, elems * sizeof(unsigned long long), ctx->stream.get()));
-    return PSSGPU_OK;
-}
-
-int alloc_fk_tables(pssgpu_ctx *ctx, int K)
-{
-    const size_t elems = 2ull << (2 * K);
-    if (elems != ctx->fk_elems) {
-        ctx->fk_elems = 0;
-        CU(alloc(ctx->d_fk, elems * sizeof(unsigned long long)));
-        ctx->fk_elems = elems;
+    if (elems != have) {
+        if (buf) CU(cudaStreamSynchronize(ctx->stream.get()));
+        have = 0;
+        CU(alloc(buf, elems * sizeof(unsigned long long)));
+        have = elems;
     }
-    CU(cudaMemsetAsync(ctx->d_fk.get(), 0, elems * sizeof(unsigned long long), ctx->stream.get()));
+    CU(cudaMemsetAsync(buf.get(), 0, elems * sizeof(unsigned long long), ctx->stream.get()));
     return PSSGPU_OK;
 }
 
@@ -655,17 +649,19 @@ int begin_tally(pssgpu_ctx *ctx, const char *fn, int mode, const pssgpu_pss_para
     // the parameters were accepted: no tally is open until the begin completes (a table it failed to allocate must
     // never be fed)
     ctx->mode = -1;
-    CU(cudaStreamSynchronize(ctx->stream.get()));
+    // Everything below is queued behind the launches of the previous tally, which may still run, except the BAM
+    // ingest bookkeeping bam_reset clears: it describes work on the stream, so a context that ingested BAM drains it.
+    // (`cur` stays: copy_stream has already waited for the last tally that read d_stage[cur].)
+    if (ctx->bam) CU(cudaStreamSynchronize(ctx->stream.get()));
     if (!ctx->d_stats) CU(alloc(ctx->d_stats, 2 * kStN * sizeof(unsigned long long)));
     if (!ctx->d_range_ctr) CU(alloc(ctx->d_range_ctr, sizeof(unsigned int)));
     CU(cudaMemsetAsync(ctx->d_stats.get(), 0, 2 * kStN * sizeof(unsigned long long), ctx->stream.get()));
     if (ctx->dbg_cap) CU(cudaMemsetAsync(ctx->d_dbg_n.get(), 0, sizeof(unsigned long long), ctx->stream.get()));
     ctx->carry_len = 0;
-    ctx->cur = 0;
     ctx->fed_bytes = 0;
     bam_reset(ctx);
-    if (pss && (rc = alloc_pss_tables(ctx, c.R)) != PSSGPU_OK) return rc;
-    if (fk && (rc = alloc_fk_tables(ctx, cf.K)) != PSSGPU_OK) return rc;
+    if (pss && (rc = zero_table(ctx, ctx->d_tables, ctx->pss_elems, 2 * (size_t)(c.R + 2) * 16)) != PSSGPU_OK) return rc;
+    if (fk && (rc = zero_table(ctx, ctx->d_fk, ctx->fk_elems, 2ull << (2 * cf.K))) != PSSGPU_OK) return rc;
     if (mode == kModeBoth) {
         c.mode = kModeBoth;
         ctx->cfg_fk = cf;

@@ -97,6 +97,7 @@ struct pssgpu_ctx {
     pssgpu::TallyCfg  cfg{};
     pssgpu::TallyCfg  cfg_fk{};               // fragkon options of the fused mode
     pssgpu::DevPtr<unsigned long long> d_tables;      // pss: 2*(R+2)*16
+    size_t    pss_elems = 0;
     pssgpu::DevPtr<unsigned long long> d_fk;          // fragkon: 2*4^K
     size_t    fk_elems = 0;
     pssgpu::DevPtr<unsigned long long> d_stats;       // 2 x kStN: outcomes, and fragkon's outcomes in the fused mode
